@@ -39,6 +39,16 @@ def make_inputs(batch, seed):
     return a, mat
 
 
+DUMP_ROWS = 256  # ciphertexts --dump-outputs writes: 256 x 3 limbs x 2 columns x 4096 coefficients in float64 = 48 MiB
+
+
+def dump_rows(batch):
+    """Indices of the ciphertexts --dump-outputs writes: a fixed, seeded sample of the batch, in ascending order."""
+    if batch <= DUMP_ROWS:
+        return np.arange(batch)
+    return np.sort(np.random.default_rng(2024).choice(batch, DUMP_ROWS, replace=False))
+
+
 def peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -199,7 +209,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
     ap.add_argument("--no-aux", action="store_true", help="skip the auxiliary measurements")
     ap.add_argument("--no-cggi", action="store_true", help="skip the CGGI bootstraps/s object")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the key-switch results of the last timed step (rank 0, a fixed seeded sample of the batch) to "
+                         "DIR/glwe_keyswitch.npy as float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU implementation only")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)
@@ -304,6 +321,10 @@ def main():
     e2e_value = world * B * e2e_steps / float(t.item())
     check = m.vec_znx_to_numpy(res_dev)
     assert np.array_equal(check, r_host), "device-resident and host-path results differ"
+    if args.dump_outputs and rank == 0:
+        # res_dev still holds the last timed step (the e2e leg writes r_host only); normalised digits are exact in float64
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "glwe_keyswitch.npy"), check[dump_rows(B)].astype(np.float64))
 
     # ---- roofline of the dominant kernel ----------------------------------------------------------------------------
     n = w["n"]

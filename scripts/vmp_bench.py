@@ -1,5 +1,5 @@
-import sys, ctypes as C
-sys.path.insert(0, '/root/repo')
+import os, sys, ctypes as C
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import poulpy_b200 as pb
 lib = pb.lib()
