@@ -454,6 +454,31 @@ int pgb_cggi_blind_rotate_extended_batched(pgb_module *m, pgb_vec_znx *res, cons
  * stride bt->stride_a; res = device int64 [count][n_lwe + 1]; two_n_domain = 2 * lut.domain_size(); rot_left = LookUpTableRotationDirection::Left. */
 int pgb_cggi_mod_switch_2n_batched(pgb_module *m, int64_t *res, const pgb_vec_znx *lwe, uint64_t lwe_base2k, uint64_t two_n_domain,
                                    int rot_left, const pgb_batch *bt);
+/* ---- LWE <-> GLWE (poulpy-core/src/conversion/glwe_to_lwe.rs, lwe_to_glwe.rs, keyswitching/lwe.rs) ----
+ * An LWE is a one-column VecZnx of n = n_lwe + 1 coefficients per limb, (b, a_0, .., a_{n_lwe-1}), phase b + <a, s_lwe>, 1 <= n_lwe <= N;
+ * its GLWE embedding is the rank-1 secret s_glwe(X) = s_lwe(X^-1).  Batches as everywhere (stride_res / stride_a, at least one item),
+ * count in [1, 65535]; LWE data and strides are multiples of 8 bytes, GLWE data and strides multiples of 16, scratch 256-byte aligned.
+ * There is no in-place form: any overlap of res and a is PGB_ERR_ALIAS.
+ * sample_extract: a = rank-1 GLWE; limbs i < min(res.size, a.size) get (a[0][i][0], a[1][i][0..n_lwe)), the other limbs of res are zeroed.
+ * lwe_keyswitch: key = VmpPMat(dnum, 1, 2, key_size) from embed(s_in) to embed(s_out); a is embedded into a rank-1 GLWE, key-switched with
+ *   pgb_glwe_keyswitch_batched into res.size limbs of res_base2k and sample-extracted.
+ * glwe_to_lwe: a = GLWE of rank k, key = VmpPMat(dnum, k, 2, key_size) to embed(s_lwe); key-switch to rank 1, then sample-extract.
+ * lwe_to_glwe: res = GLWE of rank k, key = VmpPMat(dnum, 1, k + 1, key_size) from embed(s_lwe); embed, then key-switch into res.
+ * The *_tmp_bytes take the arguments of pgb_glwe_keyswitch_tmp_bytes: the staged rank-1 GLWE(s) plus the inner key-switch's scratch. */
+int pgb_lwe_sample_extract_batched(pgb_module *m, pgb_vec_znx *res, const pgb_vec_znx *a, const pgb_batch *bt);
+size_t pgb_lwe_keyswitch_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_t a_size, uint64_t a_base2k, const pgb_vmp_pmat *key,
+                                   uint64_t key_base2k, uint64_t dsize, uint64_t batch);
+int pgb_lwe_keyswitch_batched(pgb_module *m, pgb_vec_znx *res, uint64_t res_base2k, const pgb_vec_znx *a, uint64_t a_base2k,
+                              const pgb_vmp_pmat *key, uint64_t key_base2k, uint64_t dsize, const pgb_batch *bt, void *scratch, size_t scratch_len);
+size_t pgb_glwe_to_lwe_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_t a_size, uint64_t a_base2k, const pgb_vmp_pmat *key,
+                                 uint64_t key_base2k, uint64_t dsize, uint64_t batch);
+int pgb_glwe_to_lwe_batched(pgb_module *m, pgb_vec_znx *res, uint64_t res_base2k, const pgb_vec_znx *a, uint64_t a_base2k,
+                            const pgb_vmp_pmat *key, uint64_t key_base2k, uint64_t dsize, const pgb_batch *bt, void *scratch, size_t scratch_len);
+size_t pgb_lwe_to_glwe_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_t a_size, uint64_t a_base2k, const pgb_vmp_pmat *key,
+                                 uint64_t key_base2k, uint64_t dsize, uint64_t batch);
+int pgb_lwe_to_glwe_batched(pgb_module *m, pgb_vec_znx *res, uint64_t res_base2k, const pgb_vec_znx *a, uint64_t a_base2k,
+                            const pgb_vmp_pmat *key, uint64_t key_base2k, uint64_t dsize, const pgb_batch *bt, void *scratch, size_t scratch_len);
+
 /* execute_standard (algorithm.rs:370-443, block_size == 1 keys): per LWE coefficient one GGSW x GLWE external product, X^{a_i} - 1, add;
  * one glwe_normalize_assign at the end.  Same argument conventions as pgb_cggi_blind_rotate_batched. */
 size_t pgb_cggi_blind_rotate_standard_tmp_bytes(const pgb_module *m, uint64_t rank, uint64_t res_size, uint64_t res_base2k,

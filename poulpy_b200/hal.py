@@ -82,7 +82,8 @@ def lib():
         for name in ("pgb_glwe_keyswitch_tmp_bytes", "pgb_glwe_external_product_tmp_bytes", "pgb_cggi_blind_rotate_tmp_bytes",
                      "pgb_cggi_blind_rotate_standard_tmp_bytes", "pgb_cggi_blind_rotate_extended_tmp_bytes", "pgb_vmp_apply_dft_tmp_bytes", "pgb_glwe_tensor_apply_tmp_bytes",
                      "pgb_glwe_tensor_relinearize_tmp_bytes", "pgb_glwe_automorphism_tmp_bytes", "pgb_glwe_automorphism_add_assign_tmp_bytes",
-                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_vec_znx_big_automorphism_assign_tmp_bytes", "pgb_ggsw_expand_row_tmp_bytes",
+                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
+                     "pgb_vec_znx_big_automorphism_assign_tmp_bytes", "pgb_ggsw_expand_row_tmp_bytes",
                      "pgb_bytes_of_vmp_pmat", "pgb_size_of_scalar_prep", "pgb_size_of_scalar_big"):
             getattr(_lib, name).restype = C.c_size_t
     return _lib
@@ -775,6 +776,54 @@ class Module:
         _check(lib().pgb_cggi_mod_switch_2n_batched(self._h, C.c_void_p(out.ptr), C.byref(lv), _u64(lwe_base2k), _u64(two_n_domain),
                                                     C.c_int(1 if rot_left else 0), C.byref(bt)))
         return out
+
+    # --- LWE <-> GLWE (poulpy-core/src/conversion/glwe_to_lwe.rs, lwe_to_glwe.rs, keyswitching/lwe.rs) ----------------------------------
+    # An LWE batch is a DevBuf of `batch` one-column VecZnx(n_lwe + 1, size) (b, a_0, ..), item b at b * stride bytes (default: back to
+    # back, stride = size * (n_lwe + 1) * 8).  Asynchronous like every batched call: sync() before reading the results.
+    @staticmethod
+    def _lwe(buf: DevBuf, n_lwe, size):
+        return _VZ(buf.ptr, n_lwe + 1, 1, size, size)
+
+    @staticmethod
+    def _lwe_stride(n_lwe, size, stride):
+        return size * (n_lwe + 1) * 8 if stride is None else stride
+
+    def _lwe_call(self, name, r, res_size, res_base2k, av, a_size, a_base2k, key: VmpPMat, key_base2k, dsize, bt, scratch):
+        ks = key.struct()
+        need = getattr(lib(), name + "_tmp_bytes")(self._h, _u64(res_size), _u64(a_size), _u64(a_base2k), C.byref(ks), _u64(key_base2k),
+                                                   _u64(dsize), _u64(bt.count))
+        if scratch is None or scratch.nbytes < need:
+            scratch = self._scratch(need)
+        _check(getattr(lib(), name + "_batched")(self._h, C.byref(r), _u64(res_base2k), C.byref(av), _u64(a_base2k), C.byref(ks),
+                                                 _u64(key_base2k), _u64(dsize), C.byref(bt), C.c_void_p(scratch.ptr), C.c_size_t(scratch.nbytes)))
+        return scratch
+
+    def lwe_sample_extract(self, res: DevBuf, n_lwe, res_size, a: VecZnx, res_stride=None):
+        """LWE::sample_extract of the a.batch rank-1 GLWEs of `a` into the LWE batch `res`."""
+        bt = _BT(a.batch, self._lwe_stride(n_lwe, res_size, res_stride), a.batch_stride, 0)
+        r, av = self._lwe(res, n_lwe, res_size), a.struct()
+        _check(lib().pgb_lwe_sample_extract_batched(self._h, C.byref(r), C.byref(av), C.byref(bt)))
+
+    def lwe_keyswitch(self, res: DevBuf, n_out, res_size, res_base2k, a: DevBuf, n_in, a_size, a_base2k, key: VmpPMat, key_base2k, batch,
+                      dsize=1, scratch: DevBuf = None, res_stride=None, a_stride=None):
+        """LWE::keyswitch of `batch` LWEs of dimension n_in into dimension n_out; key = VmpPMat(dnum, 1, 2, key_size)."""
+        bt = _BT(batch, self._lwe_stride(n_out, res_size, res_stride), self._lwe_stride(n_in, a_size, a_stride), 0)
+        return self._lwe_call("pgb_lwe_keyswitch", self._lwe(res, n_out, res_size), res_size, res_base2k, self._lwe(a, n_in, a_size), a_size,
+                              a_base2k, key, key_base2k, dsize, bt, scratch)
+
+    def glwe_to_lwe(self, res: DevBuf, n_lwe, res_size, res_base2k, a: VecZnx, a_base2k, key: VmpPMat, key_base2k, dsize=1,
+                    scratch: DevBuf = None, res_stride=None):
+        """LWE::from_glwe of the a.batch GLWEs of rank k; key = VmpPMat(dnum, k, 2, key_size)."""
+        bt = _BT(a.batch, self._lwe_stride(n_lwe, res_size, res_stride), a.batch_stride, 0)
+        return self._lwe_call("pgb_glwe_to_lwe", self._lwe(res, n_lwe, res_size), res_size, res_base2k, a.struct(), a.size, a_base2k, key,
+                              key_base2k, dsize, bt, scratch)
+
+    def lwe_to_glwe(self, res: VecZnx, res_base2k, a: DevBuf, n_lwe, a_size, a_base2k, key: VmpPMat, key_base2k, dsize=1,
+                    scratch: DevBuf = None, a_stride=None):
+        """GLWE::from_lwe of res.batch LWEs into GLWEs of rank k; key = VmpPMat(dnum, 1, k + 1, key_size)."""
+        bt = _BT(res.batch, res.batch_stride, self._lwe_stride(n_lwe, a_size, a_stride), 0)
+        return self._lwe_call("pgb_lwe_to_glwe", res.struct(), res.size, res_base2k, self._lwe(a, n_lwe, a_size), a_size, a_base2k, key,
+                              key_base2k, dsize, bt, scratch)
 
     def cggi_blind_rotate_standard(self, res: VecZnx, res_base2k, lwe_2n: DevBuf, n_lwe, lut: VecZnx, brk: VmpPMat, brk_base2k,
                                    scratch: DevBuf = None):
