@@ -209,6 +209,11 @@ int pgb_vmp_apply_dft(pgb_module *m, pgb_vec_znx_dft *res, const pgb_vec_znx *a,
                       size_t scratch_len);
 /* HalImpl::vmp_prepare :620 (ntt120/vmp.rs:64-119, fft64/vmp.rs:52-93); `a` is a MatZnx of i64. */
 int pgb_vmp_prepare(pgb_module *m, pgb_vmp_pmat *res, const pgb_mat_znx *a);
+/* count MatZnx -> count VmpPMat in one forward-transform launch: item b reads a->data + b*stride_a and writes res->data + b*stride_res
+ * (VmpPMat data and stride multiples of 16 bytes, MatZnx multiples of 8, strides at least one matrix; count in [1, 65535]).  res and a
+ * must not overlap (PGB_ERR_ALIAS).  Like pgb_vmp_prepare it drops the cached gadget forms of every pinned key inside the written extent.
+ * Asynchronous (call pgb_module_sync before reading). */
+int pgb_vmp_prepare_batched(pgb_module *m, pgb_vmp_pmat *res, const pgb_mat_znx *a, const pgb_batch *bt);
 /* HalImpl::vmp_apply_dft_to_dft :653 (ntt120/vmp.rs:301-341 + core :169-288; fft64/vmp.rs:144-264).
  * Overwrites res; limb_offset is in limbs and is scaled by cols_out exactly as ntt120/vmp.rs:335. */
 int pgb_vmp_apply_dft_to_dft(pgb_module *m, pgb_vec_znx_dft *res, const pgb_vec_znx_dft *a, const pgb_vmp_pmat *pmat,
@@ -272,6 +277,22 @@ size_t pgb_glwe_external_product_tmp_bytes(const pgb_module *m, uint64_t res_siz
 int pgb_glwe_external_product_batched(pgb_module *m, pgb_vec_znx *res, uint64_t res_base2k, const pgb_vec_znx *a,
                                       uint64_t a_base2k, const pgb_vmp_pmat *ggsw, uint64_t ggsw_base2k, uint64_t dsize,
                                       const pgb_batch *bt, void *scratch, size_t scratch_len);
+
+/* CMux (poulpy-bin-fhe: glwe_sub, glwe_normalize_inplace, glwe_external_product_inplace, glwe_add_inplace, glwe_normalize_inplace).
+ * t, f, res: GLWEs VecZnx(k + 1, .) in base 2^base2k; item b at data + b*stride (bt->stride_res for res, bt->stride_a for t, bt->stride_b
+ * for f; t and f may use stride 0 to share one operand).  s: prepared GGSWs VmpPMat(dnum, k + 1, k + 1, s_size) in base 2^ggsw_base2k,
+ * item b's selector at s->data + b*ggsw_stride (0 = one selector shared by the batch; otherwise a multiple of 16 of at least
+ * pgb_bytes_of_vmp_pmat).  Per item:
+ *   1. d[i] = t[i] - f[i] (wrapping i64) for i < res.size, a limb missing from an operand reads as 0;   2. d = vec_znx_normalize_assign(d);
+ *   3. e = glwe_external_product(d, s_b) into res.size limbs of base2k (any dsize, mixed ggsw_base2k);
+ *   4. e[i] += f[i] (wrapping i64) for i < min(res.size, f.size);   5. res = vec_znx_normalize_assign(e).
+ * count in [1, 65535]; GLWE data and strides multiples of 16; scratch 256-byte aligned.  res must not overlap t, f, a selector or the
+ * scratch (PGB_ERR_ALIAS); t and f are read-only and may overlap each other.  Every check runs before the first launch. */
+size_t pgb_glwe_cmux_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_t t_size, uint64_t f_size, uint64_t base2k,
+                               const pgb_vmp_pmat *s, uint64_t ggsw_base2k, uint64_t dsize, uint64_t batch);
+int pgb_glwe_cmux_batched(pgb_module *m, pgb_vec_znx *res, const pgb_vec_znx *t, const pgb_vec_znx *f, uint64_t base2k,
+                          const pgb_vmp_pmat *s, uint64_t ggsw_stride, uint64_t ggsw_base2k, uint64_t dsize,
+                          const pgb_batch *bt, void *scratch, size_t scratch_len);
 
 /* Pinned keys.  The single-kernel gadget products derive per-key forms of a prepared key before they run (NTT120: the collapsed key and
  * the bit bound of the key's coefficients, three small launches; FFT64: a re-laid-out copy, one launch).  Every buffer is caller-owned, so

@@ -135,6 +135,17 @@ def circuit_bootstrap_to_constant(module: "hal.Module", lwe_dev: "hal.DevBuf", b
     return ggsw
 
 
+def prepare_ggsw(module: "hal.Module", ggsw_buf: "hal.DevBuf", batch, dnum, rank, size) -> "hal.VmpPMat":
+    """GGSW::prepare of a circuit-bootstrapping output (`batch` consecutive MatZnx(dnum, rank+1, rank+1, size), as returned by
+    circuit_bootstrap_to_constant / _to_exponent) -> a batched VmpPMat, one prepared GGSW per item, in one launch; it drives
+    Module.glwe_cmux with one selector per ciphertext.  Asynchronous: the module's stream orders it before the next call."""
+    cols = rank + 1
+    mat = hal.MatZnx(ggsw_buf, module.n, dnum, cols, cols, size, batch=batch, batch_stride=module.n * dnum * cols * cols * size * 8)
+    pmat = module.vmp_pmat_alloc(dnum, cols, cols, size, batch=batch)
+    module.vmp_prepare_batched(pmat, mat)
+    return pmat
+
+
 # ---- glwe_pack / post_process / exponent mode -----------------------------------------------------------------------------------
 class DeviceGlweOps:
     """The GLWE operations `pack_internal` and `post_process` are made of, on batches of device-resident GLWEs (VecZnx with a batch axis)

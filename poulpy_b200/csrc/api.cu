@@ -599,6 +599,36 @@ extern "C" int pgb_vmp_prepare(pgb_module *m, pgb_vmp_pmat *res, const pgb_mat_z
     else PGB_TRY(fft64_forward(m, in, out, (int)polys, 1));
     return sync_if(m, true);
 }
+// count MatZnx (a.data + b * stride_a) -> count VmpPMat (res.data + b * stride_res): the same per-polynomial forward transform as
+// pgb_vmp_prepare, as ONE launch over count * polys polynomials (the batch stride of the LimbSets).  Asynchronous like every batched entry.
+extern "C" int pgb_vmp_prepare_batched(pgb_module *m, pgb_vmp_pmat *res, const pgb_mat_znx *a, const pgb_batch *bt) {
+    PGB_REQUIRE(bt && bt->count >= 1 && bt->count <= 65535, "vmp_prepare_batched: batch count must be in [1, 65535]");
+    CHECK_N(res, "vmp_prepare_batched(res)");
+    CHECK_N(a, "vmp_prepare_batched(a)");
+    PGB_REQUIRE(res->rows == a->rows && res->cols_in == a->cols_in && res->cols_out == a->cols_out && res->size == a->size,
+                "vmp_prepare_batched: shape mismatch between VmpPMat and MatZnx");
+    const uint64_t n = m->n, pb = prep_bytes(m), B = bt->count;
+    const uint64_t polys = a->rows * a->cols_in * a->cols_out * a->size;
+    const uint64_t res_item = polys * n * pb, a_item = polys * n * 8;
+    PGB_REQUIRE(polys >= 1 && polys * B <= 0x7fffffffull, "vmp_prepare_batched: %llu polynomials per call (must be in [1, 2^31))",
+                (unsigned long long)(polys * B));
+    PGB_REQUIRE(res->data && (uintptr_t)res->data % 16 == 0 && bt->stride_res % 16 == 0 && (B == 1 || bt->stride_res >= res_item),
+                "vmp_prepare_batched: VmpPMat data and stride must be multiples of 16 bytes, the stride at least one matrix (%llu bytes)",
+                (unsigned long long)res_item);
+    PGB_REQUIRE(a->data && (uintptr_t)a->data % 8 == 0 && bt->stride_a % 8 == 0 && (B == 1 || bt->stride_a >= a_item),
+                "vmp_prepare_batched: MatZnx data and stride must be multiples of 8 bytes, the stride at least one matrix (%llu bytes)",
+                (unsigned long long)a_item);
+    const uint64_t res_ext = batch_extent(res_item, bt->stride_res, B);
+    if (ranges_overlap(res->data, res_ext, a->data, batch_extent(a_item, bt->stride_a, B))) {
+        pgb_set_error("vmp_prepare_batched: res and a must not overlap");
+        return PGB_ERR_ALIAS;
+    }
+    key_cache_invalidate(m, res->data, res_ext); // every pinned key inside the written extent loses its cached gadget forms
+    LimbSet in = {(char *)a->data, n * 8, bt->stride_a};
+    LimbSet out = {(char *)res->data, n * pb, bt->stride_res};
+    if (m->flavour == PGB_NTT120) return ntt120_forward(m, in, out, (int)polys, (int)B);
+    return fft64_forward(m, in, out, (int)polys, (int)B);
+}
 
 int vmp_apply_impl(pgb_module *m, pgb_vec_znx_dft *res, const pgb_vec_znx_dft *a, const pgb_vmp_pmat *pmat, uint64_t limb_offset,
                    const pgb_batch *bt) {

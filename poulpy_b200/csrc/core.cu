@@ -318,10 +318,6 @@ extern "C" int pgb_glwe_external_product_batched(pgb_module *m, pgb_vec_znx *res
                                      (int)cols, nullptr, 0, 0, 0, (char *)res->data, bt->stride_res, res->cols * n * 8, (int)res->size,
                                      (int)ggsw_base2k, 0, (int)B, (const char *)ain.data, ain_bs, n * ain.cols * ain.size);
         }
-        for (uint64_t j = 0; j < cols; j++) PGB_TRY(pgb_vec_znx_dft_apply_batched(m, 1, 0, &a_dft, j, &ain, j, &btd));
-        PGB_CHECK_CUDA(cudaMemsetAsync(res_dft.data, 0, B * res_dft_bs, m->stream)); // res_dft.zero() (:123)
-        pgb_batch btv = {B, res_dft_bs, a_dft_bs, 0};
-        PGB_TRY(vmp_apply_impl(m, &res_dft, &a_dft, ggsw, 0, &btv));
     } else {
         if (dsize == 2 && res_base2k == ggsw_base2k && m->flavour == PGB_FFT64 && !opt_on(m, PGB_OPT_NO_FUSION) && cols * a_size <= 16 &&
             fft64_gadget_supported(m, (int)(cols * a_size), (int)cols, (int)ggsw->size, (int)ggsw_base2k, (int)B))
@@ -354,36 +350,60 @@ extern "C" int pgb_glwe_external_product_batched(pgb_module *m, pgb_vec_znx *res
                 ar.used = mark; // redo the batch limb by limb
             }
         }
-        PGB_CHECK_CUDA(cudaMemsetAsync(res_dft.data, 0, B * res_dft_bs, m->stream)); // res_dft.zero() (:123)
-        pgb_vec_znx_dft tmp = mk(ar.take(B * res_dft_bs), n, cols, ggsw->size);
-        PGB_REQUIRE(tmp.data, "glwe_external_product: scratch exhausted");
+    }
+    void *tmp = nullptr;
+    if (dsize > 1) {
+        tmp = ar.take(B * res_dft_bs);
+        PGB_REQUIRE(tmp, "glwe_external_product: scratch exhausted");
+    }
+    return external_product_limbwise(m, res, bt->stride_res, res_base2k, &ain, ain_bs, ggsw, 0, ggsw_base2k, dsize, B, &res_dft, &a_dft, tmp);
+}
+
+// glwe_external_product_internal (:197-271) as the limb-wise HAL sequence, then the normalisation into res (:138-140).  ain is already in
+// ggsw_base2k; res_dft (cols, ggsw.size), a_dft (cols, ceil(ain.size / dsize)) and, for dsize > 1, `tmp` (the size of res_dft) are the
+// caller's scratch.  ggsw_bs strides the GGSW per item (0: one GGSW for the whole batch).
+int external_product_limbwise(pgb_module *m, pgb_vec_znx *res, uint64_t res_bs, uint64_t res_base2k, const pgb_vec_znx *ain, uint64_t ain_bs,
+                              const pgb_vmp_pmat *ggsw, uint64_t ggsw_bs, uint64_t ggsw_base2k, uint64_t dsize, uint64_t B,
+                              pgb_vec_znx_dft *res_dft, pgb_vec_znx_dft *a_dft, void *tmp_data) {
+    const uint64_t n = m->n, pb = prep_bytes(m), cols = ggsw->cols_in, a_size = ain->size;
+    const uint64_t res_dft_bs = n * cols * ggsw->size * pb, a_dft_bs = n * cols * a_dft->size * pb;
+    if (dsize == 1) {
+        pgb_batch btd = {B, a_dft_bs, ain_bs, 0};
+        for (uint64_t j = 0; j < cols; j++) PGB_TRY(pgb_vec_znx_dft_apply_batched(m, 1, 0, a_dft, j, ain, j, &btd));
+        PGB_CHECK_CUDA(cudaMemsetAsync(res_dft->data, 0, B * res_dft_bs, m->stream)); // res_dft.zero() (:123)
+        pgb_batch btv = {B, res_dft_bs, a_dft_bs, ggsw_bs};
+        PGB_TRY(vmp_apply_impl(m, res_dft, a_dft, ggsw, 0, &btv));
+    } else {
+        PGB_CHECK_CUDA(cudaMemsetAsync(res_dft->data, 0, B * res_dft_bs, m->stream)); // res_dft.zero() (:123)
+        pgb_vec_znx_dft tmp = mk(tmp_data, n, cols, ggsw->size);
         // the temporary starts zeroed (a fresh allocation in the oracle's model of the scratch arena): with dsize > 1 the FFT64 vmp leaves
         // limbs past the shifted key untouched, so the result must not depend on what a reused scratch held before
         PGB_CHECK_CUDA(cudaMemsetAsync(tmp.data, 0, B * res_dft_bs, m->stream));
         // a_dft.data_mut().fill(0) (:226): FFT64 dft_apply leaves limbs past a.size untouched inside min_steps
-        PGB_CHECK_CUDA(cudaMemsetAsync(a_dft.data, 0, B * a_dft_bs, m->stream));
+        PGB_CHECK_CUDA(cudaMemsetAsync(a_dft->data, 0, B * a_dft_bs, m->stream));
         for (uint64_t di = 0; di < dsize; di++) {
-            a_dft.size = (a_size + di) / dsize;
+            a_dft->size = (a_size + di) / dsize;
             const int64_t cut = (int64_t)(dsize - di) - 2;
-            res_dft.size = ggsw->size - (uint64_t)(cut > 0 ? cut : 0);
+            res_dft->size = ggsw->size - (uint64_t)(cut > 0 ? cut : 0);
             pgb_batch btd = {B, a_dft_bs, ain_bs, 0};
-            for (uint64_t j = 0; j < cols; j++) PGB_TRY(pgb_vec_znx_dft_apply_batched(m, dsize, dsize - 1 - di, &a_dft, j, &ain, j, &btd));
+            for (uint64_t j = 0; j < cols; j++) PGB_TRY(pgb_vec_znx_dft_apply_batched(m, dsize, dsize - 1 - di, a_dft, j, ain, j, &btd));
             if (di == 0) {
-                pgb_batch btv = {B, res_dft_bs, a_dft_bs, 0};
-                PGB_TRY(vmp_apply_impl(m, &res_dft, &a_dft, ggsw, 0, &btv));
+                pgb_batch btv = {B, res_dft_bs, a_dft_bs, ggsw_bs};
+                PGB_TRY(vmp_apply_impl(m, res_dft, a_dft, ggsw, 0, &btv));
             } else {
-                tmp.size = res_dft.size;
-                pgb_batch btv = {B, res_dft_bs, a_dft_bs, 0};
-                PGB_TRY(vmp_apply_impl(m, &tmp, &a_dft, ggsw, di, &btv));
+                tmp.size = res_dft->size;
+                pgb_batch btv = {B, res_dft_bs, a_dft_bs, ggsw_bs};
+                PGB_TRY(vmp_apply_impl(m, &tmp, a_dft, ggsw, di, &btv));
                 pgb_batch bta = {B, res_dft_bs, res_dft_bs, 0};
-                for (uint64_t c = 0; c < cols; c++) PGB_TRY(pgb_vec_znx_dft_add_assign_batched(m, &res_dft, c, &tmp, c, &bta));
+                for (uint64_t c = 0; c < cols; c++) PGB_TRY(pgb_vec_znx_dft_add_assign_batched(m, res_dft, c, &tmp, c, &bta));
             }
         }
+        res_dft->size = ggsw->size;
     }
     pgb_batch btc = {B, res_dft_bs, 0, 0};
-    PGB_TRY(pgb_vec_znx_idft_apply_consume_batched(m, &res_dft, &btc));
-    pgb_vec_znx_big res_big = res_dft;
-    pgb_batch btn = {B, bt->stride_res, res_dft_bs, 0};
+    PGB_TRY(pgb_vec_znx_idft_apply_consume_batched(m, res_dft, &btc));
+    pgb_vec_znx_big res_big = *res_dft;
+    pgb_batch btn = {B, res_bs, res_dft_bs, 0};
     for (uint64_t j = 0; j < res->cols; j++)
         PGB_TRY(big_normalize_impl(m, res, res_base2k, 0, j, &res_big, ggsw_base2k, j, 0, true, &btn));
     return PGB_OK;

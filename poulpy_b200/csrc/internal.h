@@ -43,9 +43,11 @@ bool ntt120_fused_supported(const pgb_module *m);
 int ntt120_fused_back(pgb_module *m, const char *a_dft, uint64_t a_bs, const char *pmat, int R, int C, int cols_out, const char *small,
                       uint64_t small_bs, uint64_t small_limb_stride, int small_size, char *res, uint64_t res_bs, uint64_t res_limb_stride,
                       int res_size, int base2k, int64_t res_offset, int batch, const char *glwe, uint64_t glwe_bs, uint64_t glwe_words,
-                      const int *skip = nullptr, bool skip_list = false, bool direct = false, bool small_all_cols = false);
+                      const int *skip = nullptr, bool skip_list = false, bool direct = false, bool small_all_cols = false,
+                      uint64_t pmat_bs = 0);
 // direct: a_dft already holds the C = cols_out * size product polys (limb-major, column-minor), pmat / R are ignored: inverse transform +
-// CRT + add_small + normalize only; small_all_cols: `small` is added on every output column (CGGI: acc += ...), not only on column 0
+// CRT + add_small + normalize only; small_all_cols: `small` is added on every output column (CGGI: acc += ...), not only on column 0;
+// pmat_bs: item b multiplies by the matrix at pmat + b * pmat_bs (0 = one matrix for the whole batch; the collapsed-key path needs 0)
 // max bit length of the integer coefficients of `polys` DFT polys -> *bits_dev (coef_ws: polys * 16n bytes of device scratch)
 int ntt120_key_max_bits(pgb_module *m, const char *pmat, int polys, char *coef_ws, int *bits_dev);
 // ntt120_gadget.cu
@@ -112,6 +114,11 @@ void key_cache_destroy(pgb_module *m);
 // core.cu: lazily grown device workspace of the host front ends; whether a host pointer is page-locked
 int ensure_ws(pgb_module *m, size_t len);
 bool is_pinned(const void *p);
+// core.cu: the limb-wise external product (vmp per item with matrix stride ggsw_bs, 0 = shared) and its normalisation into res; the
+// input ain is in ggsw_base2k, res_dft / a_dft / tmp (dsize > 1 only) are scratch of the external product's layout
+int external_product_limbwise(pgb_module *m, pgb_vec_znx *res, uint64_t res_bs, uint64_t res_base2k, const pgb_vec_znx *ain, uint64_t ain_bs,
+                              const pgb_vmp_pmat *ggsw, uint64_t ggsw_bs, uint64_t ggsw_base2k, uint64_t dsize, uint64_t B,
+                              pgb_vec_znx_dft *res_dft, pgb_vec_znx_dft *a_dft, void *tmp);
 // api.cu (used by core.cu)
 int vmp_apply_impl(pgb_module *m, pgb_vec_znx_dft *res, const pgb_vec_znx_dft *a, const pgb_vmp_pmat *pmat, uint64_t limb_offset,
                    const pgb_batch *bt);

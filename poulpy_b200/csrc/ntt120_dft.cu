@@ -448,7 +448,7 @@ __global__ void __launch_bounds__(256) ntt120_inv_top8_kernel(TopJobs jb, const 
 // poulpy-cpu-ref/src/reference/ntt120/vec_znx_big.rs:367-446).
 struct FusedArgs {
     const char *a_dft;  uint64_t a_bs;      // R polys (16n B each) per ciphertext
-    const char *pmat;                        // [R][C] polys
+    const char *pmat;   uint64_t pmat_bs;   // [R][C] polys; item b's matrix at pmat + b * pmat_bs (0 = one matrix for the batch)
     const char *small;  uint64_t small_bs;  uint64_t small_limb_stride; int small_size; // i64 limbs added to column 0 (or null)
     char *res;          uint64_t res_bs;    uint64_t res_limb_stride;                    // i64 output, column c at + c*n*8
     int R, C, cols_out;
@@ -554,7 +554,6 @@ template <int L> __global__ void __launch_bounds__(Geo<L>::T, 2) ntt120_fused_ba
     extern __shared__ __align__(16) uint32_t smem[];
     constexpr int n = G::NB;
     const int t = threadIdx.x;
-    const uint32_t *pm = reinterpret_cast<const uint32_t *>(p.pmat);
     const size_t poly = (size_t)4 * n; // u32 words per poly
     const size_t res_ls = p.res_limb_stride / 8, small_ls = p.small_limb_stride / 8;
     const int K = p.K, lsh = p.lsh, w = lsh == 0 ? K : K - lsh;
@@ -569,6 +568,7 @@ template <int L> __global__ void __launch_bounds__(Geo<L>::T, 2) ntt120_fused_ba
         const size_t b = work / p.cols_out;
         if (skip && skip[b]) continue; // handled by the collapsed-key kernel
         const uint32_t *a = reinterpret_cast<const uint32_t *>(p.a_dft + b * p.a_bs);
+        const uint32_t *pm = reinterpret_cast<const uint32_t *>(p.pmat + b * p.pmat_bs);
         long long *res = reinterpret_cast<long long *>(p.res + b * p.res_bs) + (size_t)col * n;
         const long long *small = (p.small && (col == 0 || p.small_all_cols))
                                      ? reinterpret_cast<const long long *>(p.small + b * p.small_bs) + (p.small_all_cols ? (size_t)col * n : 0)
@@ -1116,10 +1116,10 @@ static uint32_t pow2_mod_q(uint64_t e, uint32_t q) {
 int ntt120_fused_back(pgb_module *m, const char *a_dft, uint64_t a_bs, const char *pmat, int R, int C, int cols_out, const char *small,
                       uint64_t small_bs, uint64_t small_limb_stride, int small_size, char *res, uint64_t res_bs, uint64_t res_limb_stride,
                       int res_size, int base2k, int64_t res_offset, int batch, const char *glwe, uint64_t glwe_bs, uint64_t glwe_words,
-                      const int *skip, bool skip_list, bool direct, bool small_all_cols) {
+                      const int *skip, bool skip_list, bool direct, bool small_all_cols, uint64_t pmat_bs) {
     FusedArgs p;
     memset(&p, 0, sizeof p);
-    p.a_dft = a_dft; p.a_bs = a_bs; p.pmat = pmat; p.small = small; p.small_bs = small_bs; p.small_limb_stride = small_limb_stride;
+    p.a_dft = a_dft; p.a_bs = a_bs; p.pmat = pmat; p.pmat_bs = pmat_bs; p.small = small; p.small_bs = small_bs; p.small_limb_stride = small_limb_stride;
     p.small_size = small_size; p.res = res; p.res_bs = res_bs; p.res_limb_stride = res_limb_stride;
     p.R = R; p.C = C; p.cols_out = cols_out;
     p.direct = direct ? 1 : 0; p.small_all_cols = small_all_cols ? 1 : 0;
@@ -1141,7 +1141,7 @@ int ntt120_fused_back(pgb_module *m, const char *a_dft, uint64_t a_bs, const cha
     const int S = p.a_size;
     const uint64_t key_bytes = (uint64_t)R * C * poly_bytes;
     const int *ok = skip;
-    const bool try_collapse = glwe && !skip && !direct && res_offset == 0 && S >= 2 && S <= 32 && (int64_t)batch * cols_out >= 64 && key_bytes <= ((uint64_t)64 << 20) &&
+    const bool try_collapse = glwe && !skip && !direct && pmat_bs == 0 && res_offset == 0 && S >= 2 && S <= 32 && (int64_t)batch * cols_out >= 64 && key_bytes <= ((uint64_t)64 << 20) &&
                               (S - 1) * base2k + 3 < 118 && !opt_on(m, PGB_OPT_NO_COLLAPSE);
     if (try_collapse) {
         // workspace: [collapsed key | key coefficients (i128) | key_bits | ok flags]

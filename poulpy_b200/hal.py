@@ -82,7 +82,7 @@ def lib():
         for name in ("pgb_glwe_keyswitch_tmp_bytes", "pgb_glwe_external_product_tmp_bytes", "pgb_cggi_blind_rotate_tmp_bytes",
                      "pgb_cggi_blind_rotate_standard_tmp_bytes", "pgb_cggi_blind_rotate_extended_tmp_bytes", "pgb_vmp_apply_dft_tmp_bytes", "pgb_glwe_tensor_apply_tmp_bytes",
                      "pgb_glwe_tensor_relinearize_tmp_bytes", "pgb_glwe_automorphism_tmp_bytes", "pgb_glwe_automorphism_add_assign_tmp_bytes",
-                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
+                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_glwe_cmux_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
                      "pgb_vec_znx_big_automorphism_assign_tmp_bytes", "pgb_ggsw_expand_row_tmp_bytes",
                      "pgb_bytes_of_vmp_pmat", "pgb_size_of_scalar_prep", "pgb_size_of_scalar_big"):
             getattr(_lib, name).restype = C.c_size_t
@@ -215,9 +215,13 @@ class ScalarZnx(SvpPPol):
 
 
 class VmpPMat:
-    def __init__(self, buf, n, rows, cols_in, cols_out, size, offset=0):
+    """One matrix, or (batch > 1) `batch` matrices of the same shape laid out batch_stride bytes apart (e.g. one prepared GGSW per
+    ciphertext)."""
+
+    def __init__(self, buf, n, rows, cols_in, cols_out, size, offset=0, batch=1, batch_stride=0):
         self.buf, self.n, self.rows, self.cols_in, self.cols_out, self.size = buf, n, rows, cols_in, cols_out, size
         self.offset = offset
+        self.batch, self.batch_stride = batch, batch_stride
 
     def struct(self):
         return _PM(self.buf.ptr + self.offset, self.n, self.size, self.rows, self.cols_in, self.cols_out)
@@ -292,8 +296,9 @@ class Module:
     def svp_ppol_alloc(self, cols):
         return SvpPPol(self._buf(self.n * cols * self.prep_bytes), self.n, cols)
 
-    def vmp_pmat_alloc(self, rows, cols_in, cols_out, size):
-        return VmpPMat(self._buf(self.n * rows * cols_in * cols_out * size * self.prep_bytes), self.n, rows, cols_in, cols_out, size)
+    def vmp_pmat_alloc(self, rows, cols_in, cols_out, size, batch=1):
+        stride = self.n * rows * cols_in * cols_out * size * self.prep_bytes
+        return VmpPMat(self._buf(stride * batch), self.n, rows, cols_in, cols_out, size, batch=batch, batch_stride=stride if batch > 1 else 0)
 
     def vec_znx_from_numpy(self, arr):
         """arr: int64 (size, cols, n) or (batch, size, cols, n)."""
@@ -447,6 +452,13 @@ class Module:
         ps, ms = pmat.struct(), mat.struct()
         _check(lib().pgb_vmp_prepare(self._h, C.byref(ps), C.byref(ms)))
 
+    def vmp_prepare_batched(self, pmat: VmpPMat, mat: MatZnx):
+        """pgb_vmp_prepare_batched: the pmat.batch matrices of `mat` in one launch (asynchronous: sync() before reading)."""
+        assert pmat.batch == mat.batch, (pmat.batch, mat.batch)
+        ps, ms = pmat.struct(), mat.struct()
+        bt = _BT(pmat.batch, pmat.batch_stride, mat.batch_stride, 0)
+        _check(lib().pgb_vmp_prepare_batched(self._h, C.byref(ps), C.byref(ms), C.byref(bt)))
+
     def vmp_apply_dft_to_dft(self, res, a, pmat: VmpPMat, limb_offset=0):
         r, av, ps = res.struct(), a.struct(), pmat.struct()
         if res.batch > 1:
@@ -529,6 +541,23 @@ class Module:
         _check(lib().pgb_glwe_external_product_batched(self._h, C.byref(r), _u64(res_base2k), C.byref(av), _u64(a_base2k), C.byref(ks),
                                                        _u64(ggsw_base2k), _u64(dsize), C.byref(bt), C.c_void_p(scratch.ptr),
                                                        C.c_size_t(scratch.nbytes)))
+        return scratch
+
+    def glwe_cmux(self, res: VecZnx, t: VecZnx, f: VecZnx, base2k, s: VmpPMat, ggsw_base2k, dsize=1, scratch: DevBuf = None):
+        """CMux of res.batch ciphertexts: res = normalize(normalize(t - f) x s + f).  A batched `s` (a VmpPMat with a batch stride, e.g.
+        from vmp_pmat_alloc(..., batch=B) or circuit.prepare_ggsw) gives ciphertext b the selector at s + b * s.batch_stride; an `s` without
+        one is shared by the batch.  t / f with batch 1 are shared by the batch.  Asynchronous."""
+        assert s.batch_stride == 0 or s.batch >= res.batch, (s.batch, res.batch)
+        ks = s.struct()
+        need = lib().pgb_glwe_cmux_tmp_bytes(self._h, _u64(res.size), _u64(t.size), _u64(f.size), _u64(base2k), C.byref(ks), _u64(ggsw_base2k),
+                                             _u64(dsize), _u64(res.batch))
+        if scratch is None or scratch.nbytes < need:
+            scratch = self._scratch(need)
+        r, tv, fv = res.struct(), t.struct(), f.struct()
+        bt = _BT(res.batch, res.batch_stride, t.batch_stride if t.batch > 1 else 0, f.batch_stride if f.batch > 1 else 0)
+        _check(lib().pgb_glwe_cmux_batched(self._h, C.byref(r), C.byref(tv), C.byref(fv), _u64(base2k), C.byref(ks),
+                                           _u64(s.batch_stride), _u64(ggsw_base2k), _u64(dsize), C.byref(bt),
+                                           C.c_void_p(scratch.ptr), C.c_size_t(scratch.nbytes)))
         return scratch
 
     def gadget_key_pin(self, key: VmpPMat):
