@@ -9,9 +9,6 @@ static inline bool R_ok(uint64_t cols, uint64_t dnum) {
     return R == 1 || R == 2 || R == 3 || R == 4 || R == 6 || R == 8;
 }
 
-static const uint64_t ALIGN = 256;
-static inline uint64_t align_up(uint64_t x) { return (x + ALIGN - 1) / ALIGN * ALIGN; }
-
 // x_pow_a[i] = svp_prepare(X^i), i in [0, 2n)  (cggi/key_prepared.rs:66-75, utils.rs:6-41 with y = 0)
 __global__ void xpow_fill_kernel(long long *buf, uint32_t n) {
     const uint32_t ai = blockIdx.x; // [0, 2n)
@@ -428,11 +425,6 @@ __global__ void __launch_bounds__(256) cggi_xai_ext_fft64_kernel(XaiExtArgs p) {
     a[c + m] = (a[c + m] + pi) - vi[c + m];
 }
 
-static pgb_vec_znx mkv(void *data, uint64_t n, uint64_t cols, uint64_t size) {
-    pgb_vec_znx v = {data, n, cols, size, size};
-    return v;
-}
-
 int cggi_blind_rotate_impl(pgb_module *m, pgb_vec_znx *res, const int64_t *lwe_2n, uint64_t n_lwe, const pgb_vec_znx *lut,
                            const pgb_vmp_pmat *brk, const pgb_svp_ppol *x_pow_a, uint64_t block_size, uint64_t base2k, const pgb_batch *bt,
                            void *scratch, size_t scratch_len) {
@@ -448,18 +440,13 @@ int cggi_blind_rotate_impl(pgb_module *m, pgb_vec_znx *res, const int64_t *lwe_2
         pgb_set_error("cggi_blind_rotate: scratch of %zu bytes < required %zu", scratch_len, need);
         return PGB_ERR_SCRATCH;
     }
-    char *sp = (char *)scratch;
-    auto take = [&](uint64_t bytes) {
-        char *p = sp;
-        sp += align_up(bytes);
-        return (void *)p;
-    };
+    Arena ar = {(char *)scratch, scratch_len, 0};
     const uint64_t acc_bs = n * cols * dnum * pb, vres_bs = n * cols * bsize * pb, xai_bs = n * bsize * pb, big_bs = n * bsize * bb;
-    pgb_vec_znx_dft acc_dft = mkv(take(B * acc_bs), n, cols, dnum);
-    pgb_vec_znx_dft vmp_res = mkv(take(B * vres_bs), n, cols, bsize);
-    pgb_vec_znx_dft acc_add = mkv(take(B * vres_bs), n, cols, bsize);
-    (void)take(B * xai_bs); // vmp_xai of the reference: not materialised (fused)
-    pgb_vec_znx_big acc_big = mkv(take(B * big_bs), n, 1, bsize);
+    pgb_vec_znx_dft acc_dft = mk(ar.take(B * acc_bs), n, cols, dnum);
+    pgb_vec_znx_dft vmp_res = mk(ar.take(B * vres_bs), n, cols, bsize);
+    pgb_vec_znx_dft acc_add = mk(ar.take(B * vres_bs), n, cols, bsize);
+    ar.take(B * xai_bs); // vmp_xai of the reference: not materialised (fused)
+    pgb_vec_znx_big acc_big = mk(ar.take(B * big_bs), n, 1, bsize);
     const uint64_t brk_bytes = pgb_bytes_of_vmp_pmat(m, brk->rows, brk->cols_in, brk->cols_out, brk->size);
     const uint64_t lwe_stride = n_lwe + 1;
 
@@ -621,18 +608,13 @@ extern "C" int pgb_cggi_blind_rotate_extended_batched(pgb_module *m, pgb_vec_znx
         pgb_set_error("cggi_blind_rotate_extended: scratch of %zu bytes < required %zu", scratch_len, need);
         return PGB_ERR_SCRATCH;
     }
-    char *sp = (char *)scratch;
-    auto take = [&](uint64_t bytes) {
-        char *q = sp;
-        sp += align_up(bytes);
-        return (void *)q;
-    };
+    Arena ar = {(char *)scratch, scratch_len, 0};
     const uint64_t acc_item = n * cols * res->size * 8, accd_bs = n * cols * dnum * pb, vres_bs = n * cols * bsize * pb, big_bs = n * bsize * bb;
-    pgb_vec_znx acc = mkv(take(items * acc_item), n, cols, res->size);
-    pgb_vec_znx_dft acc_dft = mkv(take(items * accd_bs), n, cols, dnum);
-    pgb_vec_znx_dft vmp_res = mkv(take(items * vres_bs), n, cols, bsize);
-    pgb_vec_znx_dft acc_add = mkv(take(items * vres_bs), n, cols, bsize);
-    pgb_vec_znx_big acc_big = mkv(take(items * big_bs), n, 1, bsize);
+    pgb_vec_znx acc = mk(ar.take(items * acc_item), n, cols, res->size);
+    pgb_vec_znx_dft acc_dft = mk(ar.take(items * accd_bs), n, cols, dnum);
+    pgb_vec_znx_dft vmp_res = mk(ar.take(items * vres_bs), n, cols, bsize);
+    pgb_vec_znx_dft acc_add = mk(ar.take(items * vres_bs), n, cols, bsize);
+    pgb_vec_znx_big acc_big = mk(ar.take(items * big_bs), n, 1, bsize);
     const uint64_t brk_bytes = pgb_bytes_of_vmp_pmat(m, brk->rows, brk->cols_in, brk->cols_out, brk->size);
     const uint64_t lwe_stride = n_lwe + 1;
     // acc[i].zero(); acc[i][0] = X^{b_hi (+1)} * lut[j] (:159-190)
@@ -789,9 +771,10 @@ extern "C" int pgb_cggi_blind_rotate_standard_batched(pgb_module *m, pgb_vec_znx
         return PGB_ERR_SCRATCH;
     }
     const uint64_t tmp_bs = n * cols * res->size * 8;
-    pgb_vec_znx tmp = mkv(scratch, n, cols, res->size);
-    char *ep_scratch = (char *)scratch + align_up(B * tmp_bs);
-    const size_t ep_len = scratch_len - (size_t)align_up(B * tmp_bs);
+    Arena ar = {(char *)scratch, scratch_len, 0};
+    pgb_vec_znx tmp = mk(ar.take(B * tmp_bs), n, cols, res->size);
+    char *ep_scratch = ar.rest();
+    const size_t ep_len = ar.rest_len();
     const uint64_t brk_bytes = pgb_bytes_of_vmp_pmat(m, brk->rows, brk->cols_in, brk->cols_out, brk->size);
     const uint64_t lwe_stride = n_lwe + 1;
     // out.zero(); out[0] = X^b * LUT (:412-415)

@@ -8,9 +8,6 @@
 // normalise run on the routes described at pgb_glwe_cmux_batched.
 #include "internal.h"
 
-static const uint64_t ALIGN = 256;
-static inline uint64_t align_up(uint64_t x) { return (x + ALIGN - 1) / ALIGN * ALIGN; }
-
 // ---- d = normalize_assign(t - f) -------------------------------------------------------------------------------------------------------
 // One thread per (coefficient, column, ciphertext).  Limb j < size of d is t[j] - f[j] in wrapping i64 (a limb missing from an operand
 // reads as 0), normalised from the last limb up with the carry in a register: the lsh = 0 steps of vec_znx_normalize_assign
@@ -101,7 +98,8 @@ extern "C" size_t pgb_glwe_cmux_tmp_bytes(const pgb_module *m, uint64_t res_size
 }
 
 // Routes (all bit-exact with the five steps; DESIGN.md §3.5b):
-//  * ggsw_stride == 0: d in scratch, then pgb_glwe_external_product_batched (gadget kernels included), add f, normalise.
+//  * ggsw_stride == 0: d in scratch, then pgb_glwe_external_product_batched (with its single-kernel routes, gadget_fused in core.cu),
+//    add f, normalise.
 //  * per-item selectors, dsize == 1, ggsw_base2k == base2k, f.size <= min(res.size, s.size), fusion on:
 //      NTT120 (n = 2^9 .. 2^13): d -> forward transform -> ntt120_fused_back with the per-item matrix stride and small = f on every column;
 //      FFT64 (fft64_fused_back_supported): d and res = f -> forward transform -> vmp with the per-item matrix stride -> fft64_fused_back,
@@ -152,14 +150,14 @@ extern "C" int pgb_glwe_cmux_batched(pgb_module *m, pgb_vec_znx *res, const pgb_
     // ---- step 1 + 2 on every route: d = normalize(t - f), res.size limbs -----------------------------------------------------------------
     const uint64_t S = s->size, rs = res->size;
     const uint64_t d_bs = n * cols * rs * 8;
-    char *sp = (char *)scratch, *rest = sp + align_up(B * d_bs);
-    const size_t rest_len = scratch_len - (size_t)(rest - sp);
-    pgb_vec_znx d = {sp, n, cols, rs, rs};
+    Arena ar = {(char *)scratch, scratch_len, 0};
+    char *sp = (char *)ar.take(B * d_bs);
+    pgb_vec_znx d = mk(sp, n, cols, rs);
 
     if (ggsw_stride == 0) { // one selector for the batch: the external product with every route it has
         PGB_TRY(launch_diff(m, sp, d_bs, rs, t, bt->stride_a, f, bt->stride_b, nullptr, 0, base2k, B));
         pgb_batch bte = {B, bt->stride_res, d_bs, 0};
-        PGB_TRY(pgb_glwe_external_product_batched(m, res, base2k, &d, base2k, s, ggsw_base2k, dsize, &bte, rest, rest_len));
+        PGB_TRY(pgb_glwe_external_product_batched(m, res, base2k, &d, base2k, s, ggsw_base2k, dsize, &bte, ar.rest(), ar.rest_len()));
         return add_f_normalize(m, res, bt->stride_res, f, bt->stride_b, base2k, B);
     }
 
@@ -167,7 +165,7 @@ extern "C" int pgb_glwe_cmux_batched(pgb_module *m, pgb_vec_znx *res, const pgb_
     const uint64_t R = umin64(s->rows * cols, cols * rs); // rows of the vector-matrix product (external_product/glwe.rs:231)
     const uint64_t a_dft_bs = n * cols * rs * pb, res_dft_bs = n * cols * S * pb;
     if (fuse && ntt120_fused_supported(m)) {
-        char *a_dft = rest;
+        char *a_dft = (char *)ar.take(B * a_dft_bs);
         PGB_TRY(launch_diff(m, sp, d_bs, rs, t, bt->stride_a, f, bt->stride_b, nullptr, 0, base2k, B));
         LimbSet in = {sp, n * 8, d_bs}, out = {a_dft, n * pb, a_dft_bs}; // polys (limb, column) are consecutive on both sides
         PGB_TRY(ntt120_forward(m, in, out, (int)(rs * cols), (int)B));
@@ -176,7 +174,7 @@ extern "C" int pgb_glwe_cmux_batched(pgb_module *m, pgb_vec_znx *res, const pgb_
                                  nullptr, 0, 0, nullptr, false, false, true, ggsw_stride);
     }
     if (fuse && fft64_fused_back_supported(m, (int)S)) {
-        char *res_dft = rest, *a_dft = rest + align_up(B * res_dft_bs);
+        char *res_dft = (char *)ar.take(B * res_dft_bs), *a_dft = (char *)ar.take(B * a_dft_bs);
         PGB_TRY(launch_diff(m, sp, d_bs, rs, t, bt->stride_a, f, bt->stride_b, (char *)res->data, bt->stride_res, base2k, B));
         LimbSet in = {sp, n * 8, d_bs}, out = {a_dft, n * pb, a_dft_bs};
         PGB_TRY(fft64_forward(m, in, out, (int)(rs * cols), (int)B));
@@ -187,25 +185,15 @@ extern "C" int pgb_glwe_cmux_batched(pgb_module *m, pgb_vec_znx *res, const pgb_
     }
 
     // ---- limb-wise: the external product's HAL sequence with the per-item matrix stride -----------------------------------------------
-    char *cur = rest;
-    auto take = [&cur](uint64_t bytes) { char *p = cur; cur += align_up(bytes); return p; };
-    pgb_vec_znx_dft res_dft = {take(B * res_dft_bs), n, cols, S, S};
-    pgb_vec_znx ain = d;
-    uint64_t ain_bs = d_bs;
-    if (ggsw_base2k != base2k) {
-        const uint64_t cs = div_ceil64(rs * base2k, ggsw_base2k);
-        ain_bs = n * cols * cs * 8;
-        ain = {take(B * ain_bs), n, cols, cs, cs};
-    }
-    const uint64_t a_dft_max = div_ceil64(ain.size, dsize);
-    pgb_vec_znx_dft a_dft = {take(B * n * cols * a_dft_max * pb), n, cols, a_dft_max, a_dft_max};
-    void *tmp = dsize > 1 ? take(B * res_dft_bs) : nullptr;
-    PGB_REQUIRE((uint64_t)(cur - sp) <= scratch_len, "glwe_cmux: scratch exhausted");
+    pgb_vec_znx_dft res_dft = mk(ar.take(B * res_dft_bs), n, cols, S);
     PGB_TRY(launch_diff(m, sp, d_bs, rs, t, bt->stride_a, f, bt->stride_b, nullptr, 0, base2k, B));
-    if (ggsw_base2k != base2k) { // glwe_normalize of the input into ggsw_base2k, as the external product does
-        pgb_batch btn = {B, ain_bs, d_bs, 0};
-        for (uint64_t c = 0; c < cols; c++) PGB_TRY(big_normalize_impl(m, &ain, ggsw_base2k, 0, c, &d, base2k, c, 0, false, &btn));
-    }
+    pgb_vec_znx ain; // the input in ggsw_base2k, as the external product does
+    uint64_t ain_bs;
+    PGB_TRY(glwe_to_base2k(m, ar, &d, d_bs, base2k, ggsw_base2k, B, &ain, &ain_bs));
+    const uint64_t a_dft_max = div_ceil64(ain.size, dsize);
+    pgb_vec_znx_dft a_dft = mk(ar.take(B * n * cols * a_dft_max * pb), n, cols, a_dft_max);
+    void *tmp = dsize > 1 ? ar.take(B * res_dft_bs) : nullptr;
+    PGB_REQUIRE(res_dft.data && ain.data && a_dft.data && (dsize == 1 || tmp), "glwe_cmux: scratch exhausted");
     PGB_TRY(external_product_limbwise(m, res, bt->stride_res, base2k, &ain, ain_bs, s, ggsw_stride, ggsw_base2k, dsize, B, &res_dft, &a_dft, tmp));
     return add_f_normalize(m, res, bt->stride_res, f, bt->stride_b, base2k, B);
 }

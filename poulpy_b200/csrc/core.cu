@@ -12,33 +12,27 @@
 
 #include "internal.h"
 
-static const uint64_t ALIGN = 256;
-static inline uint64_t align_up(uint64_t x) { return (x + ALIGN - 1) / ALIGN * ALIGN; }
-
-struct Arena {
-    char *base;
-    size_t len, used;
-    void *take(size_t bytes) {
-        size_t off = align_up(used);
-        if (off + bytes > len) return nullptr;
-        used = off + bytes;
-        return base + off;
-    }
-};
-
-static pgb_vec_znx mk(void *data, uint64_t n, uint64_t cols, uint64_t size) {
-    pgb_vec_znx v = {data, n, cols, size, size};
-    return v;
-}
-
 // glwe_normalize (poulpy-core/src/operations/glwe.rs:1286-1310) into a buffer of size ceil(a.size*a_base2k / base2k)
 static uint64_t conv_size(uint64_t a_size, uint64_t a_base2k, uint64_t base2k) { return div_ceil64(a_size * a_base2k, base2k); }
 
-// ---- gglwe_product_dft (keyswitching/glwe.rs:298-380) / the dsize loop of the external product ------------------
+int glwe_to_base2k(pgb_module *m, Arena &ar, const pgb_vec_znx *a, uint64_t a_bs, uint64_t from, uint64_t to, uint64_t B, pgb_vec_znx *out,
+                   uint64_t *out_bs) {
+    *out = *a;
+    *out_bs = a_bs;
+    if (from == to) return PGB_OK;
+    const uint64_t cs = conv_size(a->size, from, to);
+    *out_bs = m->n * a->cols * cs * 8;
+    *out = mk(ar.take(B * *out_bs), m->n, a->cols, cs);
+    pgb_batch btn = {B, *out_bs, a_bs, 0};
+    for (uint64_t i = 0; i < a->cols; i++) PGB_TRY(big_normalize_impl(m, out, to, 0, i, a, from, i, 0, false, &btn));
+    return PGB_OK;
+}
+
+// ---- gglwe_product_dft (keyswitching/glwe.rs:298-380) ---------------------------------------------------------------------------
 // res_dft(cols_out, pmat.size) <- a_dft(cols, a_size) x pmat ; ai / tmp are scratch DFT buffers for dsize > 1.
 static int gadget_product(pgb_module *m, pgb_vec_znx_dft *res, const pgb_vec_znx_dft *a, const pgb_vmp_pmat *pmat, uint64_t dsize,
-                          bool bound_by_dnum, pgb_vec_znx_dft *ai, pgb_vec_znx_dft *tmp, uint64_t res_bs, uint64_t a_bs, uint64_t ai_bs,
-                          uint64_t tmp_bs, uint64_t batch) {
+                          pgb_vec_znx_dft *ai, pgb_vec_znx_dft *tmp, uint64_t res_bs, uint64_t a_bs, uint64_t ai_bs, uint64_t tmp_bs,
+                          uint64_t batch) {
     if (dsize == 1) {
         pgb_batch bt = {batch, res_bs, a_bs, 0};
         return vmp_apply_impl(m, res, a, pmat, 0, &bt);
@@ -46,9 +40,7 @@ static int gadget_product(pgb_module *m, pgb_vec_znx_dft *res, const pgb_vec_znx
     const uint64_t a_size = a->size, dnum = pmat->rows, cols = a->cols, cols_out = res->cols;
     const uint64_t res_max = res->size;
     for (uint64_t di = 0; di < dsize; di++) {
-        uint64_t sz = (a_size + di) / dsize;
-        if (bound_by_dnum) sz = umin64(sz, dnum);
-        ai->size = sz;
+        ai->size = umin64((a_size + di) / dsize, dnum);
         const int64_t cut = (int64_t)(dsize - di) - 2;
         res->size = pmat->size - (uint64_t)(cut > 0 ? cut : 0);
         pgb_batch btc = {batch, ai_bs, a_bs, 0};
@@ -75,6 +67,135 @@ static bool gadget_likely_fits(uint64_t n, uint64_t R, uint64_t S, uint64_t K) {
     uint64_t rn = 0;
     while (((uint64_t)1 << rn) < R * n) rn++;
     return rn + (S - 1) * K + 3 + 2 * K <= 118;
+}
+
+// glwe_keyswitch_internal (keyswitching/glwe.rs:207-239) from the transformed input on: res_dft <- a_dft x key, left in res_dft as a big
+// (ScalarBig elements, same memory).  For dsize > 1 the digit buffer ai and the temporary come from `ar` for this call only, so a caller
+// that runs several products gets the same buffers each time.
+static int keyswitch_core(pgb_module *m, Arena &ar, const char *what, pgb_vec_znx_dft *res_dft, uint64_t res_dft_bs, const pgb_vec_znx_dft *a_dft,
+                          uint64_t a_dft_bs, const pgb_vmp_pmat *key, uint64_t dsize, uint64_t B) {
+    const uint64_t n = m->n, pb = prep_bytes(m);
+    const size_t mark = ar.used;
+    pgb_vec_znx_dft ai = *a_dft, tmp = *res_dft;
+    uint64_t ai_bs = 0, tmp_bs = 0;
+    if (dsize > 1) {
+        const uint64_t ai_max = umin64(div_ceil64(a_dft->size, dsize), key->rows);
+        ai_bs = n * a_dft->cols * ai_max * pb;
+        ai = mk(ar.take(B * ai_bs), n, a_dft->cols, ai_max);
+        tmp_bs = res_dft_bs;
+        tmp = mk(ar.take(B * tmp_bs), n, res_dft->cols, key->size);
+        PGB_REQUIRE(ai.data && tmp.data, "%s: scratch exhausted", what);
+        PGB_CHECK_CUDA(cudaMemsetAsync(ai.data, 0, B * ai_bs, m->stream));   // ai_dft.zero()       (:337)
+        PGB_CHECK_CUDA(cudaMemsetAsync(tmp.data, 0, B * tmp_bs, m->stream)); // res_dft_tmp.zero()  (:342)
+    }
+    ar.used = mark;
+    PGB_CHECK_CUDA(cudaMemsetAsync(res_dft->data, 0, B * res_dft_bs, m->stream)); // res_dft.zero() (:90)
+    PGB_TRY(gadget_product(m, res_dft, a_dft, key, dsize, &ai, &tmp, res_dft_bs, a_dft_bs, ai_bs, tmp_bs, B));
+    pgb_batch btc = {B, res_dft_bs, 0, 0};
+    return pgb_vec_znx_idft_apply_consume_batched(m, res_dft, &btc);
+}
+
+// ---- the single-kernel gadget product ---------------------------------------------------------------------------------------------
+// One product res <- a x key as the gadget kernels (fft64_gadget.cu, ntt120_gadget.cu) see it.  a is in the key's base 2^base2k; rows of
+// the product are the columns row_col0 .. row_col0 + key.cols_in of a (row_col0 = 1 for the key-switch family, whose column 0 is added to
+// output column 0, 0 for the external product).
+struct GadgetJob {
+    const pgb_vec_znx *a;
+    uint64_t a_bs, row_col0;
+    const pgb_vmp_pmat *key;
+    uint64_t dsize, base2k;
+    int small_size;  // limbs of column 0 of a added to the output
+    int group_limit; // bound on the limbs of a digit group (dnum for the key-switch family, 0 = none for the external product)
+    int aut_mode;    // 0: none; 1..3: X -> X^aut_p, then add / sub / sub_negate a (post_size limbs); 4: X -> X^aut_p only
+    int64_t aut_p;
+    int post_size;
+    pgb_vec_znx *res;
+    uint64_t res_bs;
+    int alias; // vec_znx_alias_class(res, a): nonzero when res overlaps a
+    uint64_t B;
+};
+
+// Runs the job on a single-kernel route when one fits: returns 1 when the batch is done, 0 when the caller must run the limb-wise
+// sequence, < 0 on error.  Routes:
+//  * FFT64, dsize <= 2: the gadget kernel, with nothing to check after the launch.
+//  * NTT120, dsize == 1, no automorphism: the gadget kernel, then the ciphertexts it flagged (integers that could leave the collapsed-key
+//    bound) are redone on the device by the forward transform and the fused back end of their skip list: no host round trip.  Without
+//    the gadget kernel, the forward transform into a_dft and the fused back end (vmp -> idft -> CRT -> add_small -> normalize).
+//  * NTT120, dsize > 1 (when gadget_likely_fits) or automorphism: the gadget kernel, then the count of flagged ciphertexts is read back;
+//    any flagged one sends the whole batch to the limb-wise sequence.
+// The output is staged when res overlaps a and the kernel cannot write over a: the automorphism epilogue gathers a at permuted positions,
+// and after a read-back the limb-wise sequence must still find a intact.  The staging buffer is `stage` when given (used only if
+// stage_cap bytes per item hold the output), else taken from `ar`; when none can be had the route is skipped.  ar supplies the flag list.
+static int gadget_fused(pgb_module *m, const GadgetJob &j, Arena &ar, pgb_vec_znx_dft *a_dft, uint64_t a_dft_bs, char *stage_buf,
+                        uint64_t stage_cap) {
+    if (opt_on(m, PGB_OPT_NO_FUSION)) return 0;
+    const pgb_vec_znx &a = *j.a, &res = *j.res;
+    const pgb_vmp_pmat &key = *j.key;
+    const uint64_t n = m->n, B = j.B, row_cols = key.cols_in, cols_out = key.cols_out, key_rows = key.rows * key.cols_in;
+    const uint64_t R = j.dsize == 1 ? umin64(key_rows, row_cols * a.size) : row_cols * a.size;
+    const int C = (int)(cols_out * key.size), S = (int)key.size, K = (int)j.base2k;
+    const bool f64 = j.dsize <= 2 && fft64_gadget_supported(m, (int)R, (int)cols_out, S, K, (int)B);
+    const bool gadget = f64 || ntt120_gadget_supported(m, (int)R, (int)cols_out, S, K, (int)B);
+    const bool plain = j.dsize == 1 && j.aut_mode == 0, skip_list = plain && !f64, read_back = !f64 && !plain;
+    if (!gadget && !(skip_list && ntt120_fused_supported(m))) return 0;
+    if (read_back && j.dsize > 1 && !gadget_likely_fits(n, R, key.size, j.base2k)) return 0;
+    // column 0 of a is the small term of the key-switch family's fused back end
+    const char *small = j.row_col0 ? (const char *)a.data : nullptr;
+    const uint64_t small_bs = j.row_col0 ? j.a_bs : 0, small_ls = j.row_col0 ? a.cols * n * 8 : 0;
+    if (!gadget) {
+        pgb_batch btd = {B, a_dft_bs, j.a_bs, 0};
+        for (uint64_t c = 0; c < row_cols; c++) PGB_TRY(pgb_vec_znx_dft_apply_batched(m, 1, 0, a_dft, c, &a, c + j.row_col0, &btd));
+        PGB_TRY(ntt120_fused_back(m, (const char *)a_dft->data, a_dft_bs, (const char *)key.data, (int)R, C, (int)cols_out, small, small_bs,
+                                  small_ls, j.small_size, (char *)res.data, j.res_bs, res.cols * n * 8, (int)res.size, K, 0, (int)B,
+                                  (const char *)a.data, j.a_bs, n * a.cols * a.size));
+        return 1;
+    }
+    const size_t mark = ar.used;
+    int *ok = (int *)ar.take((2 * B + 1) * sizeof(int)); // flags | count of flagged | their indices
+    const bool stage = j.alias != 0 && (j.aut_mode != 0 || read_back);
+    char *out = (char *)res.data;
+    uint64_t out_bs = j.res_bs;
+    if (stage) {
+        out_bs = n * cols_out * res.size * 8;
+        out = stage_buf ? (out_bs <= stage_cap ? stage_buf : nullptr) : (char *)ar.take(B * out_bs);
+    }
+    if (!ok || !out) {
+        ar.used = mark;
+        return 0;
+    }
+    // a plain dsize-1 product passes no digit-group geometry: its pinned-key signature then does not depend on a.size
+    const int a_size = plain ? 0 : (int)a.size, g_rows = plain ? 0 : (int)key_rows, g_limit = plain ? 0 : j.group_limit;
+    if (f64)
+        PGB_TRY(fft64_gadget_fused(m, (const char *)a.data, j.a_bs, (int)a.cols, (int)row_cols, (int)j.row_col0, (int)R, (const char *)key.data, C,
+                                   (int)cols_out, j.small_size, out, out_bs, (int)res.size, K, (int)B, (int)j.dsize, a_size, g_rows, g_limit,
+                                   j.aut_mode, j.aut_p, j.post_size));
+    else
+        PGB_TRY(ntt120_gadget_fused(m, (const char *)a.data, j.a_bs, (int)a.cols, (int)row_cols, (int)j.row_col0, (int)R, (const char *)key.data, C,
+                                    (int)cols_out, j.small_size, out, out_bs, (int)res.size, K, (int)B, ok, (int)j.dsize, a_size, g_rows, g_limit,
+                                    j.aut_mode, j.aut_p, j.post_size));
+    if (skip_list) {
+        const uint64_t pb = prep_bytes(m);
+        for (uint64_t c = 0; c < row_cols; c++) {
+            LimbSet in = {(char *)a.data + limb_off(n, a.cols, c + j.row_col0, 0, 8), a.cols * n * 8, j.a_bs};
+            LimbSet o = {(char *)a_dft->data + limb_off(n, row_cols, c, 0, pb), row_cols * n * pb, a_dft_bs};
+            PGB_TRY(ntt120_forward_skip(m, in, o, (int)a.size, (int)B, ok, true));
+        }
+        PGB_TRY(ntt120_fused_back(m, (const char *)a_dft->data, a_dft_bs, (const char *)key.data, (int)R, C, (int)cols_out, small, small_bs,
+                                  small_ls, j.small_size, (char *)res.data, j.res_bs, res.cols * n * 8, (int)res.size, K, 0, (int)B, nullptr, 0,
+                                  0, ok, true));
+        return 1;
+    }
+    if (read_back) {
+        int nfail = 0;
+        PGB_CHECK_CUDA(cudaMemcpyAsync(&nfail, ok + B, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
+        PGB_CHECK_CUDA(cudaStreamSynchronize(m->stream));
+        if (nfail != 0) {
+            ar.used = mark;
+            return 0;
+        }
+    }
+    if (stage) PGB_CHECK_CUDA(cudaMemcpy2DAsync(res.data, j.res_bs, out, out_bs, out_bs, B, cudaMemcpyDeviceToDevice, m->stream));
+    return 1;
 }
 
 // ---- key-switch --------------------------------------------------------------------------------------------------------
@@ -123,106 +244,21 @@ extern "C" int pgb_glwe_keyswitch_batched(pgb_module *m, pgb_vec_znx *res, uint6
     const uint64_t res_dft_bs = n * cols_out * key->size * pb;
     pgb_vec_znx_dft res_dft = mk(ar.take(B * res_dft_bs), n, cols_out, key->size);
     // (:92-100) cross-base2k input conversion
-    pgb_vec_znx ain = *a;
-    uint64_t ain_bs = bt->stride_a;
-    if (a_base2k != key_base2k) {
-        const uint64_t cs = conv_size(a->size, a_base2k, key_base2k);
-        ain_bs = n * a->cols * cs * 8;
-        ain = mk(ar.take(B * ain_bs), n, a->cols, cs);
-        pgb_batch btn = {B, ain_bs, bt->stride_a, 0};
-        for (uint64_t i = 0; i < a->cols; i++)
-            PGB_TRY(big_normalize_impl(m, &ain, key_base2k, 0, i, a, a_base2k, i, 0, false, &btn));
-    }
+    pgb_vec_znx ain;
+    uint64_t ain_bs;
+    PGB_TRY(glwe_to_base2k(m, ar, a, bt->stride_a, a_base2k, key_base2k, B, &ain, &ain_bs));
     // glwe_keyswitch_internal (:207-239)
     const uint64_t a_dft_bs = n * rank_in * ain.size * pb;
     pgb_vec_znx_dft a_dft = mk(ar.take(B * a_dft_bs), n, rank_in, ain.size);
+    if (res_base2k == key_base2k) { // one kernel per batch; in place, its output is staged in the res_dft block, still unused here
+        const GadgetJob job = {&ain, ain_bs, 1, key, dsize, key_base2k, (int)umin64(ain.size, key->size), (int)key->rows, 0, 0, 0,
+                               res, bt->stride_res, alias, B};
+        const int done = gadget_fused(m, job, ar, &a_dft, a_dft_bs, (char *)res_dft.data, res_dft_bs);
+        if (done) return done < 0 ? done : PGB_OK;
+    }
     pgb_batch btd = {B, a_dft_bs, ain_bs, 0};
-    if (dsize == 1 && res_base2k == key_base2k && m->flavour == PGB_FFT64 && !opt_on(m, PGB_OPT_NO_FUSION)) {
-        const uint64_t R = umin64(key->rows * key->cols_in, rank_in * ain.size);
-        if (fft64_gadget_supported(m, (int)R, (int)cols_out, (int)key->size, (int)key_base2k, (int)B)) // one kernel per batch (fft64_gadget.cu)
-            return fft64_gadget_fused(m, (const char *)ain.data, ain_bs, (int)ain.cols, (int)rank_in, 1, (int)R, (const char *)key->data,
-                                      (int)(cols_out * key->size), (int)cols_out, (int)umin64(ain.size, key->size), (char *)res->data,
-                                      bt->stride_res, (int)res->size, (int)key_base2k, (int)B);
-    }
-    if (dsize == 1 && res_base2k == key_base2k && ntt120_fused_supported(m) && !opt_on(m, PGB_OPT_NO_FUSION)) {
-        const uint64_t R = umin64(key->rows * key->cols_in, rank_in * ain.size);
-        const int small_size = (int)umin64(ain.size, key->size);
-        if (ntt120_gadget_supported(m, (int)R, (int)cols_out, (int)key->size, (int)key_base2k, (int)B)) {
-            // one kernel per batch: i64 in -> i64 out (ntt120_gadget.cu); ciphertexts whose integers could leave the collapsed-key
-            // bound are flagged in `ok` and redone by the per-limb kernels below (normally none)
-            int *ok = (int *)ar.take((2 * B + 1) * sizeof(int)); // flags | count of flagged | their indices
-            PGB_REQUIRE(ok != nullptr, "glwe_keyswitch: scratch exhausted");
-            PGB_TRY(ntt120_gadget_fused(m, (const char *)ain.data, ain_bs, (int)ain.cols, (int)rank_in, 1, (int)R, (const char *)key->data,
-                                        (int)(cols_out * key->size), (int)cols_out, small_size, (char *)res->data, bt->stride_res,
-                                        (int)res->size, (int)key_base2k, (int)B, ok));
-            for (uint64_t c = 0; c < rank_in; c++) {
-                LimbSet in = {(char *)ain.data + limb_off(n, ain.cols, c + 1, 0, 8), ain.cols * n * 8, ain_bs};
-                LimbSet out = {(char *)a_dft.data + limb_off(n, rank_in, c, 0, pb), rank_in * n * pb, a_dft_bs};
-                PGB_TRY(ntt120_forward_skip(m, in, out, (int)ain.size, (int)B, ok, true));
-            }
-            return ntt120_fused_back(m, (const char *)a_dft.data, a_dft_bs, (const char *)key->data, (int)R, (int)(cols_out * key->size),
-                                     (int)cols_out, (const char *)ain.data, ain_bs, ain.cols * n * 8, small_size, (char *)res->data,
-                                     bt->stride_res, res->cols * n * 8, (int)res->size, (int)key_base2k, 0, (int)B, nullptr, 0, 0, ok, true);
-        }
-        // fused back end: vmp -> idft -> CRT -> add_small -> normalize per (ciphertext, column), nothing but a_dft touches HBM
-        for (uint64_t c = 0; c < rank_in; c++) PGB_TRY(pgb_vec_znx_dft_apply_batched(m, 1, 0, &a_dft, c, &ain, c + 1, &btd));
-        return ntt120_fused_back(m, (const char *)a_dft.data, a_dft_bs, (const char *)key->data, (int)R, (int)(cols_out * key->size),
-                                 (int)cols_out, (const char *)ain.data, ain_bs, ain.cols * n * 8, small_size,
-                                 (char *)res->data, bt->stride_res, res->cols * n * 8, (int)res->size, (int)key_base2k, 0, (int)B,
-                                 (const char *)ain.data, ain_bs, n * ain.cols * ain.size);
-    }
-    if (dsize == 2 && res_base2k == key_base2k && m->flavour == PGB_FFT64 && !opt_on(m, PGB_OPT_NO_FUSION) && rank_in * ain.size <= 16 &&
-        fft64_gadget_supported(m, (int)(rank_in * ain.size), (int)cols_out, (int)key->size, (int)key_base2k, (int)B))
-        return fft64_gadget_fused(m, (const char *)ain.data, ain_bs, (int)ain.cols, (int)rank_in, 1, (int)(rank_in * ain.size), (const char *)key->data,
-                                  (int)(cols_out * key->size), (int)cols_out, (int)umin64(ain.size, key->size), (char *)res->data, bt->stride_res,
-                                  (int)res->size, (int)key_base2k, (int)B, 2, (int)ain.size, (int)(key->rows * key->cols_in), (int)key->rows);
-    if (dsize > 1 && res_base2k == key_base2k && m->flavour == PGB_NTT120 && !opt_on(m, PGB_OPT_NO_FUSION) &&
-        ntt120_gadget_supported(m, (int)(rank_in * ain.size), (int)cols_out, (int)key->size, (int)key_base2k, (int)B) &&
-        gadget_likely_fits(n, rank_in * ain.size, key->size, key_base2k)) {
-        // digit groups folded into the collapsed key (ntt120_gadget_fused): same single kernel as dsize == 1.  The per-limb fallback for
-        // flagged ciphertexts is the generic sequence below, so the count of flagged ones is read back (one 4-byte copy + sync).
-        // In place (res == a) the kernel's output is staged in the (otherwise unused) res_dft block: a flagged ciphertext sends the WHOLE
-        // batch to the limb-wise sequence below, which must still find the inputs intact.  An in-place call whose staging does not fit
-        // there takes the limb-wise sequence directly.
-        const uint64_t stage_bs = n * cols_out * res->size * 8;
-        const bool stage = alias == 1;
-        if (!stage || stage_bs <= res_dft_bs) {
-            const size_t mark = ar.used;
-            int *ok = (int *)ar.take((2 * B + 1) * sizeof(int));
-            PGB_REQUIRE(ok != nullptr, "glwe_keyswitch: scratch exhausted");
-            char *out = stage ? (char *)res_dft.data : (char *)res->data;
-            const uint64_t out_bs = stage ? stage_bs : bt->stride_res;
-            PGB_TRY(ntt120_gadget_fused(m, (const char *)ain.data, ain_bs, (int)ain.cols, (int)rank_in, 1, (int)(rank_in * ain.size), (const char *)key->data,
-                                        (int)(cols_out * key->size), (int)cols_out, (int)umin64(ain.size, key->size), out, out_bs,
-                                        (int)res->size, (int)key_base2k, (int)B, ok, (int)dsize, (int)ain.size, (int)(key->rows * key->cols_in),
-                                        (int)key->rows));
-            int nfail = 0;
-            PGB_CHECK_CUDA(cudaMemcpyAsync(&nfail, ok + B, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
-            PGB_CHECK_CUDA(cudaStreamSynchronize(m->stream));
-            if (nfail == 0) {
-                if (stage) PGB_CHECK_CUDA(cudaMemcpy2DAsync(res->data, bt->stride_res, out, out_bs, out_bs, B, cudaMemcpyDeviceToDevice, m->stream));
-                return PGB_OK;
-            }
-            ar.used = mark; // some integers could leave the collapsed-key bound: redo the batch limb by limb
-        }
-    }
     for (uint64_t c = 0; c < rank_in; c++) PGB_TRY(pgb_vec_znx_dft_apply_batched(m, 1, 0, &a_dft, c, &ain, c + 1, &btd));
-    pgb_vec_znx_dft ai = a_dft, tmp = res_dft;
-    uint64_t ai_bs = 0, tmp_bs = 0;
-    if (dsize > 1) {
-        const uint64_t ai_max = umin64(div_ceil64(ain.size, dsize), key->rows);
-        ai_bs = n * rank_in * ai_max * pb;
-        ai = mk(ar.take(B * ai_bs), n, rank_in, ai_max);
-        tmp_bs = res_dft_bs;
-        tmp = mk(ar.take(B * tmp_bs), n, cols_out, key->size);
-        PGB_REQUIRE(ai.data && tmp.data, "glwe_keyswitch: scratch exhausted");
-        PGB_CHECK_CUDA(cudaMemsetAsync(ai.data, 0, B * ai_bs, m->stream));   // ai_dft.zero()       (:337)
-        PGB_CHECK_CUDA(cudaMemsetAsync(tmp.data, 0, B * tmp_bs, m->stream)); // res_dft_tmp.zero()  (:342)
-    }
-    PGB_CHECK_CUDA(cudaMemsetAsync(res_dft.data, 0, B * res_dft_bs, m->stream)); // res_dft.zero() (:90)
-    PGB_TRY(gadget_product(m, &res_dft, &a_dft, key, dsize, true, &ai, &tmp, res_dft_bs, a_dft_bs, ai_bs, tmp_bs, B));
-    pgb_batch btc = {B, res_dft_bs, 0, 0};
-    PGB_TRY(pgb_vec_znx_idft_apply_consume_batched(m, &res_dft, &btc));
+    PGB_TRY(keyswitch_core(m, ar, "glwe_keyswitch", &res_dft, res_dft_bs, &a_dft, a_dft_bs, key, dsize, B));
     pgb_vec_znx_big res_big = res_dft; // same memory, ScalarBig elements
     pgb_batch bts = {B, res_dft_bs, ain_bs, 0};
     PGB_TRY(big_add_small_impl(m, &res_big, 0, &ain, 0, &bts));
@@ -272,84 +308,17 @@ extern "C" int pgb_glwe_external_product_batched(pgb_module *m, pgb_vec_znx *res
     Arena ar = {(char *)scratch, scratch_len, 0};
     const uint64_t res_dft_bs = n * cols * ggsw->size * pb;
     pgb_vec_znx_dft res_dft = mk(ar.take(B * res_dft_bs), n, cols, ggsw->size);
-    pgb_vec_znx ain = *a;
-    uint64_t ain_bs = bt->stride_a;
-    if (a_base2k != ggsw_base2k) {
-        const uint64_t cs = conv_size(a->size, a_base2k, ggsw_base2k);
-        ain_bs = n * a->cols * cs * 8;
-        ain = mk(ar.take(B * ain_bs), n, a->cols, cs);
-        pgb_batch btn = {B, ain_bs, bt->stride_a, 0};
-        for (uint64_t i = 0; i < a->cols; i++)
-            PGB_TRY(big_normalize_impl(m, &ain, ggsw_base2k, 0, i, a, a_base2k, i, 0, false, &btn));
-    }
+    pgb_vec_znx ain;
+    uint64_t ain_bs;
+    PGB_TRY(glwe_to_base2k(m, ar, a, bt->stride_a, a_base2k, ggsw_base2k, B, &ain, &ain_bs));
     // glwe_external_product_internal (:197-271)
-    const uint64_t a_size = ain.size;
-    const uint64_t a_dft_max = dsize == 1 ? a_size : div_ceil64(a_size, dsize);
+    const uint64_t a_dft_max = div_ceil64(ain.size, dsize);
     const uint64_t a_dft_bs = n * cols * a_dft_max * pb;
     pgb_vec_znx_dft a_dft = mk(ar.take(B * a_dft_bs), n, cols, a_dft_max);
-    if (dsize == 1) {
-        pgb_batch btd = {B, a_dft_bs, ain_bs, 0};
-        if (res_base2k == ggsw_base2k && m->flavour == PGB_FFT64 && !opt_on(m, PGB_OPT_NO_FUSION)) {
-            const uint64_t R = umin64(ggsw->rows * ggsw->cols_in, cols * a_size);
-            if (fft64_gadget_supported(m, (int)R, (int)cols, (int)ggsw->size, (int)ggsw_base2k, (int)B)) // fft64_gadget.cu
-                return fft64_gadget_fused(m, (const char *)ain.data, ain_bs, (int)ain.cols, (int)cols, 0, (int)R, (const char *)ggsw->data,
-                                          (int)(cols * ggsw->size), (int)cols, 0, (char *)res->data, bt->stride_res, (int)res->size,
-                                          (int)ggsw_base2k, (int)B);
-        }
-        if (res_base2k == ggsw_base2k && ntt120_fused_supported(m) && !opt_on(m, PGB_OPT_NO_FUSION)) {
-            const uint64_t R = umin64(ggsw->rows * ggsw->cols_in, cols * a_size);
-            if (ntt120_gadget_supported(m, (int)R, (int)cols, (int)ggsw->size, (int)ggsw_base2k, (int)B)) {
-                int *ok = (int *)ar.take((2 * B + 1) * sizeof(int)); // flags | count of flagged | their indices
-                PGB_REQUIRE(ok != nullptr, "glwe_external_product: scratch exhausted");
-                PGB_TRY(ntt120_gadget_fused(m, (const char *)ain.data, ain_bs, (int)ain.cols, (int)cols, 0, (int)R, (const char *)ggsw->data,
-                                            (int)(cols * ggsw->size), (int)cols, 0, (char *)res->data, bt->stride_res, (int)res->size,
-                                            (int)ggsw_base2k, (int)B, ok));
-                for (uint64_t j = 0; j < cols; j++) {
-                    LimbSet in = {(char *)ain.data + limb_off(n, ain.cols, j, 0, 8), ain.cols * n * 8, ain_bs};
-                    LimbSet out = {(char *)a_dft.data + limb_off(n, cols, j, 0, pb), cols * n * pb, a_dft_bs};
-                    PGB_TRY(ntt120_forward_skip(m, in, out, (int)a_size, (int)B, ok, true));
-                }
-                return ntt120_fused_back(m, (const char *)a_dft.data, a_dft_bs, (const char *)ggsw->data, (int)R, (int)(cols * ggsw->size),
-                                         (int)cols, nullptr, 0, 0, 0, (char *)res->data, bt->stride_res, res->cols * n * 8, (int)res->size,
-                                         (int)ggsw_base2k, 0, (int)B, nullptr, 0, 0, ok, true);
-            }
-            for (uint64_t j = 0; j < cols; j++) PGB_TRY(pgb_vec_znx_dft_apply_batched(m, 1, 0, &a_dft, j, &ain, j, &btd));
-            return ntt120_fused_back(m, (const char *)a_dft.data, a_dft_bs, (const char *)ggsw->data, (int)R, (int)(cols * ggsw->size),
-                                     (int)cols, nullptr, 0, 0, 0, (char *)res->data, bt->stride_res, res->cols * n * 8, (int)res->size,
-                                     (int)ggsw_base2k, 0, (int)B, (const char *)ain.data, ain_bs, n * ain.cols * ain.size);
-        }
-    } else {
-        if (dsize == 2 && res_base2k == ggsw_base2k && m->flavour == PGB_FFT64 && !opt_on(m, PGB_OPT_NO_FUSION) && cols * a_size <= 16 &&
-            fft64_gadget_supported(m, (int)(cols * a_size), (int)cols, (int)ggsw->size, (int)ggsw_base2k, (int)B))
-            return fft64_gadget_fused(m, (const char *)ain.data, ain_bs, (int)ain.cols, (int)cols, 0, (int)(cols * a_size), (const char *)ggsw->data,
-                                      (int)(cols * ggsw->size), (int)cols, 0, (char *)res->data, bt->stride_res, (int)res->size, (int)ggsw_base2k,
-                                      (int)B, 2, (int)a_size, (int)(ggsw->rows * ggsw->cols_in), 0);
-        if (res_base2k == ggsw_base2k && m->flavour == PGB_NTT120 && !opt_on(m, PGB_OPT_NO_FUSION) &&
-            ntt120_gadget_supported(m, (int)(cols * a_size), (int)cols, (int)ggsw->size, (int)ggsw_base2k, (int)B) &&
-            gadget_likely_fits(n, cols * a_size, ggsw->size, ggsw_base2k)) {
-            // digit groups folded into the collapsed key, as in the key-switch; no bound on the limbs of a group here (:233).  In place the
-            // output is staged in the unused res_dft block so that a flagged ciphertext can still redo the batch from intact inputs.
-            const uint64_t stage_bs = n * cols * res->size * 8;
-            const bool stage = alias == 1;
-            if (!stage || stage_bs <= res_dft_bs) {
-                const size_t mark = ar.used;
-                int *ok = (int *)ar.take((2 * B + 1) * sizeof(int));
-                PGB_REQUIRE(ok != nullptr, "glwe_external_product: scratch exhausted");
-                char *out = stage ? (char *)res_dft.data : (char *)res->data;
-                const uint64_t out_bs = stage ? stage_bs : bt->stride_res;
-                PGB_TRY(ntt120_gadget_fused(m, (const char *)ain.data, ain_bs, (int)ain.cols, (int)cols, 0, (int)(cols * a_size), (const char *)ggsw->data,
-                                            (int)(cols * ggsw->size), (int)cols, 0, out, out_bs, (int)res->size, (int)ggsw_base2k,
-                                            (int)B, ok, (int)dsize, (int)a_size, (int)(ggsw->rows * ggsw->cols_in), 0));
-                int nfail = 0;
-                PGB_CHECK_CUDA(cudaMemcpyAsync(&nfail, ok + B, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
-                PGB_CHECK_CUDA(cudaStreamSynchronize(m->stream));
-                if (nfail == 0) {
-                    if (stage) PGB_CHECK_CUDA(cudaMemcpy2DAsync(res->data, bt->stride_res, out, out_bs, out_bs, B, cudaMemcpyDeviceToDevice, m->stream));
-                    return PGB_OK;
-                }
-                ar.used = mark; // redo the batch limb by limb
-            }
-        }
+    if (res_base2k == ggsw_base2k) { // as in the key-switch; no bound on the limbs of a digit group here (:233)
+        const GadgetJob job = {&ain, ain_bs, 0, ggsw, dsize, ggsw_base2k, 0, 0, 0, 0, 0, res, bt->stride_res, alias, B};
+        const int done = gadget_fused(m, job, ar, &a_dft, a_dft_bs, (char *)res_dft.data, res_dft_bs);
+        if (done) return done < 0 ? done : PGB_OK;
     }
     void *tmp = nullptr;
     if (dsize > 1) {
@@ -544,22 +513,7 @@ extern "C" int pgb_glwe_tensor_relinearize_batched(pgb_module *m, pgb_vec_znx *r
             PGB_TRY(pgb_vec_znx_dft_apply_batched(m, 1, 0, &a_dft, i, a, cols + i, &btd));
         }
     }
-    pgb_vec_znx_dft ai = a_dft, tmp = res_dft;
-    uint64_t ai_bs = 0, tmp_bs = 0;
-    if (dsize > 1) {
-        const uint64_t ai_max = umin64(div_ceil64(a_dft_size, dsize), tsk->rows);
-        ai_bs = n * pairs * ai_max * pb;
-        ai = mk(ar.take(B * ai_bs), n, pairs, ai_max);
-        tmp_bs = res_dft_bs;
-        tmp = mk(ar.take(B * tmp_bs), n, cols, tsk->size);
-        PGB_REQUIRE(ai.data && tmp.data, "glwe_tensor_relinearize: scratch exhausted");
-        PGB_CHECK_CUDA(cudaMemsetAsync(ai.data, 0, B * ai_bs, m->stream));
-        PGB_CHECK_CUDA(cudaMemsetAsync(tmp.data, 0, B * tmp_bs, m->stream));
-    }
-    PGB_CHECK_CUDA(cudaMemsetAsync(res_dft.data, 0, B * res_dft_bs, m->stream));
-    PGB_TRY(gadget_product(m, &res_dft, &a_dft, tsk, dsize, true, &ai, &tmp, res_dft_bs, a_dft_bs, ai_bs, tmp_bs, B)); // :593
-    pgb_batch btc = {B, res_dft_bs, 0, 0};
-    PGB_TRY(pgb_vec_znx_idft_apply_consume_batched(m, &res_dft, &btc));
+    PGB_TRY(keyswitch_core(m, ar, "glwe_tensor_relinearize", &res_dft, res_dft_bs, &a_dft, a_dft_bs, tsk, dsize, B)); // :593
     pgb_vec_znx_big res_big = res_dft;
     for (uint64_t i = 0; i < cols; i++) { // :596-606 (sic: the reference tests res_base2k == key_base2k)
         if (res_base2k == key_base2k) {
@@ -577,56 +531,15 @@ extern "C" int pgb_glwe_tensor_relinearize_batched(pgb_module *m, pgb_vec_znx *r
     return PGB_OK;
 }
 
-// Single-kernel route of the automorphism family (ntt120_gadget.cu / fft64_gadget.cu, automorphism epilogue): key-switch, X -> X^p and
-// the addition / subtraction of the input in one launch per batch.  aut_mode 1..3 = op 0..2 of pgb_glwe_automorphism_op_batched, 4 = plain
-// glwe_automorphism.  Returns 1 when the batch was finished here, 0 when the caller must run the limb-wise sequence (unsupported geometry
-// or a ciphertext flagged by the collapsed-key bound), < 0 on error.  `ar` supplies the flag list and, when res overlaps a, the staging
-// buffer of the outputs (the epilogue gathers column 0 of a at permuted positions, so it cannot run in place).
+// The automorphism family on the single-kernel route (gadget_fused with the kernels' automorphism epilogue): key-switch, X -> X^p and the
+// addition / subtraction of the input in one launch per batch.  aut_mode 1..3 = op 0..2 of pgb_glwe_automorphism_op_batched, 4 = plain
+// glwe_automorphism.  Returns as gadget_fused; `ar` supplies the flag list and, when res overlaps a, the staging buffer of the outputs.
 static int automorphism_fused(pgb_module *m, int aut_mode, pgb_vec_znx *res, uint64_t res_bs, const pgb_vec_znx *a, uint64_t a_bs,
                               const pgb_vmp_pmat *key, uint64_t base2k, int64_t p, uint64_t dsize, uint64_t B, Arena &ar) {
-    if (opt_on(m, PGB_OPT_NO_FUSION)) return 0;
-    const uint64_t n = m->n, rank_in = key->cols_in, cols = key->cols_out;
-    const uint64_t Rfull = rank_in * a->size, R = dsize == 1 ? umin64(key->rows * key->cols_in, Rfull) : Rfull;
-    const bool f64 = m->flavour == PGB_FFT64;
-    if (f64) {
-        if (dsize > 2 || R > 16 || !fft64_gadget_supported(m, (int)R, (int)cols, (int)key->size, (int)base2k, (int)B)) return 0;
-    } else {
-        if (!ntt120_fused_supported(m) || !ntt120_gadget_supported(m, (int)R, (int)cols, (int)key->size, (int)base2k, (int)B)) return 0;
-        if (dsize > 1 && !gadget_likely_fits(n, R, key->size, base2k)) return 0;
-    }
-    const size_t mark = ar.used;
-    int *ok = (int *)ar.take((2 * B + 1) * sizeof(int));
-    const char *r0 = (const char *)res->data, *r1 = r0 + (B - 1) * res_bs + n * cols * res->size * 8;
-    const char *a0 = (const char *)a->data, *a1 = a0 + (B - 1) * a_bs + n * a->cols * a->size * 8;
-    const bool aliased = r0 < a1 && a0 < r1;
-    char *out = (char *)res->data;
-    uint64_t out_bs = res_bs;
-    if (aliased) {
-        out_bs = n * cols * res->size * 8;
-        out = (char *)ar.take(B * out_bs);
-    }
-    if (!ok || !out) {
-        ar.used = mark;
-        return 0;
-    }
     const int small = (int)umin64(a->size, key->size);
-    if (f64) { // no bound to check in this flavour: the kernel restates the f64 pipeline itself
-        PGB_TRY(fft64_gadget_fused(m, (const char *)a->data, a_bs, (int)a->cols, (int)rank_in, 1, (int)R, (const char *)key->data,
-                                   (int)(cols * key->size), (int)cols, small, out, out_bs, (int)res->size, (int)base2k, (int)B, (int)dsize,
-                                   (int)a->size, (int)(key->rows * key->cols_in), (int)key->rows, aut_mode, p, aut_mode == 4 ? 0 : small));
-        if (aliased) PGB_CHECK_CUDA(cudaMemcpy2DAsync(res->data, res_bs, out, out_bs, out_bs, B, cudaMemcpyDeviceToDevice, m->stream));
-        return 1;
-    }
-    PGB_TRY(ntt120_gadget_fused(m, (const char *)a->data, a_bs, (int)a->cols, (int)rank_in, 1, (int)R, (const char *)key->data,
-                                (int)(cols * key->size), (int)cols, small, out, out_bs, (int)res->size, (int)base2k, (int)B, ok, (int)dsize,
-                                (int)a->size, (int)(key->rows * key->cols_in), (int)key->rows, aut_mode, p, aut_mode == 4 ? 0 : small));
-    int nfail = 0;
-    PGB_CHECK_CUDA(cudaMemcpyAsync(&nfail, ok + B, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
-    PGB_CHECK_CUDA(cudaStreamSynchronize(m->stream));
-    if (nfail == 0 && aliased)
-        PGB_CHECK_CUDA(cudaMemcpy2DAsync(res->data, res_bs, out, out_bs, out_bs, B, cudaMemcpyDeviceToDevice, m->stream));
-    if (nfail != 0) ar.used = mark;
-    return nfail == 0 ? 1 : 0;
+    const GadgetJob job = {a, a_bs, 1, key, dsize, base2k, small, (int)key->rows, aut_mode, p, aut_mode == 4 ? 0 : small, res, res_bs,
+                           vec_znx_alias_class(res, res_bs, a, a_bs, B), B};
+    return gadget_fused(m, job, ar, nullptr, 0, nullptr, 0);
 }
 
 // ---- glwe_automorphism (poulpy-core/src/automorphism/glwe_ct.rs:51-72; SURVEY 8f N4): key-switch with the automorphism key, then
@@ -647,17 +560,15 @@ extern "C" int pgb_glwe_automorphism_batched(pgb_module *m, pgb_vec_znx *res, ui
         return PGB_ERR_SCRATCH;
     }
     const uint64_t n = m->n, B = bt->count, tmp_bs = n * res->cols * res->size * 8;
+    Arena ar = {(char *)scratch, scratch_len, 0};
     if (res_base2k == key_base2k && a_base2k == key_base2k && a->cols == key->cols_in + 1) {
-        Arena ar = {(char *)scratch, scratch_len, 0};
         const int done = automorphism_fused(m, 4, res, bt->stride_res, a, bt->stride_a, key, key_base2k, p, dsize, B, ar);
         if (done < 0) return done;
         if (done) return PGB_OK;
     }
-    pgb_vec_znx tmp = mk(scratch, n, res->cols, res->size);
-    char *ks_scratch = (char *)scratch + align_up(B * tmp_bs);
+    pgb_vec_znx tmp = mk(ar.take(B * tmp_bs), n, res->cols, res->size);
     pgb_batch btk = {B, tmp_bs, bt->stride_a, 0};
-    PGB_TRY(pgb_glwe_keyswitch_batched(m, &tmp, res_base2k, a, a_base2k, key, key_base2k, dsize, &btk, ks_scratch,
-                                       scratch_len - (size_t)align_up(B * tmp_bs)));
+    PGB_TRY(pgb_glwe_keyswitch_batched(m, &tmp, res_base2k, a, a_base2k, key, key_base2k, dsize, &btk, ar.rest(), ar.rest_len()));
     pgb_batch bta = {B, bt->stride_res, tmp_bs, 0};
     for (uint64_t i = 0; i < res->cols; i++) PGB_TRY(pgb_vec_znx_automorphism_batched(m, p, res, i, &tmp, i, &bta));
     return PGB_OK;
@@ -717,36 +628,15 @@ extern "C" int pgb_glwe_automorphism_op_batched(pgb_module *m, int op, pgb_vec_z
     const uint64_t res_dft_bs = n * cols * key->size * pb, big2_bs = n * cols * key->size * bb;
     pgb_vec_znx_dft res_dft = mk(ar.take(B * res_dft_bs), n, cols, key->size);
     pgb_vec_znx_big big2 = mk(ar.take(B * big2_bs), n, cols, key->size);
-    pgb_vec_znx ain = *a;
-    uint64_t ain_bs = bt->stride_a;
-    if (res_base2k != key_base2k) { // (:161-168) res_conv = glwe_normalize(res) at the key's base2k
-        const uint64_t cs = conv_size(res->size, res_base2k, key_base2k);
-        ain_bs = n * res->cols * cs * 8;
-        ain = mk(ar.take(B * ain_bs), n, res->cols, cs);
-        pgb_batch btn = {B, ain_bs, bt->stride_a, 0};
-        for (uint64_t i = 0; i < res->cols; i++) PGB_TRY(big_normalize_impl(m, &ain, key_base2k, 0, i, a, res_base2k, i, 0, false, &btn));
-    }
+    pgb_vec_znx ain; // (:161-168) res_conv = glwe_normalize(res) at the key's base2k
+    uint64_t ain_bs;
+    PGB_TRY(glwe_to_base2k(m, ar, a, bt->stride_a, res_base2k, key_base2k, B, &ain, &ain_bs));
     // glwe_keyswitch_internal (keyswitching/glwe.rs:207-239)
     const uint64_t a_dft_bs = n * rank_in * ain.size * pb;
     pgb_vec_znx_dft a_dft = mk(ar.take(B * a_dft_bs), n, rank_in, ain.size);
     pgb_batch btd = {B, a_dft_bs, ain_bs, 0};
     for (uint64_t c = 0; c < rank_in; c++) PGB_TRY(pgb_vec_znx_dft_apply_batched(m, 1, 0, &a_dft, c, &ain, c + 1, &btd));
-    pgb_vec_znx_dft ai = a_dft, tmp = res_dft;
-    uint64_t ai_bs = 0, tmp_bs = 0;
-    if (dsize > 1) {
-        const uint64_t ai_max = umin64(div_ceil64(ain.size, dsize), key->rows);
-        ai_bs = n * rank_in * ai_max * pb;
-        ai = mk(ar.take(B * ai_bs), n, rank_in, ai_max);
-        tmp_bs = res_dft_bs;
-        tmp = mk(ar.take(B * tmp_bs), n, cols, key->size);
-        PGB_REQUIRE(ai.data && tmp.data, "glwe_automorphism_op: scratch exhausted");
-        PGB_CHECK_CUDA(cudaMemsetAsync(ai.data, 0, B * ai_bs, m->stream));
-        PGB_CHECK_CUDA(cudaMemsetAsync(tmp.data, 0, B * tmp_bs, m->stream));
-    }
-    PGB_CHECK_CUDA(cudaMemsetAsync(res_dft.data, 0, B * res_dft_bs, m->stream));
-    PGB_TRY(gadget_product(m, &res_dft, &a_dft, key, dsize, true, &ai, &tmp, res_dft_bs, a_dft_bs, ai_bs, tmp_bs, B));
-    pgb_batch btc = {B, res_dft_bs, 0, 0};
-    PGB_TRY(pgb_vec_znx_idft_apply_consume_batched(m, &res_dft, &btc));
+    PGB_TRY(keyswitch_core(m, ar, "glwe_automorphism_op", &res_dft, res_dft_bs, &a_dft, a_dft_bs, key, dsize, B));
     pgb_vec_znx_big res_big = res_dft;
     pgb_batch bts = {B, res_dft_bs, ain_bs, 0};
     PGB_TRY(big_add_small_impl(m, &res_big, 0, &ain, 0, &bts));
@@ -796,25 +686,16 @@ extern "C" int pgb_glwe_trace_assign_batched(pgb_module *m, pgb_vec_znx *res, ui
         return PGB_ERR_SCRATCH;
     }
     const uint64_t n = m->n, B = bt->count;
-    pgb_vec_znx cur = *res;
-    uint64_t cur_bs = bt->stride_res;
-    char *sc = (char *)scratch;
-    size_t sc_len = scratch_len;
-    if (res_base2k != key_base2k) { // (:156-165) work on a copy at the key's base2k
-        const uint64_t cs = conv_size(res->size, res_base2k, key_base2k);
-        cur_bs = n * res->cols * cs * 8;
-        cur = mk(sc, n, res->cols, cs);
-        sc += align_up(B * cur_bs);
-        sc_len -= (size_t)align_up(B * cur_bs);
-        pgb_batch btn = {B, cur_bs, bt->stride_res, 0};
-        for (uint64_t i = 0; i < res->cols; i++) PGB_TRY(big_normalize_impl(m, &cur, key_base2k, 0, i, res, res_base2k, i, 0, false, &btn));
-    }
+    Arena ar = {(char *)scratch, scratch_len, 0};
+    pgb_vec_znx cur; // (:156-165) work on a copy at the key's base2k
+    uint64_t cur_bs;
+    PGB_TRY(glwe_to_base2k(m, ar, res, bt->stride_res, res_base2k, key_base2k, B, &cur, &cur_bs));
     // The rounds run out of place, alternating between `cur` and a second buffer (glwe_automorphism_add_assign is res = aut(ks(res)) +
     // res; the single-kernel route cannot run in place), and the result is copied back if it ends in the second one.
     const uint64_t alt_bs = n * cur.cols * cur.size * 8;
-    pgb_vec_znx alt = mk(sc, n, cur.cols, cur.size);
-    sc += align_up(B * alt_bs);
-    sc_len -= (size_t)align_up(B * alt_bs);
+    pgb_vec_znx alt = mk(ar.take(B * alt_bs), n, cur.cols, cur.size);
+    char *sc = ar.rest();
+    const size_t sc_len = ar.rest_len();
     pgb_vec_znx home = cur;
     const uint64_t home_bs = cur_bs;
     uint64_t alt_stride = alt_bs;
@@ -883,16 +764,6 @@ extern "C" int pgb_ggsw_expand_row_batched(pgb_module *m, pgb_mat_znx *ggsw, uin
     pgb_vec_znx_dft a_dft = mk(ar.take(B * a_dft_bs), n, rank, conv);
     pgb_vec_znx a_0 = mk(ar.take(B * a0_bs), n, 1, conv);
     pgb_vec_znx_dft res_dft = mk(ar.take(B * res_dft_bs), n, cols, tsk[0].size);
-    pgb_vec_znx_dft ai = a_dft, tmp = res_dft;
-    uint64_t ai_bs = 0, tmp_bs = 0;
-    if (dsize > 1) {
-        const uint64_t ai_max = umin64(div_ceil64(conv, dsize), tsk[0].rows);
-        ai_bs = n * rank * ai_max * pb;
-        ai = mk(ar.take(B * ai_bs), n, rank, ai_max);
-        tmp_bs = res_dft_bs;
-        tmp = mk(ar.take(B * tmp_bs), n, cols, tsk[0].size);
-        PGB_REQUIRE(ai.data && tmp.data, "ggsw_expand_row: scratch exhausted");
-    }
     for (uint64_t row = 0; row < dnum; row++) {
         pgb_vec_znx mi = mk((char *)ggsw->data + (row * cols + 0) * glwe_bytes, n, cols, size); // res.at(row, 0)
         const pgb_vec_znx *small = &mi; // column 0 of the row's GLWE joins output column `col`
@@ -911,14 +782,7 @@ extern "C" int pgb_ggsw_expand_row_batched(pgb_module *m, pgb_mat_znx *ggsw, uin
             small_bs = a0_bs;
         }
         for (uint64_t col = 1; col < cols; col++) { // ggsw_expand_rows_internal (:182-268)
-            if (dsize > 1) {
-                PGB_CHECK_CUDA(cudaMemsetAsync(ai.data, 0, B * ai_bs, m->stream));
-                PGB_CHECK_CUDA(cudaMemsetAsync(tmp.data, 0, B * tmp_bs, m->stream));
-            }
-            PGB_CHECK_CUDA(cudaMemsetAsync(res_dft.data, 0, B * res_dft_bs, m->stream));
-            PGB_TRY(gadget_product(m, &res_dft, &a_dft, &tsk[col - 1], dsize, true, &ai, &tmp, res_dft_bs, a_dft_bs, ai_bs, tmp_bs, B));
-            pgb_batch btc = {B, res_dft_bs, 0, 0};
-            PGB_TRY(pgb_vec_znx_idft_apply_consume_batched(m, &res_dft, &btc));
+            PGB_TRY(keyswitch_core(m, ar, "ggsw_expand_row", &res_dft, res_dft_bs, &a_dft, a_dft_bs, &tsk[col - 1], dsize, B));
             pgb_vec_znx_big res_big = res_dft;
             pgb_batch bts = {B, res_dft_bs, small_bs, 0};
             PGB_TRY(big_add_small_impl(m, &res_big, col, small, 0, &bts));

@@ -374,7 +374,8 @@ bool plan(const pgb_module *m, int R, int cols_out, int S, int *lpr_out, bool *t
 bool fft64_gadget_supported(const pgb_module *m, int R, int cols_out, int S, int base2k, int batch) {
     if (m->flavour != PGB_FFT64 || m->log_n < 9 || m->log_n > 12) return false;
     if (opt_on(m, PGB_OPT_NO_GADGET)) return false;
-    if (cols_out < 1 || cols_out > 4 || R < 1 || S < 1 || base2k < 1 || base2k > 63 || batch < 1) return false;
+    // FGadgetArgs holds the row tables of at most 16 input polys
+    if (cols_out < 1 || cols_out > 4 || R < 1 || R > 16 || S < 1 || base2k < 1 || base2k > 63 || batch < 1) return false;
     int lpr;
     bool tws;
     size_t smem;

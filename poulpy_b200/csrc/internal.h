@@ -5,6 +5,27 @@
 static inline uint64_t prep_bytes(const pgb_module *m) { return m->flavour == PGB_NTT120 ? 16 : 8; }
 static inline uint64_t big_bytes(const pgb_module *m) { return m->flavour == PGB_NTT120 ? 16 : 8; }
 
+// ---- scratch arena: every buffer carved from a caller's scratch starts at a 256-byte aligned offset -----------------------------------
+static const uint64_t ALIGN = 256;
+static inline uint64_t align_up(uint64_t x) { return (x + ALIGN - 1) / ALIGN * ALIGN; }
+struct Arena {
+    char *base;
+    size_t len, used;
+    void *take(size_t bytes) { // null when the buffer does not fit
+        size_t off = align_up(used);
+        if (off + bytes > len) return nullptr;
+        used = off + bytes;
+        return base + off;
+    }
+    // what is left after the buffers taken so far, for a nested call that carves its own scratch
+    char *rest() const { return base + align_up(used); }
+    size_t rest_len() const { return len - align_up(used); }
+};
+static inline pgb_vec_znx mk(void *data, uint64_t n, uint64_t cols, uint64_t size) {
+    pgb_vec_znx v = {data, n, cols, size, size};
+    return v;
+}
+
 // ---- aliasing (poulpy-hal/docs/backend_safety_contract.md "Aliasing": never UB, detect and reject) ----------------------------------
 // byte extent of `count` items of `item` bytes laid out `stride` bytes apart (stride 0 = one shared item)
 static inline uint64_t batch_extent(uint64_t item, uint64_t stride, uint64_t count) { return (count ? (count - 1) * stride : 0) + item; }
@@ -119,6 +140,10 @@ bool is_pinned(const void *p);
 int external_product_limbwise(pgb_module *m, pgb_vec_znx *res, uint64_t res_bs, uint64_t res_base2k, const pgb_vec_znx *ain, uint64_t ain_bs,
                               const pgb_vmp_pmat *ggsw, uint64_t ggsw_bs, uint64_t ggsw_base2k, uint64_t dsize, uint64_t B,
                               pgb_vec_znx_dft *res_dft, pgb_vec_znx_dft *a_dft, void *tmp);
+// core.cu: the input of a gadget product in the key's base: a itself when the bases agree, otherwise every column of a normalised from
+// base 2^from into base 2^to (ceil(a.size * from / to) limbs), in a buffer taken from `ar`
+int glwe_to_base2k(pgb_module *m, Arena &ar, const pgb_vec_znx *a, uint64_t a_bs, uint64_t from, uint64_t to, uint64_t B, pgb_vec_znx *out,
+                   uint64_t *out_bs);
 // api.cu (used by core.cu)
 int vmp_apply_impl(pgb_module *m, pgb_vec_znx_dft *res, const pgb_vec_znx_dft *a, const pgb_vmp_pmat *pmat, uint64_t limb_offset,
                    const pgb_batch *bt);

@@ -9,9 +9,6 @@
 // 8-byte word per thread, never a 16-byte vector or a bulk copy.
 #include "internal.h"
 
-static const uint64_t ALIGN = 256;
-static inline uint64_t align_up(uint64_t x) { return (x + ALIGN - 1) / ALIGN * ALIGN; }
-
 // ---- kernels: one thread per output coefficient, grid (coefficient, limb, ciphertext) ----------------------------------------------------
 struct LweEmbedArgs {
     const char *lwe; uint64_t lwe_bs; // item b at lwe + b * lwe_bs, limb j at + j * (n_in + 1) words
@@ -141,11 +138,12 @@ extern "C" int pgb_lwe_keyswitch_batched(pgb_module *m, pgb_vec_znx *res, uint64
     PGB_REQUIRE_DISJOINT(res, bt->stride_res, a, bt->stride_a, B, 8, what);
     PGB_TRY(check_scratch(what, scratch, scratch_len, pgb_lwe_keyswitch_tmp_bytes(m, res->size, a->size, a_base2k, key, key_base2k, dsize, B)));
     const uint64_t in_bs = n * 2 * a->size * 8, out_bs = n * 2 * res->size * 8;
-    char *in = (char *)scratch, *out = in + align_up(B * in_bs), *ks = out + align_up(B * out_bs);
-    pgb_vec_znx gin = {in, n, 2, a->size, a->size}, gout = {out, n, 2, res->size, res->size};
+    Arena ar = {(char *)scratch, scratch_len, 0};
+    char *in = (char *)ar.take(B * in_bs), *out = (char *)ar.take(B * out_bs);
+    pgb_vec_znx gin = mk(in, n, 2, a->size), gout = mk(out, n, 2, res->size);
     PGB_TRY(launch_embed(m, in, in_bs, a, bt->stride_a, B));
     pgb_batch btk = {B, out_bs, in_bs, 0};
-    PGB_TRY(pgb_glwe_keyswitch_batched(m, &gout, res_base2k, &gin, a_base2k, key, key_base2k, dsize, &btk, ks, scratch_len - (size_t)(ks - in)));
+    PGB_TRY(pgb_glwe_keyswitch_batched(m, &gout, res_base2k, &gin, a_base2k, key, key_base2k, dsize, &btk, ar.rest(), ar.rest_len()));
     return launch_extract(m, res, bt->stride_res, out, out_bs, res->size, B);
 }
 
@@ -167,10 +165,11 @@ extern "C" int pgb_glwe_to_lwe_batched(pgb_module *m, pgb_vec_znx *res, uint64_t
     PGB_REQUIRE_DISJOINT(res, bt->stride_res, a, bt->stride_a, B, 8, what);
     PGB_TRY(check_scratch(what, scratch, scratch_len, pgb_glwe_to_lwe_tmp_bytes(m, res->size, a->size, a_base2k, key, key_base2k, dsize, B)));
     const uint64_t out_bs = n * 2 * res->size * 8;
-    char *out = (char *)scratch, *ks = out + align_up(B * out_bs);
-    pgb_vec_znx gout = {out, n, 2, res->size, res->size};
+    Arena ar = {(char *)scratch, scratch_len, 0};
+    char *out = (char *)ar.take(B * out_bs);
+    pgb_vec_znx gout = mk(out, n, 2, res->size);
     pgb_batch btk = {B, out_bs, bt->stride_a, 0};
-    PGB_TRY(pgb_glwe_keyswitch_batched(m, &gout, res_base2k, a, a_base2k, key, key_base2k, dsize, &btk, ks, scratch_len - (size_t)(ks - out)));
+    PGB_TRY(pgb_glwe_keyswitch_batched(m, &gout, res_base2k, a, a_base2k, key, key_base2k, dsize, &btk, ar.rest(), ar.rest_len()));
     return launch_extract(m, res, bt->stride_res, out, out_bs, res->size, B);
 }
 
@@ -192,9 +191,10 @@ extern "C" int pgb_lwe_to_glwe_batched(pgb_module *m, pgb_vec_znx *res, uint64_t
     PGB_REQUIRE_DISJOINT(res, bt->stride_res, a, bt->stride_a, B, 8, what);
     PGB_TRY(check_scratch(what, scratch, scratch_len, pgb_lwe_to_glwe_tmp_bytes(m, res->size, a->size, a_base2k, key, key_base2k, dsize, B)));
     const uint64_t in_bs = n * 2 * a->size * 8;
-    char *in = (char *)scratch, *ks = in + align_up(B * in_bs);
-    pgb_vec_znx gin = {in, n, 2, a->size, a->size};
+    Arena ar = {(char *)scratch, scratch_len, 0};
+    char *in = (char *)ar.take(B * in_bs);
+    pgb_vec_znx gin = mk(in, n, 2, a->size);
     PGB_TRY(launch_embed(m, in, in_bs, a, bt->stride_a, B));
     pgb_batch btk = {B, bt->stride_res, in_bs, 0};
-    return pgb_glwe_keyswitch_batched(m, res, res_base2k, &gin, a_base2k, key, key_base2k, dsize, &btk, ks, scratch_len - (size_t)(ks - in));
+    return pgb_glwe_keyswitch_batched(m, res, res_base2k, &gin, a_base2k, key, key_base2k, dsize, &btk, ar.rest(), ar.rest_len());
 }

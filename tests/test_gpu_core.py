@@ -372,6 +372,31 @@ def test_fft64_gadget_kernel(n):
         assert not bad, ("ep", rank, a_size, g_size, res_size, bad[:10], len(bad))
 
 
+def test_fft64_gadget_more_than_16_input_polys():
+    """The FFT64 gadget kernel takes at most 16 input polys (R = min(dnum * rank_in, rank_in * a.size)), though its shared memory would
+    hold more at n = 512.  Shapes past that bound run the limb-wise sequence: an external product with R = 18 and a key-switch with R = 20,
+    bit for bit against the oracle."""
+    n, k, batch = 512, 14, 5
+    g, o = pb.Module(n, pb.FFT64), O.OracleModule(n, pb.FFT64)
+    rng = np.random.default_rng(1450)
+    pg, po = _key(g, o, rng, 9, 2, 2, 3, k)  # rank 1, dnum 9: R = 2 * 9
+    a = fill_uniform(rng, (batch, 9, 2, n), k)
+    want = fill_uniform(rng, (batch, 3, 2, n), k)
+    res_g = g.vec_znx_from_numpy(want)
+    g.glwe_external_product(res_g, k, g.vec_znx_from_numpy(a), k, pg, k)
+    g.sync()
+    o.glwe_external_product_batch(want, k, a, k, po, k)
+    assert np.array_equal(g.vec_znx_to_numpy(res_g), want)
+    pg, po = _key(g, o, rng, 5, 4, 4, 3, k)  # rank 4 -> 3, dnum 5: R = 4 * 5
+    a = fill_uniform(rng, (batch, 5, 5, n), k)
+    want = fill_uniform(rng, (batch, 3, 4, n), k)
+    res_g = g.vec_znx_from_numpy(want)
+    g.glwe_keyswitch(res_g, k, g.vec_znx_from_numpy(a), k, pg, k)
+    g.sync()
+    o.glwe_keyswitch_batch(want, k, a, k, po, k)
+    assert np.array_equal(g.vec_znx_to_numpy(res_g), want)
+
+
 def test_fft64_gadget_bench_shape():
     """FFT64 key-switch at the bench shape (n = 4096, base2k = 18, three input limbs, key of four): fused kernel == unfused HAL sequence
     == oracle."""
