@@ -293,6 +293,21 @@ size_t pgb_glwe_cmux_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_t 
 int pgb_glwe_cmux_batched(pgb_module *m, pgb_vec_znx *res, const pgb_vec_znx *t, const pgb_vec_znx *f, uint64_t base2k,
                           const pgb_vmp_pmat *s, uint64_t ggsw_stride, uint64_t ggsw_base2k, uint64_t dsize,
                           const pgb_batch *bt, void *scratch, size_t scratch_len);
+/* Blind rotation of GLWEs by GGSW bits (a rotation by an encrypted integer, as poulpy-bin-fhe's BDD arithmetic does it): per item b,
+ * acc_0 = a_b and, for i < n_bits with p_i = (step * 2^i) mod 2n (computed without overflow for any step),
+ *   acc_{i+1} = cmux(t = X^(p_i) acc_i, f = acc_i, s_{b,i})   -- the five CMux steps above, into res.size limbs (X^p = vec_znx_rotate(p)
+ *                                                                on every column);
+ * res_b = acc_{n_bits}.  Selector s_{b,i} at s->data + b*ggsw_stride + i*bit_stride (64-bit byte offsets): ggsw_stride as for the CMux
+ * (0 = one encrypted integer for the batch), bit_stride a multiple of 16 of at least one prepared GGSW when n_bits > 1.  bt->stride_res
+ * for res, bt->stride_a for a (0 = one a, e.g. a LUT, rotated by every item's integer), bt->stride_b must be 0.  count in [1, 65535],
+ * n_bits in [1, 64]; alignment, shapes and errors as for the CMux: res must not overlap a, any selector (b, i) or the scratch
+ * (PGB_ERR_ALIAS); every check runs before the first launch.  The scratch holds one ping-pong accumulator (n_bits > 1) and the CMux's
+ * scratch for res.size-limb operands. */
+size_t pgb_glwe_blind_rotate_ggsw_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_t a_size, uint64_t base2k,
+                                            const pgb_vmp_pmat *s, uint64_t ggsw_base2k, uint64_t dsize, uint64_t n_bits, uint64_t batch);
+int pgb_glwe_blind_rotate_ggsw_batched(pgb_module *m, pgb_vec_znx *res, const pgb_vec_znx *a, uint64_t base2k, int64_t step,
+                                       uint64_t n_bits, const pgb_vmp_pmat *s, uint64_t ggsw_stride, uint64_t bit_stride,
+                                       uint64_t ggsw_base2k, uint64_t dsize, const pgb_batch *bt, void *scratch, size_t scratch_len);
 
 /* Pinned keys.  The single-kernel gadget products derive per-key forms of a prepared key before they run (NTT120: the collapsed key and
  * the bit bound of the key's coefficients, three small launches; FFT64: a re-laid-out copy, one launch).  Every buffer is caller-owned, so

@@ -82,7 +82,7 @@ def lib():
         for name in ("pgb_glwe_keyswitch_tmp_bytes", "pgb_glwe_external_product_tmp_bytes", "pgb_cggi_blind_rotate_tmp_bytes",
                      "pgb_cggi_blind_rotate_standard_tmp_bytes", "pgb_cggi_blind_rotate_extended_tmp_bytes", "pgb_vmp_apply_dft_tmp_bytes", "pgb_glwe_tensor_apply_tmp_bytes",
                      "pgb_glwe_tensor_relinearize_tmp_bytes", "pgb_glwe_automorphism_tmp_bytes", "pgb_glwe_automorphism_add_assign_tmp_bytes",
-                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_glwe_cmux_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
+                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_glwe_cmux_tmp_bytes", "pgb_glwe_blind_rotate_ggsw_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
                      "pgb_vec_znx_big_automorphism_assign_tmp_bytes", "pgb_ggsw_expand_row_tmp_bytes",
                      "pgb_bytes_of_vmp_pmat", "pgb_size_of_scalar_prep", "pgb_size_of_scalar_big"):
             getattr(_lib, name).restype = C.c_size_t
@@ -558,6 +558,29 @@ class Module:
         _check(lib().pgb_glwe_cmux_batched(self._h, C.byref(r), C.byref(tv), C.byref(fv), _u64(base2k), C.byref(ks),
                                            _u64(s.batch_stride), _u64(ggsw_base2k), _u64(dsize), C.byref(bt),
                                            C.c_void_p(scratch.ptr), C.c_size_t(scratch.nbytes)))
+        return scratch
+
+    def glwe_blind_rotate_ggsw(self, res: VecZnx, a: VecZnx, base2k, step, n_bits, s: VmpPMat, ggsw_base2k, dsize=1, ggsw_stride=None,
+                               bit_stride=None, scratch: DevBuf = None):
+        """Rotation of res.batch GLWEs by encrypted integers m_b = sum_i bit_{b,i} 2^i: res_b = a_b X^(step m_b), one CMux per bit
+        (acc <- cmux(X^(step 2^i) acc, acc, s_{b,i})).  Selector (b, i) is at s + b * ggsw_stride + i * bit_stride; the defaults are the
+        bit-major layout of circuit.prepare_ggsw over res.batch * n_bits bootstrapped bits (bit_stride = s.batch_stride, ggsw_stride =
+        n_bits * s.batch_stride); ggsw_stride = 0 shares one integer across the batch.  An `a` with batch 1 is shared by the batch.
+        Asynchronous."""
+        if bit_stride is None and ggsw_stride is None:
+            assert s.batch >= n_bits * res.batch, (s.batch, n_bits, res.batch)
+        bit_stride = s.batch_stride if bit_stride is None else bit_stride
+        ggsw_stride = n_bits * s.batch_stride if ggsw_stride is None else ggsw_stride
+        ks = s.struct()
+        need = lib().pgb_glwe_blind_rotate_ggsw_tmp_bytes(self._h, _u64(res.size), _u64(a.size), _u64(base2k), C.byref(ks), _u64(ggsw_base2k),
+                                                          _u64(dsize), _u64(n_bits), _u64(res.batch))
+        if scratch is None or scratch.nbytes < need:
+            scratch = self._scratch(need)
+        r, av = res.struct(), a.struct()
+        bt = _BT(res.batch, res.batch_stride, a.batch_stride if a.batch > 1 else 0, 0)
+        _check(lib().pgb_glwe_blind_rotate_ggsw_batched(self._h, C.byref(r), C.byref(av), _u64(base2k), C.c_int64(step), _u64(n_bits),
+                                                        C.byref(ks), _u64(ggsw_stride), _u64(bit_stride), _u64(ggsw_base2k), _u64(dsize),
+                                                        C.byref(bt), C.c_void_p(scratch.ptr), C.c_size_t(scratch.nbytes)))
         return scratch
 
     def gadget_key_pin(self, key: VmpPMat):
