@@ -308,6 +308,22 @@ size_t pgb_glwe_blind_rotate_ggsw_tmp_bytes(const pgb_module *m, uint64_t res_si
 int pgb_glwe_blind_rotate_ggsw_batched(pgb_module *m, pgb_vec_znx *res, const pgb_vec_znx *a, uint64_t base2k, int64_t step,
                                        uint64_t n_bits, const pgb_vmp_pmat *s, uint64_t ggsw_stride, uint64_t bit_stride,
                                        uint64_t ggsw_base2k, uint64_t dsize, const pgb_batch *bt, void *scratch, size_t scratch_len);
+/* CMux tree over GGSW bits (selection of one of 2^n_bits GLWEs by an encrypted integer: an encrypted-array read, or the table selection of
+ * a lookup table read by vertical packing): per item b, with leaves g_{0,j} = a_b[j] at a->data + b*bt->stride_a + j*entry_stride
+ * (j < 2^n_bits; stride_a = 0 shares one table across the batch; entry_stride a multiple of 16 of at least one GLWE of a.size limbs),
+ *   g_{i+1,j} = cmux(t = g_{i,2j+1}, f = g_{i,2j}, s_{b,i})   for i < n_bits, j < 2^(n_bits-1-i)  -- the five CMux steps above, into
+ *                                                               res.size limbs;
+ * res_b = g_{n_bits,0}: with noise-free GGSW bits m_{b,i}, leaf sum_i m_{b,i} 2^i, normalised.  Selector s_{b,i} at s->data +
+ * b*ggsw_stride + i*bit_stride, with the rules of pgb_glwe_blind_rotate_ggsw_batched (0 = one encrypted integer for the batch).
+ * bt->stride_b must be 0, count in [1, 65535], n_bits in [1, 16]; res must not overlap the table, any selector or the scratch
+ * (PGB_ERR_ALIAS); every check runs before the first launch.  Items run in chunks of whole items, each chunk the whole tree, one batched
+ * CMux per level: _tmp_bytes(batch) is the scratch of a chunk of min(batch, floor(65535 / 2^(n_bits-1))) items, and the entry takes the
+ * largest chunk whose _tmp_bytes fits scratch_len (PGB_ERR_SCRATCH when one item does not).  Results do not depend on the chunk. */
+size_t pgb_glwe_cmux_tree_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_t a_size, uint64_t base2k, const pgb_vmp_pmat *s,
+                                    uint64_t ggsw_base2k, uint64_t dsize, uint64_t n_bits, uint64_t batch);
+int pgb_glwe_cmux_tree_batched(pgb_module *m, pgb_vec_znx *res, const pgb_vec_znx *a, uint64_t entry_stride, uint64_t base2k,
+                               uint64_t n_bits, const pgb_vmp_pmat *s, uint64_t ggsw_stride, uint64_t bit_stride, uint64_t ggsw_base2k,
+                               uint64_t dsize, const pgb_batch *bt, void *scratch, size_t scratch_len);
 
 /* Pinned keys.  The single-kernel gadget products derive per-key forms of a prepared key before they run (NTT120: the collapsed key and
  * the bit bound of the key's coefficients, three small launches; FFT64: a re-laid-out copy, one launch).  Every buffer is caller-owned, so

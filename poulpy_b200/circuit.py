@@ -146,6 +146,61 @@ def prepare_ggsw(module: "hal.Module", ggsw_buf: "hal.DevBuf", batch, dnum, rank
     return pmat
 
 
+# ---- lookup-table read by vertical packing ----------------------------------------------------------------------------------------
+def lut_split(n, lut, n_bits):
+    """The vertical-packing leaves of a table of T <= 2^n_bits entries as host polynomials: with nu = min(n_bits, log2 n), polynomial p
+    holds entries p 2^nu .. p 2^nu + 2^nu - 1 in its first coefficients (missing entries are 0).  lut is (size, T): limb j of entry t,
+    most significant limb first (a 1-d lut is one limb).  -> (nu, array (2^(n_bits - nu), size, n))"""
+    lut = np.atleast_2d(np.asarray(lut, dtype=np.int64))
+    size, T = lut.shape
+    assert n & (n - 1) == 0 and 1 <= n_bits <= 64 and T <= 1 << n_bits, (n, n_bits, T)
+    nu = min(n_bits, n.bit_length() - 1)
+    full = np.zeros((size, 1 << n_bits), dtype=np.int64)
+    full[:, :T] = lut
+    polys = np.zeros((1 << (n_bits - nu), size, n), dtype=np.int64)
+    polys[:, :, :1 << nu] = full.reshape(size, 1 << (n_bits - nu), 1 << nu).transpose(1, 0, 2)
+    return nu, polys
+
+
+def lut_read(module: "hal.Module", lut, sel: "hal.VmpPMat", batch, n_bits, base2k, ggsw_base2k=None, dsize=1, ggsw_stride=None,
+             bit_stride=None, scratch: "hal.DevBuf" = None) -> "hal.DevBuf":
+    """LWE encryptions of LUT[m_b] for `batch` encrypted integers m_b = sum_i bit_{b,i} 2^i (n_bits GGSW bits each, rank 1), by vertical
+    packing: the table (see lut_split) becomes 2^(n_bits - nu) trivial GLWEs (the polynomial in the body column, the mask zero); a CMux
+    tree (Module.glwe_cmux_tree) selects polynomial m_b >> nu with bits [nu, n_bits), a blind rotation (Module.glwe_blind_rotate_ggsw,
+    step -1) by bits [0, nu) brings entry m_b to coefficient 0, and lwe_sample_extract extracts it.  Selecting first leaves one polynomial
+    per item to rotate.  Selector (b, i) is at sel + b ggsw_stride + i bit_stride, with the defaults of glwe_blind_rotate_ggsw (the
+    bit-major output of prepare_ggsw).  -> the LWE batch, int64 (batch, size, 1, n + 1) on the device, size = the table's limbs.
+    Asynchronous."""
+    n = module.n
+    cols = sel.cols_in
+    assert cols == 2, "lwe_sample_extract reads rank-1 GLWEs"
+    ggsw_base2k = base2k if ggsw_base2k is None else ggsw_base2k
+    if bit_stride is None and ggsw_stride is None:
+        assert sel.batch >= n_bits * batch, (sel.batch, n_bits, batch)
+    bit_stride = sel.batch_stride if bit_stride is None else bit_stride
+    ggsw_stride = n_bits * sel.batch_stride if ggsw_stride is None else ggsw_stride
+    nu, polys = lut_split(n, lut, n_bits)
+    size = polys.shape[1]
+    leaves = np.zeros((polys.shape[0], size, cols, n), dtype=np.int64)
+    leaves[:, :, 0] = polys
+    table = module.vec_znx_from_numpy(leaves)
+    table = hal.VecZnx(table.buf, n, cols, size)  # one table of 2^(n_bits - nu) entries, shared by the batch
+    if n_bits > nu:
+        hi = hal.VmpPMat(sel.buf, n, sel.rows, cols, cols, sel.size, offset=sel.offset + nu * bit_stride, batch=sel.batch,
+                         batch_stride=sel.batch_stride)
+        picked = module.vec_znx_alloc(cols, size, batch)
+        scratch = module.glwe_cmux_tree(picked, table, base2k, n_bits - nu, hi, ggsw_base2k, dsize, ggsw_stride=ggsw_stride,
+                                        bit_stride=bit_stride, scratch=scratch)
+    else:
+        picked = table
+    rot = module.vec_znx_alloc(cols, size, batch)
+    module.glwe_blind_rotate_ggsw(rot, picked, base2k, -1, nu, sel, ggsw_base2k, dsize, ggsw_stride=ggsw_stride, bit_stride=bit_stride,
+                                  scratch=scratch)
+    out = hal.DevBuf(batch * size * (n + 1) * 8, device=module.device)
+    module.lwe_sample_extract(out, n, size, rot)
+    return out
+
+
 # ---- glwe_pack / post_process / exponent mode -----------------------------------------------------------------------------------
 class DeviceGlweOps:
     """The GLWE operations `pack_internal` and `post_process` are made of, on batches of device-resident GLWEs (VecZnx with a batch axis)

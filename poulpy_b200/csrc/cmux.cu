@@ -6,30 +6,38 @@
 // t, f, res are GLWEs of rank k in base 2^base2k; s_b = s.data + b * ggsw_stride is a prepared GGSW (VmpPMat(dnum, k + 1, k + 1, size))
 // in base 2^ggsw_base2k.  The difference kernel below writes normalize(t - f) in one pass; the external product and the final add +
 // normalise run on the routes described at cmux_launch.  The blind rotation by GGSW bits (pgb_glwe_blind_rotate_ggsw_batched) chains one
-// CMux per bit, acc <- cmux(X^(step 2^i) acc, acc, s_{b,i}), through the same routes.
+// CMux per bit, acc <- cmux(X^(step 2^i) acc, acc, s_{b,i}), through the same routes; the CMux tree (pgb_glwe_cmux_tree_batched) runs one
+// batched CMux per level, g_{i+1,j} = cmux(g_{i,2j+1}, g_{i,2j}, s_{b,i}).
 #include "internal.h"
 
 // ---- d = normalize_assign(X^rot t - f) ------------------------------------------------------------------------------------------------
 // One thread per (coefficient, column, ciphertext).  Limb j < size of d is t[j] - f[j] in wrapping i64 (a limb missing from an operand
 // reads as 0), normalised from the last limb up with the carry in a register: the lsh = 0 steps of vec_znx_normalize_assign
 // (reference/vec_znx/normalize.rs:403-425), whose first step keeps only the digit and whose last step drops the carry.  `fr`, when set,
-// receives f (limbs >= f_size zeroed) in the same pass: the FFT64 fused route adds it inside its carry chain.
-// ROT reads t as X^rot t (rot = p mod 2n), the negacyclic index and sign of rotate_kernel (big.cu), so the blind rotation's rotated
-// operand is never written; the ROT = false instance is the CMux's kernel.
+// receives f (limbs >= f_size zeroed) in the same pass: the FFT64 fused route adds it inside its carry chain, and level 0 of the CMux tree
+// hands every route this linear copy instead of the scattered leaves.
+// DIFF_ROT reads t as X^rot t (rot = p mod 2n), the negacyclic index and sign of rotate_kernel (big.cu), so the blind rotation's rotated
+// operand is never written.  DIFF_LEAF is level 0 of the CMux tree: grid item q = b * 2^lp + j reads t and f at item b's leaves 2j + 1
+// and 2j (t_bs = f_bs = the table stride, t = f + the leaf stride, pair_bs = twice the leaf stride).  DIFF_PLAIN is the CMux's kernel.
+enum { DIFF_PLAIN = 0, DIFF_ROT = 1, DIFF_LEAF = 2 };
 struct CmuxDiffArgs {
     const char *t; uint64_t t_bs; // VecZnx(cols, t_size) per item, limb j at + j * words words
     const char *f; uint64_t f_bs; // VecZnx(cols, f_size)
     char *d;       uint64_t d_bs; // VecZnx(cols, size)
     char *fr;      uint64_t fr_bs; // VecZnx(cols, size) or null
     uint32_t words;               // n * cols: words per limb
-    uint32_t n, rot;              // ring degree, and the rotation of t in [0, 2n) (ROT only)
+    uint32_t n, rot;              // ring degree, and the rotation of t in [0, 2n) (DIFF_ROT only)
     int t_size, f_size, size, K;
+    uint64_t pair_bs; uint32_t lp; // DIFF_LEAF only
 };
-template <bool ROT>
+template <int MODE>
 __global__ void __launch_bounds__(256) cmux_diff_kernel(CmuxDiffArgs p) {
+    constexpr bool ROT = MODE == DIFF_ROT;
     const uint32_t u = blockIdx.x * blockDim.x + threadIdx.x; // column * n + coefficient
     if (u >= p.words) return;
     const size_t b = blockIdx.y, ls = p.words;
+    // operand offsets of grid item b: linear, or (DIFF_LEAF) its table and its leaf pair
+    const size_t ob = MODE == DIFF_LEAF ? (b >> p.lp) : b, oj = MODE == DIFF_LEAF ? (b & ((1u << p.lp) - 1)) * p.pair_bs : 0;
     uint32_t tu = u;
     bool neg = false;
     if (ROT) { // (X^rot t)[i] = +-t[(i - rot) mod n], negated when exactly one of i < rot mod n, rot >= n holds
@@ -37,8 +45,8 @@ __global__ void __launch_bounds__(256) cmux_diff_kernel(CmuxDiffArgs p) {
         tu = u - i + (i >= r ? i - r : i + p.n - r);
         neg = (i < r) == (p.rot < p.n);
     }
-    const long long *t = reinterpret_cast<const long long *>(p.t + b * p.t_bs) + tu;
-    const long long *f = reinterpret_cast<const long long *>(p.f + b * p.f_bs) + u;
+    const long long *t = reinterpret_cast<const long long *>(p.t + ob * p.t_bs + oj) + tu;
+    const long long *f = reinterpret_cast<const long long *>(p.f + ob * p.f_bs + oj) + u;
     long long *d = reinterpret_cast<long long *>(p.d + b * p.d_bs) + u;
     long long *fr = p.fr ? reinterpret_cast<long long *>(p.fr + b * p.fr_bs) + u : nullptr;
     const int sh = 64 - p.K;
@@ -64,15 +72,38 @@ __global__ void __launch_bounds__(256) cmux_diff_kernel(CmuxDiffArgs p) {
     }
 }
 
-static int launch_diff(pgb_module *m, char *d, uint64_t d_bs, uint64_t size, const pgb_vec_znx *t, uint64_t t_bs, uint32_t rot,
-                       const pgb_vec_znx *f, uint64_t f_bs, char *fr, uint64_t fr_bs, uint64_t base2k, uint64_t B) {
-    const uint64_t words = m->n * t->cols;
-    CmuxDiffArgs p = {(const char *)t->data, t_bs, (const char *)f->data, f_bs, d, d_bs, fr, fr_bs, (uint32_t)words, (uint32_t)m->n, rot,
-                      (int)t->size, (int)f->size, (int)size, (int)base2k};
+// level 0 of the CMux tree: CMux q = b * 2^lp + j reads t = leaf 2j + 1 and f = leaf 2j of item b, leaf l at a + b * a_bs + l * entry_stride
+struct LeafPairs {
+    const pgb_vec_znx *a;
+    uint64_t a_bs, entry_stride;
+    uint32_t lp;
+};
+
+// the CMux operands: t (read as X^rot t) and f, item q at + q * t_bs / f_bs, or the leaf pairs of `lv` when it is set
+struct CmuxIn {
+    const pgb_vec_znx *t; uint64_t t_bs; uint32_t rot;
+    const pgb_vec_znx *f; uint64_t f_bs;
+    const LeafPairs *lv;
+};
+
+static int launch_diff(pgb_module *m, char *d, uint64_t d_bs, uint64_t size, const CmuxIn &in, char *fr, uint64_t fr_bs, uint64_t base2k,
+                       uint64_t B) {
+    const uint64_t words = m->n * in.t->cols;
+    CmuxDiffArgs p = {(const char *)in.t->data, in.t_bs, (const char *)in.f->data, in.f_bs, d, d_bs, fr, fr_bs, (uint32_t)words,
+                      (uint32_t)m->n, in.rot, (int)in.t->size, (int)in.f->size, (int)size, (int)base2k, 0, 0};
+    if (in.lv) {
+        p.t = (const char *)in.lv->a->data + in.lv->entry_stride;
+        p.f = (const char *)in.lv->a->data;
+        p.t_bs = p.f_bs = in.lv->a_bs;
+        p.t_size = p.f_size = (int)in.lv->a->size;
+        p.pair_bs = 2 * in.lv->entry_stride;
+        p.lp = in.lv->lp;
+    }
     const dim3 grid((uint32_t)((words + 255) / 256), (uint32_t)B);
     { ProfScope _ps(m, PROF_NORMALIZE);
-    if (rot) cmux_diff_kernel<true><<<grid, 256, 0, m->stream>>>(p);
-    else cmux_diff_kernel<false><<<grid, 256, 0, m->stream>>>(p);
+    if (in.lv) cmux_diff_kernel<DIFF_LEAF><<<grid, 256, 0, m->stream>>>(p);
+    else if (in.rot) cmux_diff_kernel<DIFF_ROT><<<grid, 256, 0, m->stream>>>(p);
+    else cmux_diff_kernel<DIFF_PLAIN><<<grid, 256, 0, m->stream>>>(p);
     }
     PGB_CHECK_CUDA(cudaGetLastError());
     return PGB_OK;
@@ -114,8 +145,8 @@ extern "C" size_t pgb_glwe_cmux_tmp_bytes(const pgb_module *m, uint64_t res_size
 }
 
 // Steps 1-5 for B items after the caller's checks: t is read as X^rot t (rot in [0, 2n); 0 for the CMux), item b's selector at
-// s->data + b * ggsw_stride, and the buffers come from `scratch` (pgb_glwe_cmux_tmp_bytes of res.size limbs).  Routes (all bit-exact with
-// the five steps; DESIGN.md §3.5b):
+// s->data + (b >> sel_shift) * ggsw_stride, and the buffers come from `scratch` (pgb_glwe_cmux_tmp_bytes of res.size limbs, plus one more
+// GLWE batch of res.size limbs when in.lv is set).  Routes (all bit-exact with the five steps; DESIGN.md §3.5b):
 //  * ggsw_stride == 0: d in scratch, then pgb_glwe_external_product_batched (with its single-kernel routes, gadget_fused in core.cu),
 //    add f, normalise.
 //  * per-item selectors, dsize == 1, ggsw_base2k == base2k, f.size <= min(res.size, s.size), fusion on:
@@ -124,50 +155,63 @@ extern "C" size_t pgb_glwe_cmux_tmp_bytes(const pgb_module *m, uint64_t res_size
 //      which adds res's own limbs inside its carry chain.
 //    Both replace normalize(normalize(big) + f) by normalize(big + f): equal because f has no limb where the big integer is truncated.
 //  * anything else: d -> (base conversion) -> the limb-wise external product with the per-item matrix stride -> add f, normalise.
-static int cmux_launch(pgb_module *m, pgb_vec_znx *res, uint64_t res_bs, const pgb_vec_znx *t, uint64_t t_bs, uint32_t rot, const pgb_vec_znx *f,
-                       uint64_t f_bs, uint64_t base2k, const pgb_vmp_pmat *s, uint64_t ggsw_stride, uint64_t ggsw_base2k, uint64_t dsize,
-                       uint64_t B, void *scratch, size_t scratch_len) {
+// With leaf pairs (in.lv: level 0 of the CMux tree, f not affine in the item) the difference kernel also writes a linear copy of f, into
+// res on the FFT64 fused route as always and into a scratch batch on the others, and steps 4-5 read that copy.
+static int cmux_launch(pgb_module *m, pgb_vec_znx *res, uint64_t res_bs, const CmuxIn &in, uint64_t base2k, const pgb_vmp_pmat *s,
+                       uint64_t ggsw_stride, uint32_t sel_shift, uint64_t ggsw_base2k, uint64_t dsize, uint64_t B, void *scratch,
+                       size_t scratch_len) {
     // ---- step 1 + 2 on every route: d = normalize(t - f), res.size limbs -----------------------------------------------------------------
     const uint64_t n = m->n, cols = s->cols_in, pb = prep_bytes(m);
     const uint64_t S = s->size, rs = res->size;
     const uint64_t d_bs = n * cols * rs * 8;
+    const bool fuse = ggsw_stride != 0 && dsize == 1 && ggsw_base2k == base2k && in.f->size <= umin64(rs, S) && !opt_on(m, PGB_OPT_NO_FUSION);
+    const bool fuse_ntt = fuse && ntt120_fused_supported(m), fuse_fft = fuse && !fuse_ntt && fft64_fused_back_supported(m, (int)S);
     Arena ar = {(char *)scratch, scratch_len, 0};
     char *sp = (char *)ar.take(B * d_bs);
     pgb_vec_znx d = mk(sp, n, cols, rs);
+    const pgb_vec_znx *f = in.f;
+    uint64_t f_bs = in.f_bs;
+    // the copy of f the difference kernel writes: into res on the FFT64 fused route; with leaf pairs into scratch on the other routes,
+    // and steps 4-5 read f from it (limbs past res.size are never added)
+    char *fr = fuse_fft ? (char *)res->data : in.lv ? (char *)ar.take(B * d_bs) : nullptr;
+    const uint64_t fr_bs = fuse_fft ? res_bs : d_bs;
+    pgb_vec_znx flin;
+    if (in.lv) {
+        PGB_REQUIRE(fr, "glwe_cmux_tree: scratch exhausted");
+        flin = mk(fr, n, cols, umin64(in.f->size, rs));
+        f = &flin;
+        f_bs = fr_bs;
+    }
+    PGB_TRY(launch_diff(m, sp, d_bs, rs, in, fr, fr ? fr_bs : 0, base2k, B));
 
     if (ggsw_stride == 0) { // one selector for the batch: the external product with every route it has
-        PGB_TRY(launch_diff(m, sp, d_bs, rs, t, t_bs, rot, f, f_bs, nullptr, 0, base2k, B));
         pgb_batch bte = {B, res_bs, d_bs, 0};
         PGB_TRY(pgb_glwe_external_product_batched(m, res, base2k, &d, base2k, s, ggsw_base2k, dsize, &bte, ar.rest(), ar.rest_len()));
         return add_f_normalize(m, res, res_bs, f, f_bs, base2k, B);
     }
 
-    const bool fuse = dsize == 1 && ggsw_base2k == base2k && f->size <= umin64(rs, S) && !opt_on(m, PGB_OPT_NO_FUSION);
     const uint64_t R = umin64(s->rows * cols, cols * rs); // rows of the vector-matrix product (external_product/glwe.rs:231)
     const uint64_t a_dft_bs = n * cols * rs * pb, res_dft_bs = n * cols * S * pb;
-    if (fuse && ntt120_fused_supported(m)) {
+    if (fuse_ntt) {
         char *a_dft = (char *)ar.take(B * a_dft_bs);
-        PGB_TRY(launch_diff(m, sp, d_bs, rs, t, t_bs, rot, f, f_bs, nullptr, 0, base2k, B));
-        LimbSet in = {sp, n * 8, d_bs}, out = {a_dft, n * pb, a_dft_bs}; // polys (limb, column) are consecutive on both sides
-        PGB_TRY(ntt120_forward(m, in, out, (int)(rs * cols), (int)B));
+        LimbSet li = {sp, n * 8, d_bs}, lo = {a_dft, n * pb, a_dft_bs}; // polys (limb, column) are consecutive on both sides
+        PGB_TRY(ntt120_forward(m, li, lo, (int)(rs * cols), (int)B));
         return ntt120_fused_back(m, a_dft, a_dft_bs, (const char *)s->data, (int)R, (int)(cols * S), (int)cols, (const char *)f->data, f_bs,
                                  cols * n * 8, (int)f->size, (char *)res->data, res_bs, cols * n * 8, (int)rs, (int)base2k, 0, (int)B,
-                                 nullptr, 0, 0, nullptr, false, false, true, ggsw_stride);
+                                 nullptr, 0, 0, nullptr, false, false, true, ggsw_stride, (int)sel_shift);
     }
-    if (fuse && fft64_fused_back_supported(m, (int)S)) {
+    if (fuse_fft) {
         char *res_dft = (char *)ar.take(B * res_dft_bs), *a_dft = (char *)ar.take(B * a_dft_bs);
-        PGB_TRY(launch_diff(m, sp, d_bs, rs, t, t_bs, rot, f, f_bs, (char *)res->data, res_bs, base2k, B));
-        LimbSet in = {sp, n * 8, d_bs}, out = {a_dft, n * pb, a_dft_bs};
-        PGB_TRY(fft64_forward(m, in, out, (int)(rs * cols), (int)B));
+        LimbSet li = {sp, n * 8, d_bs}, lo = {a_dft, n * pb, a_dft_bs};
+        PGB_TRY(fft64_forward(m, li, lo, (int)(rs * cols), (int)B));
         pgb_vec_znx_dft rd = {res_dft, n, cols, S, S}, ad = {a_dft, n, cols, rs, rs};
         pgb_batch btv = {B, res_dft_bs, a_dft_bs, ggsw_stride};
-        PGB_TRY(vmp_apply_impl(m, &rd, &ad, s, 0, &btv));
+        PGB_TRY(vmp_apply_impl(m, &rd, &ad, s, 0, &btv, sel_shift));
         return fft64_fused_back(m, res_dft, res_dft_bs, (int)cols, (int)S, (char *)res->data, res_bs, (int)rs, (int)base2k, (int)B);
     }
 
     // ---- limb-wise: the external product's HAL sequence with the per-item matrix stride -----------------------------------------------
     pgb_vec_znx_dft res_dft = mk(ar.take(B * res_dft_bs), n, cols, S);
-    PGB_TRY(launch_diff(m, sp, d_bs, rs, t, t_bs, rot, f, f_bs, nullptr, 0, base2k, B));
     pgb_vec_znx ain; // the input in ggsw_base2k, as the external product does
     uint64_t ain_bs;
     PGB_TRY(glwe_to_base2k(m, ar, &d, d_bs, base2k, ggsw_base2k, B, &ain, &ain_bs));
@@ -175,7 +219,8 @@ static int cmux_launch(pgb_module *m, pgb_vec_znx *res, uint64_t res_bs, const p
     pgb_vec_znx_dft a_dft = mk(ar.take(B * n * cols * a_dft_max * pb), n, cols, a_dft_max);
     void *tmp = dsize > 1 ? ar.take(B * res_dft_bs) : nullptr;
     PGB_REQUIRE(res_dft.data && ain.data && a_dft.data && (dsize == 1 || tmp), "glwe_cmux: scratch exhausted");
-    PGB_TRY(external_product_limbwise(m, res, res_bs, base2k, &ain, ain_bs, s, ggsw_stride, ggsw_base2k, dsize, B, &res_dft, &a_dft, tmp));
+    PGB_TRY(external_product_limbwise(m, res, res_bs, base2k, &ain, ain_bs, s, ggsw_stride, sel_shift, ggsw_base2k, dsize, B, &res_dft,
+                                      &a_dft, tmp));
     return add_f_normalize(m, res, res_bs, f, f_bs, base2k, B);
 }
 
@@ -228,8 +273,8 @@ extern "C" int pgb_glwe_cmux_batched(pgb_module *m, pgb_vec_znx *res, const pgb_
         pgb_set_error("glwe_cmux: scratch must not overlap res, t, f or a selector");
         return PGB_ERR_ALIAS;
     }
-    return cmux_launch(m, res, bt->stride_res, t, bt->stride_a, 0, f, bt->stride_b, base2k, s, ggsw_stride, ggsw_base2k, dsize, B, scratch,
-                       scratch_len);
+    const CmuxIn in = {t, bt->stride_a, 0, f, bt->stride_b, nullptr};
+    return cmux_launch(m, res, bt->stride_res, in, base2k, s, ggsw_stride, 0, ggsw_base2k, dsize, B, scratch, scratch_len);
 }
 
 // ---- blind rotation by GGSW bits: acc <- cmux(X^(step 2^i) acc, acc, s_{b,i}) for i < n_bits -------------------------------------------
@@ -290,10 +335,103 @@ extern "C" int pgb_glwe_blind_rotate_ggsw_batched(pgb_module *m, pgb_vec_znx *re
         const uint32_t rot = (uint32_t)(((uint64_t)step << i) & mask);
         pgb_vmp_pmat si = *s;
         si.data = (char *)s->data + i * bit_stride;
-        PGB_TRY(cmux_launch(m, &acc[w], acc_stride[w], cur, cur_bs, rot, cur, cur_bs, base2k, &si, ggsw_stride, ggsw_base2k, dsize, B, ar.rest(),
-                            ar.rest_len()));
+        const CmuxIn in = {cur, cur_bs, rot, cur, cur_bs, nullptr};
+        PGB_TRY(cmux_launch(m, &acc[w], acc_stride[w], in, base2k, &si, ggsw_stride, 0, ggsw_base2k, dsize, B, ar.rest(), ar.rest_len()));
         cur = &acc[w];
         cur_bs = acc_stride[w];
+    }
+    return PGB_OK;
+}
+
+// ---- CMux tree: g_{0,j} = leaf j, g_{i+1,j} = cmux(g_{i,2j+1}, g_{i,2j}, s_{b,i}) for i < n_bits, res = g_{n_bits,0} ----------------------
+// Chunks of whole items run the whole tree; no level of a chunk of Bc items launches more than Bc 2^(n_bits-1) <= 65535 grid items.
+static uint64_t tree_chunk_cap(uint64_t n_bits) { return 65535 >> (n_bits - 1); }
+
+extern "C" size_t pgb_glwe_cmux_tree_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_t a_size, uint64_t base2k,
+                                               const pgb_vmp_pmat *s, uint64_t ggsw_base2k, uint64_t dsize, uint64_t n_bits, uint64_t batch) {
+    (void)a_size;
+    if (n_bits < 1 || n_bits > 16) return 0;
+    const uint64_t Bc = umin64(batch, tree_chunk_cap(n_bits)), g = m->n * s->cols_in * res_size * 8, P0 = Bc << (n_bits - 1);
+    // the level-1 and level-2 outputs (the last level writes res) | level 0's CMux scratch and its linear copy of f (the later levels run
+    // fewer CMuxes of the same shape in the same space)
+    const uint64_t lv1 = n_bits > 1 ? align_up(P0 * g) : 0, lv2 = n_bits > 2 ? align_up((P0 >> 1) * g) : 0;
+    return lv1 + lv2 + align_up(P0 * g) + pgb_glwe_cmux_tmp_bytes(m, res_size, res_size, res_size, base2k, s, ggsw_base2k, dsize, P0);
+}
+
+// Level i of a chunk is one cmux_launch over its Bc 2^(n_bits-1-i) CMuxes, q = b 2^lp + j (lp = n_bits - 1 - i): item b's outputs are
+// consecutive, so the next level reads t = g_{i,2j+1} and f = g_{i,2j} at stride 2g from the buffer base + g and base, and the selector of
+// CMux q is item q >> lp's (sel_shift = lp).  Level 0 reads the leaves through the difference kernel's DIFF_LEAF instance.
+extern "C" int pgb_glwe_cmux_tree_batched(pgb_module *m, pgb_vec_znx *res, const pgb_vec_znx *a, uint64_t entry_stride, uint64_t base2k,
+                                          uint64_t n_bits, const pgb_vmp_pmat *s, uint64_t ggsw_stride, uint64_t bit_stride,
+                                          uint64_t ggsw_base2k, uint64_t dsize, const pgb_batch *bt, void *scratch, size_t scratch_len) {
+    static const char *who = "glwe_cmux_tree";
+    uint64_t s_item;
+    PGB_REQUIRE(a, "%s: null argument", who);
+    PGB_TRY(check_common(who, m, res, s, ggsw_stride, base2k, ggsw_base2k, dsize, bt, scratch, &s_item));
+    const uint64_t B = bt->count, n = m->n, cols = s->cols_in, rs = res->size;
+    PGB_TRY(check_glwe(who, "a", m, a, cols, bt->stride_a, B, true));
+    PGB_REQUIRE(bt->stride_b == 0, "%s: stride_b must be 0", who);
+    PGB_REQUIRE(n_bits >= 1 && n_bits <= 16, "%s: n_bits must be in [1, 16]", who);
+    const uint64_t a_item = n * cols * a->size * 8;
+    PGB_REQUIRE(entry_stride % 16 == 0 && entry_stride >= a_item,
+                "%s: entry_stride %llu must be a multiple of 16 of at least one GLWE of a.size limbs (%llu bytes)", who,
+                (unsigned long long)entry_stride, (unsigned long long)a_item);
+    PGB_REQUIRE(n_bits == 1 || (bit_stride % 16 == 0 && bit_stride >= s_item),
+                "%s: bit_stride %llu must be a multiple of 16 of at least one prepared GGSW (%llu bytes)", who, (unsigned long long)bit_stride,
+                (unsigned long long)s_item);
+    // every leaf (b, j) and selector (b, i) lies in [a, a + a_ext) and [s, s + s_ext): computed in 128 bits, so a stride that wraps the
+    // address space is rejected
+    const unsigned __int128 a_ext128 = (unsigned __int128)(B - 1) * bt->stride_a + (unsigned __int128)((1ull << n_bits) - 1) * entry_stride + a_item;
+    const unsigned __int128 s_ext128 = (unsigned __int128)(B - 1) * ggsw_stride + (unsigned __int128)(n_bits - 1) * bit_stride + s_item;
+    PGB_REQUIRE(a_ext128 <= (unsigned __int128)(UINTPTR_MAX - (uintptr_t)a->data), "%s: the table extends past the end of the address space",
+                who);
+    PGB_REQUIRE(s_ext128 <= (unsigned __int128)(UINTPTR_MAX - (uintptr_t)s->data),
+                "%s: the selectors extend past the end of the address space", who);
+    const uint64_t a_ext = (uint64_t)a_ext128, s_ext = (uint64_t)s_ext128;
+    // the largest chunk of whole items whose scratch fits
+    uint64_t lo = 1, hi = umin64(B, tree_chunk_cap(n_bits));
+    if (scratch_len < pgb_glwe_cmux_tree_tmp_bytes(m, rs, a->size, base2k, s, ggsw_base2k, dsize, n_bits, 1)) {
+        pgb_set_error("%s: scratch of %zu bytes < required %llu for one item", who, scratch_len,
+                      (unsigned long long)pgb_glwe_cmux_tree_tmp_bytes(m, rs, a->size, base2k, s, ggsw_base2k, dsize, n_bits, 1));
+        return PGB_ERR_SCRATCH;
+    }
+    while (lo < hi) {
+        const uint64_t mid = (lo + hi + 1) / 2;
+        if (pgb_glwe_cmux_tree_tmp_bytes(m, rs, a->size, base2k, s, ggsw_base2k, dsize, n_bits, mid) <= scratch_len) lo = mid;
+        else hi = mid - 1;
+    }
+    const uint64_t Bc = lo;
+    const uint64_t res_ext = batch_extent(n * cols * rs * 8, bt->stride_res, B);
+    if (ranges_overlap(res->data, res_ext, a->data, a_ext) || ranges_overlap(res->data, res_ext, s->data, s_ext)) {
+        pgb_set_error("%s: res must not overlap the table or a selector", who);
+        return PGB_ERR_ALIAS;
+    }
+    if (ranges_overlap(scratch, scratch_len, res->data, res_ext) || ranges_overlap(scratch, scratch_len, a->data, a_ext) ||
+        ranges_overlap(scratch, scratch_len, s->data, s_ext)) {
+        pgb_set_error("%s: scratch must not overlap res, the table or a selector", who);
+        return PGB_ERR_ALIAS;
+    }
+
+    const uint64_t g = n * cols * rs * 8, P0 = Bc << (n_bits - 1);
+    Arena ar = {(char *)scratch, scratch_len, 0};
+    pgb_vec_znx lvl[2] = {mk(n_bits > 1 ? ar.take(P0 * g) : nullptr, n, cols, rs), mk(n_bits > 2 ? ar.take((P0 >> 1) * g) : nullptr, n, cols, rs)};
+    for (uint64_t b0 = 0; b0 < B; b0 += Bc) {
+        const uint64_t nb = umin64(Bc, B - b0);
+        pgb_vec_znx ab = *a, out_res = *res;
+        ab.data = (char *)a->data + b0 * bt->stride_a;
+        out_res.data = (char *)res->data + b0 * bt->stride_res;
+        for (uint64_t i = 0; i < n_bits; i++) {
+            const uint32_t lp = (uint32_t)(n_bits - 1 - i);
+            pgb_vmp_pmat si = *s;
+            si.data = (char *)s->data + b0 * ggsw_stride + i * bit_stride;
+            const LeafPairs lv = {&ab, bt->stride_a, entry_stride, lp};
+            pgb_vec_znx tin = lvl[(i + 1) & 1];  // g_i (i >= 1): level i's output buffer is lvl[i & 1], so g_i is in lvl[(i - 1) & 1]
+            tin.data = (char *)tin.data + g;
+            const CmuxIn in = i == 0 ? CmuxIn{&ab, 0, 0, &ab, 0, &lv} : CmuxIn{&tin, 2 * g, 0, &lvl[(i + 1) & 1], 2 * g, nullptr};
+            pgb_vec_znx *out = i + 1 == n_bits ? &out_res : &lvl[i & 1];
+            const uint64_t out_bs = i + 1 == n_bits ? bt->stride_res : g;
+            PGB_TRY(cmux_launch(m, out, out_bs, in, base2k, &si, ggsw_stride, lp, ggsw_base2k, dsize, nb << lp, ar.rest(), ar.rest_len()));
+        }
     }
     return PGB_OK;
 }

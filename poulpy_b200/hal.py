@@ -82,7 +82,7 @@ def lib():
         for name in ("pgb_glwe_keyswitch_tmp_bytes", "pgb_glwe_external_product_tmp_bytes", "pgb_cggi_blind_rotate_tmp_bytes",
                      "pgb_cggi_blind_rotate_standard_tmp_bytes", "pgb_cggi_blind_rotate_extended_tmp_bytes", "pgb_vmp_apply_dft_tmp_bytes", "pgb_glwe_tensor_apply_tmp_bytes",
                      "pgb_glwe_tensor_relinearize_tmp_bytes", "pgb_glwe_automorphism_tmp_bytes", "pgb_glwe_automorphism_add_assign_tmp_bytes",
-                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_glwe_cmux_tmp_bytes", "pgb_glwe_blind_rotate_ggsw_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
+                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_glwe_cmux_tmp_bytes", "pgb_glwe_blind_rotate_ggsw_tmp_bytes", "pgb_glwe_cmux_tree_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
                      "pgb_vec_znx_big_automorphism_assign_tmp_bytes", "pgb_ggsw_expand_row_tmp_bytes",
                      "pgb_bytes_of_vmp_pmat", "pgb_size_of_scalar_prep", "pgb_size_of_scalar_big"):
             getattr(_lib, name).restype = C.c_size_t
@@ -581,6 +581,33 @@ class Module:
         _check(lib().pgb_glwe_blind_rotate_ggsw_batched(self._h, C.byref(r), C.byref(av), _u64(base2k), C.c_int64(step), _u64(n_bits),
                                                         C.byref(ks), _u64(ggsw_stride), _u64(bit_stride), _u64(ggsw_base2k), _u64(dsize),
                                                         C.byref(bt), C.c_void_p(scratch.ptr), C.c_size_t(scratch.nbytes)))
+        return scratch
+
+    def glwe_cmux_tree(self, res: VecZnx, a: VecZnx, base2k, n_bits, s: VmpPMat, ggsw_base2k, dsize=1, entry_stride=None, ggsw_stride=None,
+                       bit_stride=None, max_chunk=None, scratch: DevBuf = None):
+        """Selection of one of 2^n_bits GLWEs per item by encrypted integers m_b = sum_i bit_{b,i} 2^i: res_b = the table's entry m_b,
+        normalised, through a tree of CMuxes (level i: g_{i+1,j} = cmux(g_{i,2j+1}, g_{i,2j}, s_{b,i})).  `a` holds the tables: item b's
+        table at a + b * a.batch_stride, its entry j at + j * entry_stride (default: one GLWE of a.size limbs, entries consecutive); an `a`
+        with batch 1 is one table shared by the batch.  Selector (b, i) is at s + b * ggsw_stride + i * bit_stride, with the defaults and
+        rules of glwe_blind_rotate_ggsw.  max_chunk bounds the items per chunk (the scratch grows with it; results do not depend on it).
+        Asynchronous."""
+        assert a.batch in (1, res.batch), (a.batch, res.batch)
+        if bit_stride is None and ggsw_stride is None:
+            assert s.batch >= n_bits * res.batch, (s.batch, n_bits, res.batch)
+        bit_stride = s.batch_stride if bit_stride is None else bit_stride
+        ggsw_stride = n_bits * s.batch_stride if ggsw_stride is None else ggsw_stride
+        entry_stride = self.n * a.cols * a.size * 8 if entry_stride is None else entry_stride
+        ks = s.struct()
+        chunk = res.batch if max_chunk is None else min(res.batch, max_chunk)
+        need = lib().pgb_glwe_cmux_tree_tmp_bytes(self._h, _u64(res.size), _u64(a.size), _u64(base2k), C.byref(ks), _u64(ggsw_base2k),
+                                                  _u64(dsize), _u64(n_bits), _u64(chunk))
+        if scratch is None or scratch.nbytes < need:
+            scratch = self._scratch(need)
+        r, av = res.struct(), a.struct()
+        bt = _BT(res.batch, res.batch_stride, a.batch_stride if a.batch > 1 else 0, 0)
+        _check(lib().pgb_glwe_cmux_tree_batched(self._h, C.byref(r), C.byref(av), _u64(entry_stride), _u64(base2k), _u64(n_bits), C.byref(ks),
+                                                _u64(ggsw_stride), _u64(bit_stride), _u64(ggsw_base2k), _u64(dsize), C.byref(bt),
+                                                C.c_void_p(scratch.ptr), C.c_size_t(need if max_chunk is not None else scratch.nbytes)))
         return scratch
 
     def gadget_key_pin(self, key: VmpPMat):
