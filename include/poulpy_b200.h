@@ -324,6 +324,40 @@ size_t pgb_glwe_cmux_tree_tmp_bytes(const pgb_module *m, uint64_t res_size, uint
 int pgb_glwe_cmux_tree_batched(pgb_module *m, pgb_vec_znx *res, const pgb_vec_znx *a, uint64_t entry_stride, uint64_t base2k,
                                uint64_t n_bits, const pgb_vmp_pmat *s, uint64_t ggsw_stride, uint64_t bit_stride, uint64_t ggsw_base2k,
                                uint64_t dsize, const pgb_batch *bt, void *scratch, size_t scratch_len);
+/* Binary decision diagram over GGSW bits: a levelled CMux circuit given as data (host memory, read during the call only; it may be freed
+ * when the entry returns).  States 0 .. n_leaves-1 are the leaves; node k (level order: the level_count[0] nodes of level 0 first) is state
+ * n_leaves + k.  Every child of a node of level i is a leaf or a node of a level < i; outputs[o] is any state. */
+typedef struct {
+    uint64_t n_leaves;           /* states 0 .. n_leaves-1 are the leaves */
+    uint64_t n_levels;
+    const uint32_t *level_bit;   /* [n_levels]: the bit every node of level i selects with */
+    const uint32_t *level_count; /* [n_levels]: nodes in level i (>= 1) */
+    const uint32_t *node_t;      /* [total nodes], level order: the state taken when the bit is 1 */
+    const uint32_t *node_f;      /* [total nodes]: the state taken when the bit is 0 */
+    uint64_t n_out;
+    const uint32_t *outputs;     /* [n_out]: state indices */
+} pgb_bdd_circuit;
+/* Per item b: leaf j is a->data + b*bt->stride_a + j*entry_stride (a.size limbs; stride_a = 0 shares the leaves across the batch;
+ * entry_stride a multiple of 16 of at least one GLWE of a.size limbs when n_leaves > 1); node k of level i is
+ *   state[n_leaves + k] = cmux(t = state[node_t[k]], f = state[node_f[k]], s_{b, level_bit[i]})  -- the five CMux steps above, into
+ *                                                                                                 res.size limbs;
+ * output o goes to res->data + b*bt->stride_res + o*out_stride: a node's res.size limbs, or a leaf's first min(a.size, res.size) limbs with
+ * the rest zeroed (no normalisation).  Selector s_{b,i} at s->data + b*ggsw_stride + i*bit_stride, with the rules of
+ * pgb_glwe_blind_rotate_ggsw_batched (0 = one encrypted integer for the batch); level_bit[i] < n_bits <= 64.  bt->stride_b must be 0,
+ * count in [1, 65535], every level width in [1, 65535], n_out >= 1; out_stride a multiple of 16 of at least one GLWE of res.size limbs when
+ * n_out > 1, and bt->stride_res a multiple of 16 of at least (n_out-1)*out_stride plus one GLWE when count > 1.  res must not overlap the
+ * leaves, any selector or the scratch (PGB_ERR_ALIAS).  Every check (null pointers, child, output and bit indices, widths, 128-bit extents,
+ * aliasing, 256-byte scratch alignment) runs on the host arrays before the first launch.  Items run in chunks of whole items; a chunk of Bc
+ * items keeps Bc * (widest level) <= 65535, and _tmp_bytes(batch) is the scratch of a chunk of min(batch, that cap) items: the circuit's
+ * descriptor table, one block of Bc*level_count[i] GLWEs of res.size limbs per level, the linear copy of f and one CMux's scratch for the
+ * widest level.  The entry takes the largest chunk whose _tmp_bytes fits scratch_len (PGB_ERR_SCRATCH when one item does not).  Results do
+ * not depend on the chunk.  A chunk launches one CMux's launches per level plus one output copy. */
+size_t pgb_glwe_bdd_eval_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_t a_size, uint64_t base2k, const pgb_vmp_pmat *s,
+                                   uint64_t ggsw_base2k, uint64_t dsize, const pgb_bdd_circuit *c, uint64_t batch);
+int pgb_glwe_bdd_eval_batched(pgb_module *m, pgb_vec_znx *res, uint64_t out_stride, const pgb_vec_znx *a, uint64_t entry_stride,
+                              uint64_t base2k, uint64_t n_bits, const pgb_vmp_pmat *s, uint64_t ggsw_stride, uint64_t bit_stride,
+                              uint64_t ggsw_base2k, uint64_t dsize, const pgb_bdd_circuit *c, const pgb_batch *bt, void *scratch,
+                              size_t scratch_len);
 
 /* Pinned keys.  The single-kernel gadget products derive per-key forms of a prepared key before they run (NTT120: the collapsed key and
  * the bit bound of the key's coefficients, three small launches; FFT64: a re-laid-out copy, one launch).  Every buffer is caller-owned, so

@@ -201,6 +201,107 @@ def lut_read(module: "hal.Module", lut, sel: "hal.VmpPMat", batch, n_bits, base2
     return out
 
 
+# ---- binary decision diagrams ------------------------------------------------------------------------------------------------------
+class BddCircuit:
+    """A levelled CMux circuit (the pgb_bdd_circuit of Module.glwe_bdd_eval).  `leaves` are the leaf values (state j < len(leaves) is leaf
+    j); `levels` is a list of (bit, [(t, f), ...]): node k, counted in level order, is state len(leaves) + k and selects t when the bit is
+    1, f when it is 0; every child must be a leaf or a node of an earlier level.  `outputs` are state indices."""
+
+    def __init__(self, leaves, levels, outputs):
+        self.leaves = list(leaves)
+        self.levels = [(int(bit), [(int(t), int(f)) for t, f in nodes]) for bit, nodes in levels]
+        self.outputs = [int(o) for o in outputs]
+
+    @property
+    def n_nodes(self):
+        return sum(len(nodes) for _, nodes in self.levels)
+
+    def struct(self):
+        """-> (hal._BDD, the arrays it points into: keep them alive while the struct is in use)"""
+        u32 = lambda xs: np.ascontiguousarray(np.asarray(xs, dtype=np.uint32).reshape(-1))  # noqa: E731
+        bits = u32([b for b, _ in self.levels])
+        counts = u32([len(nodes) for _, nodes in self.levels])
+        t = u32([t for _, nodes in self.levels for t, _ in nodes])
+        f = u32([f for _, nodes in self.levels for _, f in nodes])
+        out = u32(self.outputs)
+        p = lambda arr: arr.ctypes.data_as(C.POINTER(C.c_uint32))  # noqa: E731
+        cs = hal._BDD(len(self.leaves), len(self.levels), p(bits), p(counts), p(t), p(f), len(self.outputs), p(out))
+        return cs, (bits, counts, t, f, out)
+
+
+def bdd_from_truth_tables(tables, n_bits, order):
+    """The shared, reduced, ordered BDD of binary functions given by truth tables (tables[o][x] in {0, 1} for x < 2^n_bits, bit i of x
+    the input bit i), with the variable order `order` (a permutation of range(n_bits)): the root tests order[0], level 0 tests order[-1],
+    and empty levels are left out.  Nodes are merged through a unique table and a node whose two children are equal is dropped, so
+    children may skip levels and outputs share nodes.  Leaves are the values 0 and 1.  -> BddCircuit"""
+    assert 1 <= n_bits <= 16 and sorted(order) == list(range(n_bits)), (n_bits, order)
+    x = np.arange(1 << n_bits)
+    pos = np.zeros(1 << n_bits, dtype=np.int64)  # the index of x with order[0] as its most significant bit
+    for d, v in enumerate(order):
+        pos |= ((x >> v) & 1) << (n_bits - 1 - d)
+    unique, nodes = {}, []  # (depth, t, f) -> node id; nodes[id] = (depth, t, f); ids >= 2, leaves are 0 and 1
+
+    def mk(d, t, f):
+        if t == f:
+            return t
+        key = (d, t, f)
+        if key not in unique:
+            unique[key] = len(nodes) + 2
+            nodes.append(key)
+        return unique[key]
+
+    roots = []
+    for tab in tables:
+        tab = np.asarray(tab, dtype=np.int64)
+        assert tab.shape == (1 << n_bits,) and np.all((tab == 0) | (tab == 1))
+        cur = np.empty(1 << n_bits, dtype=np.int64)
+        cur[pos] = tab
+        cur = cur.tolist()
+        for d in range(n_bits - 1, -1, -1):  # cur[i]: the cofactor of prefix i of order[:d + 1]; its last bit is order[d]
+            cur = [mk(d, cur[2 * i + 1], cur[2 * i]) for i in range(len(cur) // 2)]
+        roots.append(cur[0])
+    state = {0: 0, 1: 1}
+    levels = []
+    for d in range(n_bits - 1, -1, -1):
+        ids = [i + 2 for i, (dd, _, _) in enumerate(nodes) if dd == d]
+        if not ids:
+            continue
+        first = 2 + sum(len(lv) for _, lv in levels)
+        for j, i in enumerate(ids):
+            state[i] = first + j
+        levels.append((order[d], [(state[nodes[i - 2][1]], state[nodes[i - 2][2]]) for i in ids]))
+    return BddCircuit([0, 1], levels, [state[r] for r in roots])
+
+
+def bdd_leaves(n, circuit, scale, size, cols=2):
+    """The leaves of bdd_eval as a host array (n_leaves, size, cols, n): trivial GLWEs whose body is the constant leaves[j] * scale in
+    the first limb, the rest zero."""
+    leaves = np.zeros((len(circuit.leaves), size, cols, n), dtype=np.int64)
+    leaves[:, 0, 0, 0] = np.asarray(circuit.leaves, dtype=np.int64) * scale
+    return leaves
+
+
+def bdd_eval(module: "hal.Module", circuit, sel: "hal.VmpPMat", batch, n_bits, base2k, scale, size=1, ggsw_base2k=None, dsize=1,
+             ggsw_stride=None, bit_stride=None, scratch: "hal.DevBuf" = None) -> "hal.DevBuf":
+    """LWE encryptions of the outputs of a BDD (BddCircuit) for `batch` items of n_bits GGSW bits each (rank 1): the leaves are the
+    trivial GLWEs of bdd_leaves (value * scale, `size` limbs), Module.glwe_bdd_eval evaluates the circuit into `size`-limb GLWEs, and
+    lwe_sample_extract extracts coefficient 0 of every output.  Selector (b, i) is at sel + b ggsw_stride + i bit_stride, with the
+    defaults of glwe_blind_rotate_ggsw (the bit-major output of prepare_ggsw).  -> the LWEs, int64 (batch, n_out, size, 1, n + 1) on the
+    device.  Asynchronous."""
+    n, cols = module.n, sel.cols_in
+    assert cols == 2, "lwe_sample_extract reads rank-1 GLWEs"
+    ggsw_base2k = base2k if ggsw_base2k is None else ggsw_base2k
+    leaves = module.vec_znx_from_numpy(bdd_leaves(n, circuit, scale, size, cols))
+    leaves = hal.VecZnx(leaves.buf, n, cols, size)  # one set of leaves, shared by the batch
+    n_out = len(circuit.outputs)
+    res = module.vec_znx_alloc(cols, size, batch * n_out)
+    module.glwe_bdd_eval(res, leaves, circuit, base2k, n_bits, sel, ggsw_base2k, dsize, ggsw_stride=ggsw_stride, bit_stride=bit_stride,
+                         scratch=scratch)
+    out = hal.DevBuf(batch * n_out * size * (n + 1) * 8, device=module.device)
+    module.lwe_sample_extract(out, n, size, res)
+    return out
+
+
 # ---- glwe_pack / post_process / exponent mode -----------------------------------------------------------------------------------
 class DeviceGlweOps:
     """The GLWE operations `pack_internal` and `post_process` are made of, on batches of device-resident GLWEs (VecZnx with a batch axis)

@@ -631,7 +631,7 @@ extern "C" int pgb_vmp_prepare_batched(pgb_module *m, pgb_vmp_pmat *res, const p
 }
 
 int vmp_apply_impl(pgb_module *m, pgb_vec_znx_dft *res, const pgb_vec_znx_dft *a, const pgb_vmp_pmat *pmat, uint64_t limb_offset,
-                   const pgb_batch *bt, uint32_t pm_shift) {
+                   const pgb_batch *bt, uint32_t pm_div) {
     CHECK_BATCH(bt);
     CHECK_N(res, "vmp_apply_dft_to_dft(res)");
     CHECK_N(a, "vmp_apply_dft_to_dft(a)");
@@ -651,18 +651,18 @@ int vmp_apply_impl(pgb_module *m, pgb_vec_znx_dft *res, const pgb_vec_znx_dft *a
         const bool quirk = (col_max & 1) && col_max < ncols;
         PGB_TRY(ntt120_vmp(m, (const char *)a->data, bt->stride_a, (char *)res->data, bt->stride_res, (const char *)pmat->data,
                            bt->stride_b, (uint32_t)row_max, (uint32_t)ncols, (uint32_t)off, (uint32_t)(active - (quirk ? 1 : 0)),
-                           (uint32_t)bt->count, pm_shift));
+                           (uint32_t)bt->count, pm_div));
         if (quirk)
             PGB_TRY(ntt120_vmp_odd_last(m, (const char *)a->data, bt->stride_a, (char *)res->data + (active - 1) * poly, bt->stride_res,
                                         (const char *)pmat->data, bt->stride_b, (uint32_t)row_max, (uint32_t)ncols, (uint32_t)(col_max - 1),
-                                        (uint32_t)bt->count, pm_shift));
+                                        (uint32_t)bt->count, pm_div));
         return raw_limbs(m, true, shift(R, active), shift(R, active), poly, (uint32_t)(res_polys - active), (uint32_t)bt->count); // :282-287
     } else {
         const uint64_t col_max = umin64(ncols, res_polys); // fft64/vmp.rs:214-215
         if (off >= col_max) return raw_limbs(m, true, R, R, poly, (uint32_t)res_polys, (uint32_t)bt->count);
         const uint64_t active = col_max - off;
         PGB_TRY(fft64_vmp(m, (const char *)a->data, bt->stride_a, (char *)res->data, bt->stride_res, (const char *)pmat->data,
-                          bt->stride_b, (uint32_t)row_max, (uint32_t)ncols, (uint32_t)off, (uint32_t)active, (uint32_t)bt->count, pm_shift));
+                          bt->stride_b, (uint32_t)row_max, (uint32_t)ncols, (uint32_t)off, (uint32_t)active, (uint32_t)bt->count, pm_div));
         // fft64/vmp.rs:263 zeroes res[col_max..] only; polys in [col_max - off, col_max) keep their previous content
         return raw_limbs(m, true, shift(R, col_max), shift(R, col_max), poly, (uint32_t)(res_polys - col_max), (uint32_t)bt->count);
     }

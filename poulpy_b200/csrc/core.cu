@@ -325,14 +325,14 @@ extern "C" int pgb_glwe_external_product_batched(pgb_module *m, pgb_vec_znx *res
         tmp = ar.take(B * res_dft_bs);
         PGB_REQUIRE(tmp, "glwe_external_product: scratch exhausted");
     }
-    return external_product_limbwise(m, res, bt->stride_res, res_base2k, &ain, ain_bs, ggsw, 0, 0, ggsw_base2k, dsize, B, &res_dft, &a_dft, tmp);
+    return external_product_limbwise(m, res, bt->stride_res, res_base2k, &ain, ain_bs, ggsw, 0, 1, ggsw_base2k, dsize, B, &res_dft, &a_dft, tmp);
 }
 
 // glwe_external_product_internal (:197-271) as the limb-wise HAL sequence, then the normalisation into res (:138-140).  ain is already in
 // ggsw_base2k; res_dft (cols, ggsw.size), a_dft (cols, ceil(ain.size / dsize)) and, for dsize > 1, `tmp` (the size of res_dft) are the
-// caller's scratch.  Item b's GGSW is at ggsw + (b >> ggsw_shift) * ggsw_bs (ggsw_bs = 0: one GGSW for the whole batch).
+// caller's scratch.  Item b's GGSW is at ggsw + (b / ggsw_div) * ggsw_bs (ggsw_bs = 0: one GGSW for the whole batch).
 int external_product_limbwise(pgb_module *m, pgb_vec_znx *res, uint64_t res_bs, uint64_t res_base2k, const pgb_vec_znx *ain, uint64_t ain_bs,
-                              const pgb_vmp_pmat *ggsw, uint64_t ggsw_bs, uint32_t ggsw_shift, uint64_t ggsw_base2k, uint64_t dsize, uint64_t B,
+                              const pgb_vmp_pmat *ggsw, uint64_t ggsw_bs, uint32_t ggsw_div, uint64_t ggsw_base2k, uint64_t dsize, uint64_t B,
                               pgb_vec_znx_dft *res_dft, pgb_vec_znx_dft *a_dft, void *tmp_data) {
     const uint64_t n = m->n, pb = prep_bytes(m), cols = ggsw->cols_in, a_size = ain->size;
     const uint64_t res_dft_bs = n * cols * ggsw->size * pb, a_dft_bs = n * cols * a_dft->size * pb;
@@ -341,7 +341,7 @@ int external_product_limbwise(pgb_module *m, pgb_vec_znx *res, uint64_t res_bs, 
         for (uint64_t j = 0; j < cols; j++) PGB_TRY(pgb_vec_znx_dft_apply_batched(m, 1, 0, a_dft, j, ain, j, &btd));
         PGB_CHECK_CUDA(cudaMemsetAsync(res_dft->data, 0, B * res_dft_bs, m->stream)); // res_dft.zero() (:123)
         pgb_batch btv = {B, res_dft_bs, a_dft_bs, ggsw_bs};
-        PGB_TRY(vmp_apply_impl(m, res_dft, a_dft, ggsw, 0, &btv, ggsw_shift));
+        PGB_TRY(vmp_apply_impl(m, res_dft, a_dft, ggsw, 0, &btv, ggsw_div));
     } else {
         PGB_CHECK_CUDA(cudaMemsetAsync(res_dft->data, 0, B * res_dft_bs, m->stream)); // res_dft.zero() (:123)
         pgb_vec_znx_dft tmp = mk(tmp_data, n, cols, ggsw->size);
@@ -358,11 +358,11 @@ int external_product_limbwise(pgb_module *m, pgb_vec_znx *res, uint64_t res_bs, 
             for (uint64_t j = 0; j < cols; j++) PGB_TRY(pgb_vec_znx_dft_apply_batched(m, dsize, dsize - 1 - di, a_dft, j, ain, j, &btd));
             if (di == 0) {
                 pgb_batch btv = {B, res_dft_bs, a_dft_bs, ggsw_bs};
-                PGB_TRY(vmp_apply_impl(m, res_dft, a_dft, ggsw, 0, &btv, ggsw_shift));
+                PGB_TRY(vmp_apply_impl(m, res_dft, a_dft, ggsw, 0, &btv, ggsw_div));
             } else {
                 tmp.size = res_dft->size;
                 pgb_batch btv = {B, res_dft_bs, a_dft_bs, ggsw_bs};
-                PGB_TRY(vmp_apply_impl(m, &tmp, a_dft, ggsw, di, &btv, ggsw_shift));
+                PGB_TRY(vmp_apply_impl(m, &tmp, a_dft, ggsw, di, &btv, ggsw_div));
                 pgb_batch bta = {B, res_dft_bs, res_dft_bs, 0};
                 for (uint64_t c = 0; c < cols; c++) PGB_TRY(pgb_vec_znx_dft_add_assign_batched(m, res_dft, c, &tmp, c, &bta));
             }

@@ -532,9 +532,9 @@ int fft64_inverse_big(pgb_module *m, LimbSet in, LimbSet out, int jobs_per_batch
 struct FVmpArgs {
     const char *a;  uint64_t a_bs;
     char *res;      uint64_t res_bs;
-    const char *pm; uint64_t pm_bs;  // item z's matrix at pm + (z >> pm_shift) * pm_bs
+    const char *pm; uint64_t pm_bs;  // item z's matrix at pm + (z / pm_div) * pm_bs
     uint32_t m2;     // double2 words per half limb (= m / 2)
-    uint32_t row_max, C, col0, ncols_out, pm_shift;
+    uint32_t row_max, C, col0, ncols_out, pm_div;
 };
 // each thread: two consecutive complex frequencies (double2 of re, double2 of im), CT output columns
 template <int CT> __global__ void __launch_bounds__(128) fft64_vmp_kernel(FVmpArgs p) {
@@ -543,7 +543,7 @@ template <int CT> __global__ void __launch_bounds__(128) fft64_vmp_kernel(FVmpAr
     const uint32_t c0 = blockIdx.y * CT;
     const size_t poly_words = (size_t)2 * p.m2; // double2 words per poly
     const double2 *a = reinterpret_cast<const double2 *>(p.a + (size_t)blockIdx.z * p.a_bs) + u;
-    const double2 *pm = reinterpret_cast<const double2 *>(p.pm + (size_t)(blockIdx.z >> p.pm_shift) * p.pm_bs) + u + (size_t)(p.col0 + c0) * poly_words;
+    const double2 *pm = reinterpret_cast<const double2 *>(p.pm + (size_t)(blockIdx.z / p.pm_div) * p.pm_bs) + u + (size_t)(p.col0 + c0) * poly_words;
     double2 *res = reinterpret_cast<double2 *>(p.res + (size_t)blockIdx.z * p.res_bs) + u + (size_t)c0 * poly_words;
     const int nc = min((uint32_t)CT, p.ncols_out - c0);
     double2 accr[CT], acci[CT];
@@ -573,9 +573,9 @@ template <int CT> __global__ void __launch_bounds__(128) fft64_vmp_kernel(FVmpAr
     }
 }
 int fft64_vmp(pgb_module *m, const char *a, uint64_t a_bs, char *res, uint64_t res_bs, const char *pm, uint64_t pm_bs,
-              uint32_t row_max, uint32_t C, uint32_t col0, uint32_t ncols_out, uint32_t batch, uint32_t pm_shift) {
+              uint32_t row_max, uint32_t C, uint32_t col0, uint32_t ncols_out, uint32_t batch, uint32_t pm_div) {
     if (ncols_out == 0 || batch == 0) return PGB_OK;
-    FVmpArgs p = {a, a_bs, res, res_bs, pm, pm_bs, (uint32_t)(m->n / 4), row_max, C, col0, ncols_out, pm_shift};
+    FVmpArgs p = {a, a_bs, res, res_bs, pm, pm_bs, (uint32_t)(m->n / 4), row_max, C, col0, ncols_out, pm_div};
     // output polys per thread: 2 (default) or 4 (PGB_OPT_VMP_CT).  Measured on B200 in the streaming regime (scripts/vmp_stream.py,
     // profiles/r2_vmp_stream.md): two polys per thread reach 95-103 % of the measured copy bandwidth at every sweep shape, four 74-89 % --
     // the re-reads of `a` that four would save are L2 hits, the extra CTAs and the 70 (vs 128) registers are what the stream needs

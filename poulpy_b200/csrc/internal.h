@@ -65,11 +65,11 @@ int ntt120_fused_back(pgb_module *m, const char *a_dft, uint64_t a_bs, const cha
                       uint64_t small_bs, uint64_t small_limb_stride, int small_size, char *res, uint64_t res_bs, uint64_t res_limb_stride,
                       int res_size, int base2k, int64_t res_offset, int batch, const char *glwe, uint64_t glwe_bs, uint64_t glwe_words,
                       const int *skip = nullptr, bool skip_list = false, bool direct = false, bool small_all_cols = false,
-                      uint64_t pmat_bs = 0, int pmat_shift = 0);
+                      uint64_t pmat_bs = 0, uint32_t pmat_div = 1);
 // direct: a_dft already holds the C = cols_out * size product polys (limb-major, column-minor), pmat / R are ignored: inverse transform +
 // CRT + add_small + normalize only; small_all_cols: `small` is added on every output column (CGGI: acc += ...), not only on column 0;
-// pmat_bs: item b multiplies by the matrix at pmat + (b >> pmat_shift) * pmat_bs (0 = one matrix for the whole batch; the collapsed-key
-// path needs 0); pmat_shift > 0 gives 2^pmat_shift consecutive items one matrix (the levels of the CMux tree)
+// pmat_bs: item b multiplies by the matrix at pmat + (b / pmat_div) * pmat_bs (0 = one matrix for the whole batch; the collapsed-key
+// path needs 0); pmat_div > 1 gives pmat_div consecutive items one matrix (the levels of the CMux tree and of a BDD)
 // max bit length of the integer coefficients of `polys` DFT polys -> *bits_dev (coef_ws: polys * 16n bytes of device scratch)
 int ntt120_key_max_bits(pgb_module *m, const char *pmat, int polys, char *coef_ws, int *bits_dev);
 // ntt120_gadget.cu
@@ -88,16 +88,16 @@ int fft64_gadget_fused(pgb_module *m, const char *in, uint64_t in_bs, int in_col
                        int key_rows = 0, int group_limit = 0, int aut_mode = 0, int64_t aut_p = 0, int post_size = 0);
 // ntt120_ops.cu
 int ntt120_vmp(pgb_module *m, const char *a, uint64_t a_bs, char *res, uint64_t res_bs, const char *pm, uint64_t pm_bs,
-               uint32_t row_max, uint32_t C, uint32_t col0, uint32_t ncols_out, uint32_t batch, uint32_t pm_shift = 0);
+               uint32_t row_max, uint32_t C, uint32_t col0, uint32_t ncols_out, uint32_t batch, uint32_t pm_div = 1);
 int ntt120_vmp_odd_last(pgb_module *m, const char *a, uint64_t a_bs, char *res_poly, uint64_t res_bs, const char *pm, uint64_t pm_bs,
-                        uint32_t row_max, uint32_t C, uint32_t last, uint32_t batch, uint32_t pm_shift = 0);
+                        uint32_t row_max, uint32_t C, uint32_t last, uint32_t batch, uint32_t pm_div = 1);
 int ntt120_ew(pgb_module *m, int op, LimbSet dst, LimbSet a, LimbSet b, uint32_t jobs, uint32_t batch);
 // fft64.cu
 int fft64_module_init(pgb_module *m);
 int fft64_forward(pgb_module *m, LimbSet in, LimbSet out, int jobs_per_batch, int batch, long long and_mask = -1);
 int fft64_inverse_big(pgb_module *m, LimbSet in, LimbSet out, int jobs_per_batch, int batch);
 int fft64_vmp(pgb_module *m, const char *a, uint64_t a_bs, char *res, uint64_t res_bs, const char *pm, uint64_t pm_bs,
-              uint32_t row_max, uint32_t C, uint32_t col0, uint32_t ncols_out, uint32_t batch, uint32_t pm_shift = 0);
+              uint32_t row_max, uint32_t C, uint32_t col0, uint32_t ncols_out, uint32_t batch, uint32_t pm_div = 1);
 int fft64_ew(pgb_module *m, int op, LimbSet dst, LimbSet a, LimbSet b, uint32_t jobs, uint32_t batch);
 // cggi_fused.cu
 bool cggi_fused_supported(const pgb_module *m, uint64_t cols, uint64_t dnum, uint64_t brk_size);
@@ -136,18 +136,18 @@ void key_cache_destroy(pgb_module *m);
 // core.cu: lazily grown device workspace of the host front ends; whether a host pointer is page-locked
 int ensure_ws(pgb_module *m, size_t len);
 bool is_pinned(const void *p);
-// core.cu: the limb-wise external product (item b's GGSW at ggsw + (b >> ggsw_shift) * ggsw_bs, ggsw_bs = 0: shared) and its
+// core.cu: the limb-wise external product (item b's GGSW at ggsw + (b / ggsw_div) * ggsw_bs, ggsw_bs = 0: shared) and its
 // normalisation into res; the input ain is in ggsw_base2k, res_dft / a_dft / tmp (dsize > 1 only) are scratch of the external product's layout
 int external_product_limbwise(pgb_module *m, pgb_vec_znx *res, uint64_t res_bs, uint64_t res_base2k, const pgb_vec_znx *ain, uint64_t ain_bs,
-                              const pgb_vmp_pmat *ggsw, uint64_t ggsw_bs, uint32_t ggsw_shift, uint64_t ggsw_base2k, uint64_t dsize, uint64_t B,
+                              const pgb_vmp_pmat *ggsw, uint64_t ggsw_bs, uint32_t ggsw_div, uint64_t ggsw_base2k, uint64_t dsize, uint64_t B,
                               pgb_vec_znx_dft *res_dft, pgb_vec_znx_dft *a_dft, void *tmp);
 // core.cu: the input of a gadget product in the key's base: a itself when the bases agree, otherwise every column of a normalised from
 // base 2^from into base 2^to (ceil(a.size * from / to) limbs), in a buffer taken from `ar`
 int glwe_to_base2k(pgb_module *m, Arena &ar, const pgb_vec_znx *a, uint64_t a_bs, uint64_t from, uint64_t to, uint64_t B, pgb_vec_znx *out,
                    uint64_t *out_bs);
-// api.cu (used by core.cu); item b's matrix at pmat + (b >> pm_shift) * bt->stride_b
+// api.cu (used by core.cu); item b's matrix at pmat + (b / pm_div) * bt->stride_b
 int vmp_apply_impl(pgb_module *m, pgb_vec_znx_dft *res, const pgb_vec_znx_dft *a, const pgb_vmp_pmat *pmat, uint64_t limb_offset,
-                   const pgb_batch *bt, uint32_t pm_shift = 0);
+                   const pgb_batch *bt, uint32_t pm_div = 1);
 int big_normalize_impl(pgb_module *m, pgb_vec_znx *res, uint64_t res_base2k, int64_t res_offset, uint64_t res_col,
                        const pgb_vec_znx_big *a, uint64_t a_base2k, uint64_t a_col, int op, bool a_is_big, const pgb_batch *bt);
 int big_add_small_impl(pgb_module *m, pgb_vec_znx_big *res, uint64_t res_col, const pgb_vec_znx *a, uint64_t a_col, const pgb_batch *bt);

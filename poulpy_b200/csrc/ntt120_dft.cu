@@ -448,10 +448,11 @@ __global__ void __launch_bounds__(256) ntt120_inv_top8_kernel(TopJobs jb, const 
 // poulpy-cpu-ref/src/reference/ntt120/vec_znx_big.rs:367-446).
 struct FusedArgs {
     const char *a_dft;  uint64_t a_bs;      // R polys (16n B each) per ciphertext
-    const char *pmat;   uint64_t pmat_bs;   // [R][C] polys; item b's matrix at pmat + (b >> pmat_shift) * pmat_bs (0 = one for the batch)
+    const char *pmat;   uint64_t pmat_bs;   // [R][C] polys; item b's matrix at pmat + (b / pmat_div) * pmat_bs (0 = one for the batch)
     const char *small;  uint64_t small_bs;  uint64_t small_limb_stride; int small_size; // i64 limbs added to column 0 (or null)
     char *res;          uint64_t res_bs;    uint64_t res_limb_stride;                    // i64 output, column c at + c*n*8
-    int R, C, cols_out, pmat_shift;
+    int R, C, cols_out;
+    uint32_t pmat_div;
     int direct;         // 1: a_dft already holds the C product polys (limb-major, column-minor): no matrix, straight to the inverse transform
     int small_all_cols; // 1: `small` is added on every output column (column c at + c*n words), not only on column 0
     // same-base2k normalisation plan (big = C / cols_out limbs)
@@ -568,7 +569,7 @@ template <int L> __global__ void __launch_bounds__(Geo<L>::T, 2) ntt120_fused_ba
         const size_t b = work / p.cols_out;
         if (skip && skip[b]) continue; // handled by the collapsed-key kernel
         const uint32_t *a = reinterpret_cast<const uint32_t *>(p.a_dft + b * p.a_bs);
-        const uint32_t *pm = reinterpret_cast<const uint32_t *>(p.pmat + (b >> p.pmat_shift) * p.pmat_bs);
+        const uint32_t *pm = reinterpret_cast<const uint32_t *>(p.pmat + (b / p.pmat_div) * p.pmat_bs);
         long long *res = reinterpret_cast<long long *>(p.res + b * p.res_bs) + (size_t)col * n;
         const long long *small = (p.small && (col == 0 || p.small_all_cols))
                                      ? reinterpret_cast<const long long *>(p.small + b * p.small_bs) + (p.small_all_cols ? (size_t)col * n : 0)
@@ -1116,12 +1117,12 @@ static uint32_t pow2_mod_q(uint64_t e, uint32_t q) {
 int ntt120_fused_back(pgb_module *m, const char *a_dft, uint64_t a_bs, const char *pmat, int R, int C, int cols_out, const char *small,
                       uint64_t small_bs, uint64_t small_limb_stride, int small_size, char *res, uint64_t res_bs, uint64_t res_limb_stride,
                       int res_size, int base2k, int64_t res_offset, int batch, const char *glwe, uint64_t glwe_bs, uint64_t glwe_words,
-                      const int *skip, bool skip_list, bool direct, bool small_all_cols, uint64_t pmat_bs, int pmat_shift) {
+                      const int *skip, bool skip_list, bool direct, bool small_all_cols, uint64_t pmat_bs, uint32_t pmat_div) {
     FusedArgs p;
     memset(&p, 0, sizeof p);
     p.a_dft = a_dft; p.a_bs = a_bs; p.pmat = pmat; p.pmat_bs = pmat_bs; p.small = small; p.small_bs = small_bs; p.small_limb_stride = small_limb_stride;
     p.small_size = small_size; p.res = res; p.res_bs = res_bs; p.res_limb_stride = res_limb_stride;
-    p.R = R; p.C = C; p.cols_out = cols_out; p.pmat_shift = pmat_shift;
+    p.R = R; p.C = C; p.cols_out = cols_out; p.pmat_div = pmat_div;
     p.direct = direct ? 1 : 0; p.small_all_cols = small_all_cols ? 1 : 0;
     p.K = base2k; p.res_size = res_size; p.a_size = C / cols_out;
     int64_t lsh = res_offset % base2k, lo = res_offset / base2k;

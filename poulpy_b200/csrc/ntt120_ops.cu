@@ -17,9 +17,9 @@ using namespace n120;
 struct VmpArgs {
     const char *a;  uint64_t a_bs;     // a polys: a + b*a_bs + r*poly_bytes
     char *res;      uint64_t res_bs;   // res polys: res + b*res_bs + c*poly_bytes
-    const char *pm; uint64_t pm_bs;    // pmat polys: pm + (b >> pm_shift)*pm_bs + (r*C + c)*poly_bytes
+    const char *pm; uint64_t pm_bs;    // pmat polys: pm + (b / pm_div)*pm_bs + (r*C + c)*poly_bytes
     uint32_t n4;                        // uint4 words per plane (= n / 4)
-    uint32_t row_max, C, col0, ncols_out, pm_shift;
+    uint32_t row_max, C, col0, ncols_out, pm_div;
 };
 
 template <int CT> __global__ void __launch_bounds__(256) ntt120_vmp_kernel(VmpArgs p) {
@@ -29,7 +29,7 @@ template <int CT> __global__ void __launch_bounds__(256) ntt120_vmp_kernel(VmpAr
     const uint32_t c0 = blockIdx.y * CT;
     const size_t poly_words = (size_t)4 * p.n4;
     const uint4 *a = reinterpret_cast<const uint4 *>(p.a + (size_t)blockIdx.z * p.a_bs) + u;
-    const uint4 *pm = reinterpret_cast<const uint4 *>(p.pm + (size_t)(blockIdx.z >> p.pm_shift) * p.pm_bs) + u + (size_t)(p.col0 + c0) * poly_words;
+    const uint4 *pm = reinterpret_cast<const uint4 *>(p.pm + (size_t)(blockIdx.z / p.pm_div) * p.pm_bs) + u + (size_t)(p.col0 + c0) * poly_words;
     uint4 *res = reinterpret_cast<uint4 *>(p.res + (size_t)blockIdx.z * p.res_bs) + u + (size_t)c0 * poly_words;
     const int nc = min((uint32_t)CT, p.ncols_out - c0);
 
@@ -118,9 +118,9 @@ template <int CT, int BT> __global__ void __launch_bounds__(256) ntt120_vmp_bt_k
 }
 
 int ntt120_vmp(pgb_module *m, const char *a, uint64_t a_bs, char *res, uint64_t res_bs, const char *pm, uint64_t pm_bs,
-               uint32_t row_max, uint32_t C, uint32_t col0, uint32_t ncols_out, uint32_t batch, uint32_t pm_shift) {
+               uint32_t row_max, uint32_t C, uint32_t col0, uint32_t ncols_out, uint32_t batch, uint32_t pm_div) {
     if (ncols_out == 0 || batch == 0) return PGB_OK;
-    VmpArgs p = {a, a_bs, res, res_bs, pm, pm_bs, (uint32_t)(m->n / 4), row_max, C, col0, ncols_out, pm_shift};
+    VmpArgs p = {a, a_bs, res, res_bs, pm, pm_bs, (uint32_t)(m->n / 4), row_max, C, col0, ncols_out, pm_div};
     const uint32_t words = (uint32_t)m->n; // uint4 words per poly
     dim3 block(256);
     const int ct_sel = (int)m->opt[PGB_OPT_VMP_CT];
@@ -163,7 +163,7 @@ __global__ void __launch_bounds__(256) ntt120_vmp_odd_last_kernel(VmpArgs p, uin
     const PrimeRt pr(u / p.n4);
     const size_t poly_words = (size_t)4 * p.n4;
     const uint4 *a = reinterpret_cast<const uint4 *>(p.a + (size_t)blockIdx.z * p.a_bs) + u;
-    const uint4 *pm = reinterpret_cast<const uint4 *>(p.pm + (size_t)(blockIdx.z >> p.pm_shift) * p.pm_bs) + u;
+    const uint4 *pm = reinterpret_cast<const uint4 *>(p.pm + (size_t)(blockIdx.z / p.pm_div) * p.pm_bs) + u;
     unsigned long long acc[4] = {0, 0, 0, 0};
     for (uint32_t i = 0; i < p.row_max; i++) {
         const uint4 av = __ldg(a + (size_t)i * poly_words);
@@ -178,8 +178,8 @@ __global__ void __launch_bounds__(256) ntt120_vmp_odd_last_kernel(VmpArgs p, uin
         make_uint4(pr.reduce(acc[0]), pr.reduce(acc[1]), pr.reduce(acc[2]), pr.reduce(acc[3]));
 }
 int ntt120_vmp_odd_last(pgb_module *m, const char *a, uint64_t a_bs, char *res_poly, uint64_t res_bs, const char *pm, uint64_t pm_bs,
-                        uint32_t row_max, uint32_t C, uint32_t last, uint32_t batch, uint32_t pm_shift) {
-    VmpArgs p = {a, a_bs, res_poly, res_bs, pm, pm_bs, (uint32_t)(m->n / 4), row_max, C, 0, 1, pm_shift};
+                        uint32_t row_max, uint32_t C, uint32_t last, uint32_t batch, uint32_t pm_div) {
+    VmpArgs p = {a, a_bs, res_poly, res_bs, pm, pm_bs, (uint32_t)(m->n / 4), row_max, C, 0, 1, pm_div};
     ProfScope _ps(m, PROF_VMP);
     ntt120_vmp_odd_last_kernel<<<dim3(((uint32_t)m->n + 255) / 256, 1, batch), 256, 0, m->stream>>>(p, last);
     PGB_CHECK_CUDA(cudaGetLastError());

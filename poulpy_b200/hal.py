@@ -46,6 +46,12 @@ class _BT(C.Structure):
     _fields_ = [("count", C.c_uint64), ("stride_res", C.c_uint64), ("stride_a", C.c_uint64), ("stride_b", C.c_uint64)]
 
 
+class _BDD(C.Structure):
+    _fields_ = [("n_leaves", C.c_uint64), ("n_levels", C.c_uint64), ("level_bit", C.POINTER(C.c_uint32)),
+                ("level_count", C.POINTER(C.c_uint32)), ("node_t", C.POINTER(C.c_uint32)), ("node_f", C.POINTER(C.c_uint32)),
+                ("n_out", C.c_uint64), ("outputs", C.POINTER(C.c_uint32))]
+
+
 _lib = None
 
 
@@ -82,7 +88,7 @@ def lib():
         for name in ("pgb_glwe_keyswitch_tmp_bytes", "pgb_glwe_external_product_tmp_bytes", "pgb_cggi_blind_rotate_tmp_bytes",
                      "pgb_cggi_blind_rotate_standard_tmp_bytes", "pgb_cggi_blind_rotate_extended_tmp_bytes", "pgb_vmp_apply_dft_tmp_bytes", "pgb_glwe_tensor_apply_tmp_bytes",
                      "pgb_glwe_tensor_relinearize_tmp_bytes", "pgb_glwe_automorphism_tmp_bytes", "pgb_glwe_automorphism_add_assign_tmp_bytes",
-                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_glwe_cmux_tmp_bytes", "pgb_glwe_blind_rotate_ggsw_tmp_bytes", "pgb_glwe_cmux_tree_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
+                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_glwe_cmux_tmp_bytes", "pgb_glwe_blind_rotate_ggsw_tmp_bytes", "pgb_glwe_cmux_tree_tmp_bytes", "pgb_glwe_bdd_eval_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
                      "pgb_vec_znx_big_automorphism_assign_tmp_bytes", "pgb_ggsw_expand_row_tmp_bytes",
                      "pgb_bytes_of_vmp_pmat", "pgb_size_of_scalar_prep", "pgb_size_of_scalar_big"):
             getattr(_lib, name).restype = C.c_size_t
@@ -608,6 +614,42 @@ class Module:
         _check(lib().pgb_glwe_cmux_tree_batched(self._h, C.byref(r), C.byref(av), _u64(entry_stride), _u64(base2k), _u64(n_bits), C.byref(ks),
                                                 _u64(ggsw_stride), _u64(bit_stride), _u64(ggsw_base2k), _u64(dsize), C.byref(bt),
                                                 C.c_void_p(scratch.ptr), C.c_size_t(need if max_chunk is not None else scratch.nbytes)))
+        return scratch
+
+    def glwe_bdd_eval(self, res: VecZnx, a: VecZnx, circuit, base2k, n_bits, s: VmpPMat, ggsw_base2k, dsize=1, entry_stride=None,
+                      out_stride=None, ggsw_stride=None, bit_stride=None, max_chunk=None, scratch: DevBuf = None):
+        """Evaluation of a binary decision diagram (circuit.BddCircuit, or anything with a `struct()` giving the pgb_bdd_circuit) over
+        GGSW bits: per item b, node k of level i is cmux(state[t_k], state[f_k], s_{b, bit_i}), and output o is the state circuit.outputs[o]
+        (a node normalised into res.size limbs, or a leaf copied).  res holds n_out GLWEs per item: res.batch = batch * n_out, item b's
+        output o at index b * n_out + o (out_stride: res.batch_stride by default).  `a` holds the leaves: item b's leaf j at
+        a + b * a.batch_stride + j * entry_stride (default: one GLWE of a.size limbs, leaves consecutive); an `a` with batch 1 is shared by
+        the batch.  Selector (b, i) is at s + b * ggsw_stride + i * bit_stride, with the defaults and rules of glwe_blind_rotate_ggsw.
+        max_chunk bounds the items per chunk (the scratch grows with it; results do not depend on it).  Asynchronous."""
+        cs, keep = circuit.struct()
+        n_out = cs.n_out
+        assert n_out >= 1 and res.batch % n_out == 0, (res.batch, n_out)
+        B = res.batch // n_out
+        assert a.batch in (1, B), (a.batch, B)
+        if bit_stride is None and ggsw_stride is None:
+            assert s.batch >= n_bits * B, (s.batch, n_bits, B)
+        bit_stride = s.batch_stride if bit_stride is None else bit_stride
+        ggsw_stride = n_bits * s.batch_stride if ggsw_stride is None else ggsw_stride
+        entry_stride = self.n * a.cols * a.size * 8 if entry_stride is None else entry_stride
+        out_stride = res.batch_stride if out_stride is None else out_stride
+        assert (B - 1) * n_out * out_stride + (n_out - 1) * out_stride + self.n * res.cols * res.size * 8 <= res.buf.nbytes - res.offset
+        ks = s.struct()
+        chunk = B if max_chunk is None else min(B, max_chunk)
+        need = lib().pgb_glwe_bdd_eval_tmp_bytes(self._h, _u64(res.size), _u64(a.size), _u64(base2k), C.byref(ks), _u64(ggsw_base2k),
+                                                 _u64(dsize), C.byref(cs), _u64(chunk))
+        if scratch is None or scratch.nbytes < need:
+            scratch = self._scratch(need)
+        r, av = res.struct(), a.struct()
+        bt = _BT(B, n_out * out_stride, a.batch_stride if a.batch > 1 else 0, 0)
+        _check(lib().pgb_glwe_bdd_eval_batched(self._h, C.byref(r), _u64(out_stride), C.byref(av), _u64(entry_stride), _u64(base2k),
+                                               _u64(n_bits), C.byref(ks), _u64(ggsw_stride), _u64(bit_stride), _u64(ggsw_base2k),
+                                               _u64(dsize), C.byref(cs), C.byref(bt), C.c_void_p(scratch.ptr),
+                                               C.c_size_t(need if max_chunk is not None else scratch.nbytes)))
+        del keep
         return scratch
 
     def gadget_key_pin(self, key: VmpPMat):
