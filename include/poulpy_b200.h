@@ -358,6 +358,27 @@ int pgb_glwe_bdd_eval_batched(pgb_module *m, pgb_vec_znx *res, uint64_t out_stri
                               uint64_t base2k, uint64_t n_bits, const pgb_vmp_pmat *s, uint64_t ggsw_stride, uint64_t bit_stride,
                               uint64_t ggsw_base2k, uint64_t dsize, const pgb_bdd_circuit *c, const pgb_batch *bt, void *scratch,
                               size_t scratch_len);
+/* glwe_pack (poulpy-core/src/glwe_packing.rs:15-170), batched: per item b, input j < n_in is the GLWE at a->data + b*bt->stride_a +
+ * j*entry_stride (stride_a = 0 shares the inputs across the batch), and res_b (res->data + b*bt->stride_res) is the GLWE whose coefficient
+ * index[j] carries the constant coefficient of input j: bit for bit what the host composition glwe_pack(ops, res, {index[j]: a_j},
+ * log_gap_out) over the batched entries computes (pack_internal per pair of round i < log_n - log_gap_out, then glwe_trace with skip =
+ * log_n - log_gap_out).  `index` is a HOST array read during the call only; indices are distinct, below n and multiples of 2^log_gap_out.
+ * One layout throughout: a.size == res.size, one base2k for GLWEs and keys.  `keys` is a HOST array of log_n prepared automorphism keys of
+ * one shape, keys[i] for pgb_trace_galois_element(i), cols_in = cols - 1, cols_out = cols.  The inputs are read-only.  n_in in [1, n],
+ * log_gap_out <= log_n, nkeys >= log_n, count in [1, 65535], bt->stride_b == 0; data and strides multiples of 16, entry_stride at least one
+ * GLWE when n_in > 1; res must not overlap the inputs, a key or the scratch (PGB_ERR_ALIAS); scratch 256-byte aligned.  Every check runs
+ * before the first launch.  Round i of a chunk is one prep kernel, at most three batched automorphism calls under keys[i] (plain
+ * glwe_automorphism for the pairs, op 0 for keys with only j, op 2 for keys with only j + t) and one combine kernel when pairs exist; then
+ * the trace (or, without rounds, one copy).  Items run in chunks of whole items, Bc * (widest round) <= 65535; _tmp_bytes(batch) is the
+ * scratch of a chunk of min(batch, that cap) items: the descriptor table, two ping-pong state blocks and the x block of Bc * (widest round)
+ * GLWEs, the y block of Bc * (most pairs of a round) GLWEs, and the automorphism / trace scratch.  The entry takes the largest chunk whose
+ * _tmp_bytes fits scratch_len (PGB_ERR_SCRATCH when one item does not); results do not depend on the chunk.  _tmp_bytes returns 0 for an
+ * invalid map. */
+size_t pgb_glwe_pack_tmp_bytes(const pgb_module *m, uint64_t size, uint64_t base2k, const pgb_vmp_pmat *key, uint64_t dsize,
+                               const uint32_t *index, uint64_t n_in, uint64_t log_gap_out, uint64_t batch);
+int pgb_glwe_pack_batched(pgb_module *m, pgb_vec_znx *res, const pgb_vec_znx *a, uint64_t entry_stride, const uint32_t *index,
+                          uint64_t n_in, uint64_t log_gap_out, uint64_t base2k, const pgb_vmp_pmat *keys, uint64_t nkeys,
+                          uint64_t dsize, const pgb_batch *bt, void *scratch, size_t scratch_len);
 
 /* Pinned keys.  The single-kernel gadget products derive per-key forms of a prepared key before they run (NTT120: the collapsed key and
  * the bit bound of the key's coefficients, three small launches; FFT64: a re-laid-out copy, one launch).  Every buffer is caller-owned, so

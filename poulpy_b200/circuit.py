@@ -302,6 +302,28 @@ def bdd_eval(module: "hal.Module", circuit, sel: "hal.VmpPMat", batch, n_bits, b
     return out
 
 
+def bdd_eval_packed(module: "hal.Module", circuit, sel: "hal.VmpPMat", batch, n_bits, base2k, scale, atk, log_gap_out=0, size=1,
+                    ggsw_base2k=None, dsize=1, dsize_atk=1, ggsw_stride=None, bit_stride=None, scratch: "hal.DevBuf" = None) -> "hal.VecZnx":
+    """The outputs of a BDD packed into one GLWE per item: the leaves and Module.glwe_bdd_eval of bdd_eval, then Module.glwe_pack with
+    output o at coefficient o << log_gap_out (n_out << log_gap_out <= n).  atk: log_n prepared automorphism keys, atk[i] for
+    Module.trace_galois_element(i), in base2k.  -> VecZnx of `batch` GLWEs (rank 1, `size` limbs) on the device.  Asynchronous."""
+    n, cols = module.n, sel.cols_in
+    n_out = len(circuit.outputs)
+    assert n_out << log_gap_out <= n, (n_out, log_gap_out, n)
+    ggsw_base2k = base2k if ggsw_base2k is None else ggsw_base2k
+    leaves = module.vec_znx_from_numpy(bdd_leaves(n, circuit, scale, size, cols))
+    leaves = hal.VecZnx(leaves.buf, n, cols, size)
+    outs = module.vec_znx_alloc(cols, size, batch * n_out)
+    scratch = module.glwe_bdd_eval(outs, leaves, circuit, base2k, n_bits, sel, ggsw_base2k, dsize, ggsw_stride=ggsw_stride,
+                                   bit_stride=bit_stride, scratch=scratch)
+    g = n * cols * size * 8
+    a = hal.VecZnx(outs.buf, n, cols, size, batch=batch, batch_stride=n_out * g)  # item b's output o at b n_out + o
+    res = module.vec_znx_alloc(cols, size, batch)
+    module.glwe_pack(res, a, [o << log_gap_out for o in range(n_out)], log_gap_out, atk, base2k, dsize_atk, entry_stride=g,
+                     scratch=scratch)
+    return res
+
+
 # ---- glwe_pack / post_process / exponent mode -----------------------------------------------------------------------------------
 class DeviceGlweOps:
     """The GLWE operations `pack_internal` and `post_process` are made of, on batches of device-resident GLWEs (VecZnx with a batch axis)

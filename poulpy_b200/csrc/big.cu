@@ -10,18 +10,7 @@
 //   poulpy-cpu-ref/src/reference/vec_znx/normalize.rs:52-380      the i64 twins
 // per coefficient instead of per slice.
 #include "internal.h"
-
-template <typename T> struct BT;
-template <> struct BT<i128> { typedef u128 U; static constexpr int BITS = 128; };
-template <> struct BT<long long> { typedef unsigned long long U; static constexpr int BITS = 64; };
-
-template <typename T> __device__ __forceinline__ T wadd(T a, T b) { return (T)((typename BT<T>::U)a + (typename BT<T>::U)b); }
-template <typename T> __device__ __forceinline__ T wsub(T a, T b) { return (T)((typename BT<T>::U)a - (typename BT<T>::U)b); }
-template <typename T> __device__ __forceinline__ T wshl(T a, int s) { return (T)((typename BT<T>::U)a << s); }
-template <typename T> __device__ __forceinline__ T get_digit(int k, T x) {
-    return (T)((typename BT<T>::U)x << (BT<T>::BITS - k)) >> (BT<T>::BITS - k);
-}
-template <typename T> __device__ __forceinline__ T get_carry(int k, T x, T d) { return wsub<T>(x, d) >> k; }
+#include "znx.cuh"
 
 __device__ __forceinline__ long long apply_op(int op, long long r, long long x) {
     if (op == 0) return x;
@@ -324,21 +313,10 @@ __global__ void __launch_bounds__(256) rotate_kernel(RotArgs q) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; // destination index
     if (i >= q.n) return;
     const long long p = q.p_dev ? q.p_dev[(size_t)blockIdx.z * q.p_stride] : q.p;
-    const uint32_t n = q.n;
-    const uint32_t mp_2n = (uint32_t)(p & (long long)(2 * n - 1));
-    const uint32_t mp_1n = mp_2n & (n - 1);
-    const bool neg_first = mp_2n < n;
     const long long *src = reinterpret_cast<const long long *>(q.a.base + (size_t)blockIdx.z * q.a.batch_stride + (size_t)blockIdx.y * q.a.limb_stride);
     long long *dst = reinterpret_cast<long long *>(q.dst.base + (size_t)blockIdx.z * q.dst.batch_stride + (size_t)blockIdx.y * q.dst.limb_stride);
-    long long v;
     bool neg;
-    if (i < mp_1n) {
-        v = src[n - mp_1n + i];
-        neg = neg_first;
-    } else {
-        v = src[i - mp_1n];
-        neg = !neg_first;
-    }
+    const long long v = rotate_read([&](uint32_t k) { return src[k]; }, i, p, q.n, &neg);
     dst[i] = neg ? (long long)(0ull - (unsigned long long)v) : v;
 }
 int znx_rotate(pgb_module *m, LimbSet dst, LimbSet a, long long p, const long long *p_dev, uint32_t p_stride, uint32_t jobs, uint32_t batch) {
@@ -422,8 +400,7 @@ int znx_automorphism(pgb_module *m, LimbSet dst, LimbSet a, long long p, uint32_
 }
 
 // vec_znx_rsh_assign (reference/vec_znx/shift.rs:186-243): right shift by k bits in base 2^K, in place, one thread per coefficient walking
-// the limbs with the carry in a register.  The three loops follow the reference verbatim, including the order of its last loop (zero
-// limb j, then step on limb steps-1-j), which is only the arithmetic shift for steps <= 1 or k a multiple of K.
+// the limbs with the carry in a register (rsh_assign_coeff, znx.cuh)
 struct RshArgs {
     LimbSet r;
     uint32_t n;
@@ -433,38 +410,7 @@ __global__ void __launch_bounds__(256) znx_rsh_assign_kernel(RshArgs q) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= q.n) return;
     char *rb = q.r.base + (size_t)blockIdx.y * q.r.batch_stride;
-#define R_AT(j) (reinterpret_cast<long long *>(rb + (size_t)(j) * q.r.limb_stride)[i])
-    typedef long long T;
-    const int K = q.K, size = q.size, k_rem = q.k % K;
-    const int steps = q.k / K + (k_rem ? 1 : 0), lsh = (K - k_rem) % K, w = lsh == 0 ? K : K - lsh;
-    T c = 0;
-    for (int j = 0; j < steps; j++) {
-        const T x = R_AT(size - j - 1);
-        const T d = get_digit<T>(w, x), co = get_carry<T>(w, x, d);
-        if (j == 0) c = co;
-        else {
-            const T s = wadd<T>(wshl<T>(d, lsh), c);
-            c = wadd<T>(co, get_carry<T>(K, s, get_digit<T>(K, s)));
-        }
-    }
-    for (int j = 0; j < size - steps; j++) {
-        const T x = R_AT(size - steps - j - 1);
-        const T d = get_digit<T>(w, x), co = get_carry<T>(w, x, d);
-        const T s = wadd<T>(wshl<T>(d, lsh), c);
-        const T out = get_digit<T>(K, s);
-        c = wadd<T>(co, get_carry<T>(K, s, out));
-        R_AT(size - j - 1) = out;
-    }
-    for (int j = 0; j < steps; j++) {
-        R_AT(j) = 0;
-        const T x = R_AT(steps - j - 1);
-        const T d = get_digit<T>(w, x);
-        const T s = wadd<T>(wshl<T>(d, lsh), c);
-        const T out = get_digit<T>(K, s);
-        if (j != 0) c = wadd<T>(get_carry<T>(w, x, d), get_carry<T>(K, s, out));
-        R_AT(steps - j - 1) = out;
-    }
-#undef R_AT
+    rsh_assign_coeff([&](int j) -> long long & { return reinterpret_cast<long long *>(rb + (size_t)j * q.r.limb_stride)[i]; }, q.size, q.K, q.k);
 }
 int znx_rsh_assign(pgb_module *m, LimbSet r, int size, int base2k, int k, uint32_t batch, uint32_t words) {
     if (size == 0 || batch == 0) return PGB_OK;

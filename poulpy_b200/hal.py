@@ -88,7 +88,7 @@ def lib():
         for name in ("pgb_glwe_keyswitch_tmp_bytes", "pgb_glwe_external_product_tmp_bytes", "pgb_cggi_blind_rotate_tmp_bytes",
                      "pgb_cggi_blind_rotate_standard_tmp_bytes", "pgb_cggi_blind_rotate_extended_tmp_bytes", "pgb_vmp_apply_dft_tmp_bytes", "pgb_glwe_tensor_apply_tmp_bytes",
                      "pgb_glwe_tensor_relinearize_tmp_bytes", "pgb_glwe_automorphism_tmp_bytes", "pgb_glwe_automorphism_add_assign_tmp_bytes",
-                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_glwe_cmux_tmp_bytes", "pgb_glwe_blind_rotate_ggsw_tmp_bytes", "pgb_glwe_cmux_tree_tmp_bytes", "pgb_glwe_bdd_eval_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
+                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_glwe_cmux_tmp_bytes", "pgb_glwe_blind_rotate_ggsw_tmp_bytes", "pgb_glwe_cmux_tree_tmp_bytes", "pgb_glwe_bdd_eval_tmp_bytes", "pgb_glwe_pack_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
                      "pgb_vec_znx_big_automorphism_assign_tmp_bytes", "pgb_ggsw_expand_row_tmp_bytes",
                      "pgb_bytes_of_vmp_pmat", "pgb_size_of_scalar_prep", "pgb_size_of_scalar_big"):
             getattr(_lib, name).restype = C.c_size_t
@@ -650,6 +650,31 @@ class Module:
                                                _u64(dsize), C.byref(cs), C.byref(bt), C.c_void_p(scratch.ptr),
                                                C.c_size_t(need if max_chunk is not None else scratch.nbytes)))
         del keep
+        return scratch
+
+    def glwe_pack(self, res: VecZnx, a: VecZnx, index, log_gap_out, keys, base2k, dsize=1, entry_stride=None, max_chunk=None,
+                  scratch: DevBuf = None):
+        """glwe_pack of n_in = len(index) GLWEs per item into one: res_b's coefficient index[j] carries the constant coefficient of item b's
+        input j, bit for bit what circuit.glwe_pack computes over circuit.DeviceGlweOps.  `a` holds the inputs: item b's input j at
+        a + b * a.batch_stride + j * entry_stride (default: one GLWE of a.size limbs, inputs consecutive); an `a` with batch 1 is shared by
+        the batch.  The inputs are read-only.  keys: log_n prepared automorphism keys, keys[i] for trace_galois_element(i).  max_chunk
+        bounds the items per chunk (the scratch grows with it; results do not depend on it).  Asynchronous."""
+        idx = np.ascontiguousarray(np.asarray(index, dtype=np.uint32).reshape(-1))
+        B = res.batch
+        assert a.batch in (1, B), (a.batch, B)
+        entry_stride = self.n * a.cols * a.size * 8 if entry_stride is None else entry_stride
+        arr = (_PM * len(keys))(*[k.struct() for k in keys])
+        chunk = B if max_chunk is None else min(B, max_chunk)
+        ip = idx.ctypes.data_as(C.POINTER(C.c_uint32))
+        need = lib().pgb_glwe_pack_tmp_bytes(self._h, _u64(res.size), _u64(base2k), C.byref(arr[0]), _u64(dsize), ip, _u64(len(idx)),
+                                             _u64(log_gap_out), _u64(chunk))
+        if scratch is None or scratch.nbytes < need:
+            scratch = self._scratch(max(need, 1))
+        r, av = res.struct(), a.struct()
+        bt = _BT(B, res.batch_stride, a.batch_stride if a.batch > 1 else 0, 0)
+        _check(lib().pgb_glwe_pack_batched(self._h, C.byref(r), C.byref(av), _u64(entry_stride), ip, _u64(len(idx)), _u64(log_gap_out),
+                                           _u64(base2k), arr, _u64(len(keys)), _u64(dsize), C.byref(bt), C.c_void_p(scratch.ptr),
+                                           C.c_size_t(need if max_chunk is not None else scratch.nbytes)))
         return scratch
 
     def gadget_key_pin(self, key: VmpPMat):
