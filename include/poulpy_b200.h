@@ -581,6 +581,22 @@ size_t pgb_glwe_to_lwe_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_
                                  uint64_t key_base2k, uint64_t dsize, uint64_t batch);
 int pgb_glwe_to_lwe_batched(pgb_module *m, pgb_vec_znx *res, uint64_t res_base2k, const pgb_vec_znx *a, uint64_t a_base2k,
                             const pgb_vmp_pmat *key, uint64_t key_base2k, uint64_t dsize, const pgb_batch *bt, void *scratch, size_t scratch_len);
+/* glwe_to_lwe at many coefficients, one key-switch per item: per item b, g_b = glwe_keyswitch(a_b) into a staged rank-1 GLWE of res.size
+ * limbs of res_base2k (the key, routes and scratch rule of pgb_glwe_to_lwe_batched), and for j < n_index the LWE at res->data +
+ * b*bt->stride_res + j*entry_stride is lwe_sample_extract(vec_znx_rotate(-index[j], g_b)): for limbs l < min(res.size, g.size),
+ * b' = g[l][0][idx] and a'_t = g[l][1][idx + t] (idx + t < N) or -g[l][1][idx + t - N]; the other limbs are zeroed.  index = {0} gives
+ * pgb_glwe_to_lwe_batched bit for bit.  This is "key-switch, then rotate": it is not bit-identical to rotating a before the key-switch (a
+ * rotation negates wrapped digits without renormalising, and the key-switch's final rounding need not be odd-symmetric), but both orders
+ * agree modulo 2^(res.size * res_base2k) within one unit of the last limb.
+ * `index` is a HOST array of n_index in [1, N] coefficients, each below N (duplicates allowed); entry_stride a multiple of 8 of at least one
+ * LWE when n_index > 1; bt->stride_res a multiple of 8 of at least (n_index-1)*entry_stride plus one LWE when count > 1; res must not
+ * overlap a over the whole extent (PGB_ERR_ALIAS).  Every check runs before the first launch.  Scratch: the index table (one upload per
+ * call) at its head, then `batch` staged GLWEs, then the key-switch's scratch; _tmp_bytes takes n_index before the batch count. */
+size_t pgb_glwe_to_lwe_indexed_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_t a_size, uint64_t a_base2k, const pgb_vmp_pmat *key,
+                                         uint64_t key_base2k, uint64_t dsize, uint64_t n_index, uint64_t batch);
+int pgb_glwe_to_lwe_indexed_batched(pgb_module *m, pgb_vec_znx *res, uint64_t entry_stride, uint64_t res_base2k, const pgb_vec_znx *a,
+                                    uint64_t a_base2k, const uint32_t *index, uint64_t n_index, const pgb_vmp_pmat *key, uint64_t key_base2k,
+                                    uint64_t dsize, const pgb_batch *bt, void *scratch, size_t scratch_len);
 size_t pgb_lwe_to_glwe_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_t a_size, uint64_t a_base2k, const pgb_vmp_pmat *key,
                                  uint64_t key_base2k, uint64_t dsize, uint64_t batch);
 int pgb_lwe_to_glwe_batched(pgb_module *m, pgb_vec_znx *res, uint64_t res_base2k, const pgb_vec_znx *a, uint64_t a_base2k,

@@ -324,6 +324,30 @@ def bdd_eval_packed(module: "hal.Module", circuit, sel: "hal.VmpPMat", batch, n_
     return res
 
 
+def ggsw_bits_from_packed(module: "hal.Module", packed: "hal.VecZnx", index, ksk: "hal.VmpPMat", n_lwe, lwe_size, brk: "hal.VmpPMat",
+                          x_pow_a, block_size, atk, tsk, base2k, rank, dnum_res, res_size, log_domain, packed_base2k=None, ksk_base2k=None,
+                          dsize_ksk=1, dsize_atk=1, dsize_tsk=1, extension_factor=1) -> "hal.VmpPMat":
+    """Packed GLWEs back to prepared GGSW bits, the inverse of bdd_eval_packed: per item b of `packed` (one GLWE per integer, any rank),
+    coefficient index[j] is read as an LWE of dimension n_lwe under the blind-rotation key's secret by Module.glwe_to_lwe_indexed (one
+    key-switch per item with ksk = VmpPMat(dnum, rank_packed, 2, .) to that secret's embedding, into lwe_size limbs of base2k), then all
+    batch * len(index) LWEs are circuit-bootstrapped (circuit_bootstrap_to_constant, same arguments) and prepared (prepare_ggsw).
+
+    Encoding: circuit bootstrapping reads bit m at m / 2^(log_domain + 1) of the LWE's torus (one padding bit), so coefficient index[j]
+    must carry its bit at that scale: a GLWE from bdd_eval_packed must have been made with scale = 2^(base2k - log_domain - 1).
+
+    -> a batched VmpPMat of batch * len(index) GGSWs (dnum_res, rank + 1, rank + 1, res_size), GGSW b * len(index) + j holding bit j of
+    item b: the bit-major selector default of glwe_blind_rotate_ggsw, glwe_cmux_tree and glwe_bdd_eval with n_bits = len(index)."""
+    index = [int(i) for i in index]
+    batch, n_bits = packed.batch, len(index)
+    packed_base2k = base2k if packed_base2k is None else packed_base2k
+    ksk_base2k = base2k if ksk_base2k is None else ksk_base2k
+    lwe = hal.DevBuf(batch * n_bits * lwe_size * (n_lwe + 1) * 8, device=module.device)
+    module.glwe_to_lwe_indexed(lwe, n_lwe, lwe_size, base2k, packed, packed_base2k, index, ksk, ksk_base2k, dsize_ksk)
+    ggsw = circuit_bootstrap_to_constant(module, lwe, batch * n_bits, n_lwe, lwe_size, base2k, brk, x_pow_a, block_size, atk, tsk, base2k,
+                                         rank, dnum_res, res_size, log_domain, dsize_atk, dsize_tsk, extension_factor)
+    return prepare_ggsw(module, ggsw, batch * n_bits, dnum_res, rank, res_size)
+
+
 # ---- glwe_pack / post_process / exponent mode -----------------------------------------------------------------------------------
 class DeviceGlweOps:
     """The GLWE operations `pack_internal` and `post_process` are made of, on batches of device-resident GLWEs (VecZnx with a batch axis)

@@ -27,19 +27,41 @@ __global__ void __launch_bounds__(256) lwe_embed_kernel(LweEmbedArgs p) {
     reinterpret_cast<long long *>(p.glwe + (size_t)blockIdx.z * p.glwe_bs)[(size_t)j * 2 * p.n + t] = v;
 }
 
+// Entry e of item b is lwe_sample_extract(vec_znx_rotate(-index[e], glwe_b)) at lwe + b * lwe_bs + e * entry_bs: b' = c0[idx], a'_t =
+// c1[idx + t], negated where idx + t wraps past N.  A null index is coefficient 0 and one entry (the plain extraction).  The entries ride in
+// grid x (tiles * entries <= 257 * 2^16 blocks), so y (limbs) and z (items) stay within 65535 for every accepted shape.
 struct LweExtractArgs {
     const char *glwe; uint64_t glwe_bs; // rank-1 GLWE VecZnx(n, 2, >= copy limbs)
     char *lwe; uint64_t lwe_bs;         // LWE VecZnx(len, 1, gridDim.y limbs)
+    const uint32_t *index; uint64_t entry_bs;
     uint32_t n, len, copy;              // len = n_lwe + 1; limbs j < copy are copied, the others zeroed
+    uint32_t tiles;                     // blocks per entry, ceil(len / 256)
 };
+template <bool INDEXED>
 __global__ void __launch_bounds__(256) lwe_extract_kernel(LweExtractArgs p) {
-    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    uint32_t x = blockIdx.x, idx = 0;
+    uint64_t entry = 0;
+    if constexpr (INDEXED) {
+        const uint32_t e = x / p.tiles;
+        x -= e * p.tiles;
+        idx = p.index[e];
+        entry = (size_t)e * p.entry_bs;
+    }
+    const uint32_t t = x * blockDim.x + threadIdx.x;
     if (t >= p.len) return;
     const uint32_t j = blockIdx.y;
     long long v = 0;
-    if (j < p.copy)
-        v = reinterpret_cast<const long long *>(p.glwe + (size_t)blockIdx.z * p.glwe_bs)[(size_t)j * 2 * p.n + (t == 0 ? 0 : p.n + t - 1)];
-    reinterpret_cast<long long *>(p.lwe + (size_t)blockIdx.z * p.lwe_bs)[(size_t)j * p.len + t] = v;
+    if (j < p.copy) {
+        const long long *g = reinterpret_cast<const long long *>(p.glwe + (size_t)blockIdx.z * p.glwe_bs);
+        if constexpr (INDEXED) {
+            const uint32_t c = idx + t - 1; // t >= 1: the mask coefficient idx + t - 1 of column 1, one wrap at most
+            g += (size_t)j * 2 * p.n;
+            v = t == 0 ? g[idx] : c < p.n ? g[p.n + c] : -g[c];
+        } else {
+            v = g[(size_t)j * 2 * p.n + (t == 0 ? 0 : p.n + t - 1)];
+        }
+    }
+    reinterpret_cast<long long *>(p.lwe + (size_t)blockIdx.z * p.lwe_bs + entry)[(size_t)j * p.len + t] = v;
 }
 
 static int launch_embed(pgb_module *m, char *glwe, uint64_t glwe_bs, const pgb_vec_znx *a, uint64_t a_bs, uint64_t B) {
@@ -51,10 +73,16 @@ static int launch_embed(pgb_module *m, char *glwe, uint64_t glwe_bs, const pgb_v
     return PGB_OK;
 }
 
-static int launch_extract(pgb_module *m, pgb_vec_znx *res, uint64_t res_bs, const char *glwe, uint64_t glwe_bs, uint64_t glwe_size, uint64_t B) {
-    LweExtractArgs p = {glwe, glwe_bs, (char *)res->data, res_bs, (uint32_t)m->n, (uint32_t)res->n, (uint32_t)umin64(res->size, glwe_size)};
+// index: a device array of n_index coefficients, or null (coefficient 0, one entry)
+static int launch_extract(pgb_module *m, pgb_vec_znx *res, uint64_t res_bs, const char *glwe, uint64_t glwe_bs, uint64_t glwe_size, uint64_t B,
+                          const uint32_t *index = nullptr, uint64_t n_index = 1, uint64_t entry_bs = 0) {
+    const uint32_t tiles = (uint32_t)((res->n + 255) / 256);
+    LweExtractArgs p = {glwe, glwe_bs, (char *)res->data, res_bs, index, entry_bs, (uint32_t)m->n, (uint32_t)res->n,
+                        (uint32_t)umin64(res->size, glwe_size), tiles};
     { ProfScope _ps(m, PROF_OTHER);
-    lwe_extract_kernel<<<dim3((uint32_t)((res->n + 255) / 256), (uint32_t)res->size, (uint32_t)B), 256, 0, m->stream>>>(p);
+    const dim3 grid((uint32_t)(tiles * n_index), (uint32_t)res->size, (uint32_t)B);
+    if (index) lwe_extract_kernel<true><<<grid, 256, 0, m->stream>>>(p);
+    else lwe_extract_kernel<false><<<grid, 256, 0, m->stream>>>(p);
     }
     PGB_CHECK_CUDA(cudaGetLastError());
     return PGB_OK;
@@ -171,6 +199,59 @@ extern "C" int pgb_glwe_to_lwe_batched(pgb_module *m, pgb_vec_znx *res, uint64_t
     pgb_batch btk = {B, out_bs, bt->stride_a, 0};
     PGB_TRY(pgb_glwe_keyswitch_batched(m, &gout, res_base2k, a, a_base2k, key, key_base2k, dsize, &btk, ar.rest(), ar.rest_len()));
     return launch_extract(m, res, bt->stride_res, out, out_bs, res->size, B);
+}
+
+// ---- GLWE -> LWE at many coefficients: glwe_keyswitch to rank 1 once per item -> one extraction per index ---------------------------------
+// Key-switching is linear, so one key-switch per item serves every coefficient: LWE (b, j) is extracted from X^-index[j] times the staged
+// GLWE, a permutation with sign flips done while copying.  Scratch: the index table, then the staged GLWEs, then the key-switch's scratch.
+extern "C" size_t pgb_glwe_to_lwe_indexed_tmp_bytes(const pgb_module *m, uint64_t res_size, uint64_t a_size, uint64_t a_base2k,
+                                                    const pgb_vmp_pmat *key, uint64_t key_base2k, uint64_t dsize, uint64_t n_index, uint64_t batch) {
+    return align_up(n_index * sizeof(uint32_t)) + pgb_glwe_to_lwe_tmp_bytes(m, res_size, a_size, a_base2k, key, key_base2k, dsize, batch);
+}
+extern "C" int pgb_glwe_to_lwe_indexed_batched(pgb_module *m, pgb_vec_znx *res, uint64_t entry_stride, uint64_t res_base2k, const pgb_vec_znx *a,
+                                               uint64_t a_base2k, const uint32_t *index, uint64_t n_index, const pgb_vmp_pmat *key,
+                                               uint64_t key_base2k, uint64_t dsize, const pgb_batch *bt, void *scratch, size_t scratch_len) {
+    const char *what = "glwe_to_lwe_indexed";
+    PGB_TRY(check_batch(what, bt));
+    const uint64_t B = bt->count, n = m->n;
+    PGB_TRY(check_lwe(what, "res", m, res, bt->stride_res, 1)); // the batch stride is checked against the entries below
+    PGB_REQUIRE(bt->stride_res % 8 == 0, "%s: stride_res %llu must be a multiple of 8", what, (unsigned long long)bt->stride_res);
+    PGB_REQUIRE(a->cols >= 2, "%s: a must be a GLWE of rank >= 1", what);
+    PGB_TRY(check_glwe(what, "a", m, a, a->cols, bt->stride_a, B));
+    PGB_TRY(check_key(what, m, key, a->cols - 1, 2, dsize));
+    // ---- the index table ----
+    PGB_REQUIRE(index != nullptr && n_index >= 1 && n_index <= n, "%s: index must be a non-null host array of n_index in [1, N = %llu] entries",
+                what, (unsigned long long)n);
+    for (uint64_t j = 0; j < n_index; j++)
+        PGB_REQUIRE(index[j] < n, "%s: index[%llu] = %u is not below N = %llu", what, (unsigned long long)j, index[j], (unsigned long long)n);
+    // ---- entry and item strides, extents in 128 bits, aliasing ----
+    const uint64_t lwe = res->n * res->size * 8;
+    PGB_REQUIRE(entry_stride % 8 == 0 && (n_index == 1 || entry_stride >= lwe),
+                "%s: entry_stride %llu must be a multiple of 8 of at least one LWE (%llu bytes)", what, (unsigned long long)entry_stride,
+                (unsigned long long)lwe);
+    const unsigned __int128 item128 = (unsigned __int128)(n_index - 1) * entry_stride + lwe; // one item's LWEs
+    PGB_REQUIRE(B == 1 || (unsigned __int128)bt->stride_res >= item128,
+                "%s: stride_res %llu must be at least (n_index - 1) * entry_stride + one LWE", what, (unsigned long long)bt->stride_res);
+    const unsigned __int128 res_ext128 = (unsigned __int128)(B - 1) * bt->stride_res + item128;
+    const unsigned __int128 a_ext128 = (unsigned __int128)(B - 1) * bt->stride_a + n * a->cols * a->size * 8;
+    PGB_REQUIRE(res_ext128 <= (unsigned __int128)(UINTPTR_MAX - (uintptr_t)res->data), "%s: res extends past the end of the address space",
+                what);
+    PGB_REQUIRE(a_ext128 <= (unsigned __int128)(UINTPTR_MAX - (uintptr_t)a->data), "%s: a extends past the end of the address space", what);
+    if (ranges_overlap(res->data, (uint64_t)res_ext128, a->data, (uint64_t)a_ext128)) {
+        pgb_set_error("%s: res and a must not overlap", what);
+        return PGB_ERR_ALIAS;
+    }
+    PGB_TRY(check_scratch(what, scratch, scratch_len,
+                          pgb_glwe_to_lwe_indexed_tmp_bytes(m, res->size, a->size, a_base2k, key, key_base2k, dsize, n_index, B)));
+    const uint64_t out_bs = n * 2 * res->size * 8;
+    Arena ar = {(char *)scratch, scratch_len, 0};
+    uint32_t *idx = (uint32_t *)ar.take(n_index * sizeof(uint32_t));
+    char *out = (char *)ar.take(B * out_bs);
+    pgb_vec_znx gout = mk(out, n, 2, res->size);
+    pgb_batch btk = {B, out_bs, bt->stride_a, 0};
+    PGB_TRY(pgb_glwe_keyswitch_batched(m, &gout, res_base2k, a, a_base2k, key, key_base2k, dsize, &btk, ar.rest(), ar.rest_len()));
+    PGB_CHECK_CUDA(cudaMemcpyAsync(idx, index, n_index * sizeof(uint32_t), cudaMemcpyHostToDevice, m->stream));
+    return launch_extract(m, res, bt->stride_res, out, out_bs, res->size, B, idx, n_index, entry_stride);
 }
 
 // ---- GLWE::from_lwe (conversion/lwe_to_glwe.rs): embed -> glwe_keyswitch to rank k ------------------------------------------------------------

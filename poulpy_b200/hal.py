@@ -88,7 +88,7 @@ def lib():
         for name in ("pgb_glwe_keyswitch_tmp_bytes", "pgb_glwe_external_product_tmp_bytes", "pgb_cggi_blind_rotate_tmp_bytes",
                      "pgb_cggi_blind_rotate_standard_tmp_bytes", "pgb_cggi_blind_rotate_extended_tmp_bytes", "pgb_vmp_apply_dft_tmp_bytes", "pgb_glwe_tensor_apply_tmp_bytes",
                      "pgb_glwe_tensor_relinearize_tmp_bytes", "pgb_glwe_automorphism_tmp_bytes", "pgb_glwe_automorphism_add_assign_tmp_bytes",
-                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_glwe_cmux_tmp_bytes", "pgb_glwe_blind_rotate_ggsw_tmp_bytes", "pgb_glwe_cmux_tree_tmp_bytes", "pgb_glwe_bdd_eval_tmp_bytes", "pgb_glwe_pack_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
+                     "pgb_glwe_trace_assign_tmp_bytes", "pgb_glwe_cmux_tmp_bytes", "pgb_glwe_blind_rotate_ggsw_tmp_bytes", "pgb_glwe_cmux_tree_tmp_bytes", "pgb_glwe_bdd_eval_tmp_bytes", "pgb_glwe_pack_tmp_bytes", "pgb_lwe_keyswitch_tmp_bytes", "pgb_glwe_to_lwe_tmp_bytes", "pgb_glwe_to_lwe_indexed_tmp_bytes", "pgb_lwe_to_glwe_tmp_bytes",
                      "pgb_vec_znx_big_automorphism_assign_tmp_bytes", "pgb_ggsw_expand_row_tmp_bytes",
                      "pgb_bytes_of_vmp_pmat", "pgb_size_of_scalar_prep", "pgb_size_of_scalar_big"):
             getattr(_lib, name).restype = C.c_size_t
@@ -963,6 +963,27 @@ class Module:
         bt = _BT(a.batch, self._lwe_stride(n_lwe, res_size, res_stride), a.batch_stride, 0)
         return self._lwe_call("pgb_glwe_to_lwe", self._lwe(res, n_lwe, res_size), res_size, res_base2k, a.struct(), a.size, a_base2k, key,
                               key_base2k, dsize, bt, scratch)
+
+    def glwe_to_lwe_indexed(self, res: DevBuf, n_lwe, res_size, res_base2k, a: VecZnx, a_base2k, index, key: VmpPMat, key_base2k, dsize=1,
+                            entry_stride=None, res_stride=None, scratch: DevBuf = None):
+        """glwe_to_lwe at the coefficients `index` (host list, each below n) of the a.batch GLWEs of rank k, with one key-switch per item:
+        LWE (b, j) = lwe_sample_extract(X^-index[j] * glwe_keyswitch(a_b)), at res + b * res_stride + j * entry_stride (defaults: one LWE
+        apart, res_stride = len(index) * entry_stride, so LWE b * len(index) + j is coefficient index[j] of item b: the item-major order of
+        circuit_bootstrap_to_constant).  index = [0] equals glwe_to_lwe.  key = VmpPMat(dnum, k, 2, key_size)."""
+        idx = np.ascontiguousarray(np.asarray(index, dtype=np.uint32).reshape(-1))
+        entry_stride = self._lwe_stride(n_lwe, res_size, entry_stride)
+        res_stride = len(idx) * entry_stride if res_stride is None else res_stride
+        ks = key.struct()
+        need = lib().pgb_glwe_to_lwe_indexed_tmp_bytes(self._h, _u64(res_size), _u64(a.size), _u64(a_base2k), C.byref(ks), _u64(key_base2k),
+                                                       _u64(dsize), _u64(len(idx)), _u64(a.batch))
+        if scratch is None or scratch.nbytes < need:
+            scratch = self._scratch(need)
+        r, av = self._lwe(res, n_lwe, res_size), a.struct()
+        bt = _BT(a.batch, res_stride, a.batch_stride, 0)
+        _check(lib().pgb_glwe_to_lwe_indexed_batched(self._h, C.byref(r), _u64(entry_stride), _u64(res_base2k), C.byref(av), _u64(a_base2k),
+                                                     idx.ctypes.data_as(C.POINTER(C.c_uint32)), _u64(len(idx)), C.byref(ks), _u64(key_base2k),
+                                                     _u64(dsize), C.byref(bt), C.c_void_p(scratch.ptr), C.c_size_t(scratch.nbytes)))
+        return scratch
 
     def lwe_to_glwe(self, res: VecZnx, res_base2k, a: DevBuf, n_lwe, a_size, a_base2k, key: VmpPMat, key_base2k, dsize=1,
                     scratch: DevBuf = None, a_stride=None):
